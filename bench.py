@@ -387,7 +387,7 @@ def run_gpu_arm(args):
     w0 = time.time()
     t_start.record()
     for _ in range(args.steps):
-        step(record=True)
+        outs = step(record=True)
     drain_comm()
     t_stop.record()
     barrier()
@@ -411,6 +411,9 @@ def run_gpu_arm(args):
 
     fwd_ms = statistics.mean(e0.elapsed_time(e1) for e0, e1, _ in kern_events)
     bwd_ms = statistics.mean(e1.elapsed_time(e2) for _, e1, e2 in kern_events)
+    if args.dump_outputs and rank == 0:                 # before the legs below run more steps on the same tensors
+        dump_outputs(args.dump_outputs, {f"call{k}_{name}": t for k, (out, (_, v, h, _)) in enumerate(zip(outs, sets))
+                                         for name, t in (("output", out), ("grad_vertical", v.grad), ("grad_horizontal", h.grad))})
 
     # ---- the reference's actual inputs are gray sections replicated x3: opt-in shortcut, reported aside
     gray = None
@@ -552,6 +555,26 @@ def run_gpu_arm(args):
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 60 * 10 ** 6                           # --dump-outputs writes at most this many bytes of array data
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each tensor of `arrays` as DIR/<name>.npy in float32.  When they do not fit in DUMP_BYTES together, each is
+    written as a 1-D sample of its flattened elements instead: sorted flat indices drawn from a seed fixed by the tensor's
+    position in `arrays`, so that two runs with the same arguments write the same elements."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    sample = sum(t.numel() for t in arrays.values()) * 4 > DUMP_BYTES
+    per = DUMP_BYTES // 4 // len(arrays)
+    for i, (name, t) in enumerate(arrays.items()):
+        t = t.detach()
+        if sample and t.numel() > per:
+            idx = np.unique(np.random.default_rng(i).integers(0, t.numel(), per))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(dirname, name + ".npy"), t.float().cpu().numpy())
 
 
 def _bind_near_gpu(dev):
@@ -992,7 +1015,12 @@ def main():
     ap.add_argument("--no-stack", action="store_true", help="skip BASELINE config 5 (the 100-section stack job)")
     ap.add_argument("--sections", type=int, default=100)
     ap.add_argument("--section-size", type=int, default=4096)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs and tap gradients as DIR/<name>.npy (float32; "
+                         "a fixed seeded sample of each when they exceed 60 MB together)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -1,21 +1,24 @@
 """Element-wise parity at BASELINE's real sizes against the REFERENCE'S OWN CUDA
-(libs/sepconv/src/SeparableConvolution_kernel.cu:25-52,77-150 compiled verbatim into oracle/_ref by
-oracle/Makefile; wrapped by tests/_ref_cuda.py), not only against size-independent properties.
+(libs/sepconv/src/SeparableConvolution_kernel.cu:25-52,77-150), not only against size-independent properties.
 
   c2   in[1,3,306,306],   v,h[1,51,256,256]    (whole section; KPN-like raw taps, |out| ~ 1e1..1e2)
   c3   in[2,3,562,562],   v,h[2,51,512,512]    (two samples of the training batch)
   c4   in[1,3,2098,2098], v,h[1,51,2048,2048]
 
-For each: the STRICT_ORDER forward is bit-equal to the reference kernel; the default (re-associated)
-forward / grad_vertical / grad_horizontal satisfy protocol P1 or P2 of SURVEY.md 8(c) element-wise over the
-whole tensor (|new - ref| <= 1e-5 * max(1, max|ref|) and err(new, fp64) <= max(1.25 * err(ref, fp64), 2e-6 * scale));
+tests/golden/sepconv_fullsize_ref.npz holds SHA-256 digests of these inputs and of the reference kernel's forward,
+grad_vertical and grad_horizontal on them (tests/golden/make_fullsize_parity_golden.py).  Whole tensors that match those
+digests bit for bit ARE the reference's outputs: the forward is the STRICT_ORDER forward of this package, the tap
+gradients are the CPU oracle's reference-order restatement (oracle/sepconv_oracle.c).  Against them, for each case, the
+default (re-associated) forward / grad_vertical / grad_horizontal satisfy protocol P1 or P2 of SURVEY.md 8(c) element-wise
+over the whole tensor (|new - ref| <= 1e-5 * max(1, max|ref|) and err(new, fp64) <= max(1.25 * err(ref, fp64), 2e-6 * scale));
 grad_input (absent in the reference) is compared with the fp64 adjoint.  fp64 truths are evaluated on the GPU with
-plain torch shifts (2 601 slice-multiply-adds); at c2 the CPU oracle (oracle/sepconv_oracle.c) is checked against
-the same reference run, which ties the three together.  Dense-tap accumulation across every tile seam of the
-full grid is what these cases add over the <= 64x64 oracle cases.
+plain torch shifts (2 601 slice-multiply-adds); at c2 the CPU oracle's forward is checked against the same reference
+output, which ties the three together.  Dense-tap accumulation across every tile seam of the full grid is what these
+cases add over the <= 64x64 oracle cases.
 
 The measured max-abs figures are written to gpurun_out/parity_fullsize.json (copied to profiles/ when run by hand).
 """
+import hashlib
 import json
 import os
 
@@ -24,9 +27,8 @@ import pytest
 import torch
 
 import oracle
-from tests import _ref_cuda
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not _ref_cuda.available(), reason="oracle/_ref not built")]
+pytestmark = pytest.mark.gpu
 
 TOL = 1e-5
 K = 51
@@ -74,6 +76,46 @@ def _kpn_like_taps(B, H, W, dev, seed, vmax):
 def _unit_taps(B, H, W, dev, seed):
     g = torch.Generator(device=dev).manual_seed(seed)
     return torch.softmax(torch.randn((B, K, H, W), device=dev, generator=g), 1).contiguous()
+
+
+def case_inputs(name, dev):
+    """(input, vertical, horizontal, grad_output) of one entry of CASES."""
+    B, H, W, kind = CASES[name]
+    inp = _em_input(B, H, W, dev, seed=700 + H)
+    if kind == "kpn":
+        v, h = _kpn_like_taps(B, H, W, dev, 31, 3.7), _kpn_like_taps(B, H, W, dev, 32, 7.4)
+    else:
+        v, h = _unit_taps(B, H, W, dev, 33), _unit_taps(B, H, W, dev, 34)
+    g = torch.randn((B, 3, H, W), device=dev, generator=torch.Generator(device=dev).manual_seed(99))
+    return inp, v, h, g
+
+
+def tail_inputs(dev):
+    """Two gray x3 512^2 frames and four unit-tap tensors: the reference's actual call."""
+    B, H, W = 1, 512, 512
+    return _em_input(B, H, W, dev, seed=41), _em_input(B, H, W, dev, seed=43), [_unit_taps(B, H, W, dev, 50 + i) for i in range(4)]
+
+
+def sha256(*tensors):
+    """SHA-256 of the tensors' bytes, in order, as uint8[32] (the format of the digests in the golden fixtures)."""
+    d = hashlib.sha256()
+    for t in tensors:
+        d.update(t.detach().contiguous().cpu().numpy())
+    return np.frombuffer(d.digest(), np.uint8)
+
+
+def _check_digest(key, what, *tensors):
+    want = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sepconv_fullsize_ref.npz"))[key + "_sha256"]
+    assert np.array_equal(sha256(*tensors), want), f"{key}: {what}"
+
+
+def _strict_forward(inp, v, h):
+    import sstem_restoration_b200 as pkg
+    pkg.set_strict_order(True)
+    try:
+        return pkg.SeparableConvolution.apply(inp, v, h)
+    finally:
+        pkg.set_strict_order(False)
 
 
 def _truth_f64(inp, v, h, g):
@@ -127,26 +169,18 @@ def test_fullsize_forward_and_tap_gradients_vs_reference_cuda(name):
     import sstem_restoration_b200 as pkg
     B, H, W, kind = CASES[name]
     dev = torch.device("cuda")
-    inp = _em_input(B, H, W, dev, seed=700 + H)
-    if kind == "kpn":
-        v, h = _kpn_like_taps(B, H, W, dev, 31, 3.7), _kpn_like_taps(B, H, W, dev, 32, 7.4)
-    else:
-        v, h = _unit_taps(B, H, W, dev, 33), _unit_taps(B, H, W, dev, 34)
-    g = torch.randn((B, 3, H, W), device=dev, generator=torch.Generator(device=dev).manual_seed(99))
+    inp, v, h, g = case_inputs(name, dev)
+    _check_digest(name + "_inputs", "not the inputs the stored reference outputs were computed from", inp, v, h, g)
 
-    ref_out = _ref_cuda.forward(inp, v, h)
-    ref_gi, ref_gv, ref_gh = _ref_cuda.backward(g, inp, v, h)
-    assert not bool(ref_gi.any())                         # SeparableConvolution.py:60: the reference never computes it
-
-    # strict order: bit-equal over the whole tensor
-    pkg.set_strict_order(True)
-    try:
-        strict = pkg.SeparableConvolution.apply(inp, v, h)
-    finally:
-        pkg.set_strict_order(False)
-    nbad = int((strict.view(torch.int32) != ref_out.view(torch.int32)).sum())
-    _record(name, strict_fwd_mismatching_elements=nbad)
-    assert nbad == 0, f"{name}: strict-order forward differs from the reference kernel in {nbad} elements"
+    # strict order: bit-equal to the reference kernel over the whole tensor
+    ref_out = _strict_forward(inp, v, h)
+    _check_digest(name + "_out", "strict-order forward is not bit-equal to the reference kernel", ref_out)
+    # the reference kernel's tap gradients: the oracle's reference-order restatement, bit-equal over the whole tensor
+    ni, nv, nh, ng = (t.cpu().numpy() for t in (inp, v, h, g))
+    ref_gv = torch.from_numpy(oracle.sepconv_grad_vertical_reforder(ng, ni, nh)).to(dev)
+    _check_digest(name + "_gv", "oracle grad_vertical is not bit-equal to the reference kernel", ref_gv)
+    ref_gh = torch.from_numpy(oracle.sepconv_grad_horizontal_reforder(ng, ni, nv)).to(dev)
+    _check_digest(name + "_gh", "oracle grad_horizontal is not bit-equal to the reference kernel", ref_gh)
 
     # default kernels
     iv = inp.clone().requires_grad_(True)
@@ -162,12 +196,9 @@ def test_fullsize_forward_and_tap_gradients_vs_reference_cuda(name):
     _record(name, gi_err_f64=gi_err, gi_scale=gscale)
     assert gi_err <= TOL * gscale, f"{name} gi: {gi_err:.3e} (scale {gscale:.3g})"
 
-    if H <= 256:                                          # tie the CPU oracle to the same reference run (seconds in C)
-        ni, nv, nh, ng = (t.cpu().numpy() for t in (inp, v, h, g))
+    if H <= 256:                                          # tie the CPU oracle's forward to the same reference output (seconds in C)
         assert np.array_equal(oracle.sepconv_forward_reforder(ni, nv, nh).view(np.uint32), ref_out.cpu().numpy().view(np.uint32))
-        assert np.array_equal(oracle.sepconv_grad_vertical_reforder(ng, ni, nh).view(np.uint32), ref_gv.cpu().numpy().view(np.uint32))
-        assert np.array_equal(oracle.sepconv_grad_horizontal_reforder(ng, ni, nv).view(np.uint32), ref_gh.cpu().numpy().view(np.uint32))
-    del t_out, t_gv, t_gh, t_gi
+    del t_out, t_gv, t_gh, t_gi, ref_gv, ref_gh
     torch.cuda.empty_cache()
 
 
@@ -176,12 +207,12 @@ def test_fullsize_gray_shortcut_and_fused_tail_vs_reference_cuda():
     fused tail within 1e-5 of mean_c(ref(i2) + ref(i1)) computed by the reference kernel."""
     import sstem_restoration_b200 as pkg
     dev = torch.device("cuda")
-    B, H, W = 1, 512, 512
-    inp = _em_input(B, H, W, dev, seed=41)
-    inp2 = _em_input(B, H, W, dev, seed=43)
-    taps = [_unit_taps(B, H, W, dev, 50 + i) for i in range(4)]
-    ref1 = _ref_cuda.forward(inp, taps[0], taps[1])
-    ref2 = _ref_cuda.forward(inp2, taps[2], taps[3])
+    inp, inp2, taps = tail_inputs(dev)
+    _check_digest("tail_512_inputs", "not the inputs the stored reference outputs were computed from", inp, inp2, *taps)
+    ref1 = _strict_forward(inp, taps[0], taps[1])
+    _check_digest("tail_512_ref1", "strict-order forward is not bit-equal to the reference kernel", ref1)
+    ref2 = _strict_forward(inp2, taps[2], taps[3])
+    _check_digest("tail_512_ref2", "strict-order forward is not bit-equal to the reference kernel", ref2)
     general = pkg.SeparableConvolution.apply(inp, taps[0], taps[1])
     pkg.set_gray_replicated("assert")
     try:
