@@ -25,8 +25,9 @@ UNITS = [
     ("sepconv_k51_bwd.cu", ["-DSSTEM_BWD_PART=1"], "_p1"),
     ("sepconv_k51_bwd.cu", ["-DSSTEM_BWD_PART=2"], "_p2"),
     ("sepconv_k51_bwd.cu", ["-DSSTEM_BWD_PART=3"], "_p3"),
-    ("sepconv_k51_bwd2.cu", [], ""),
+    ("sepconv_k51_bwd3.cu", [], ""),
     ("sepconv_k51_fwd3.cu", [], ""),
+    ("sepconv_layout.cu", [], ""),
     ("sepconv_k51_gi.cu", [], ""),
     ("sepconv_k51_tail.cu", [], ""),
     ("warp.cu", [], ""),

@@ -66,10 +66,6 @@ extern "C" int sstem_sepconv_backward(const float* grad_output, const float* inp
 }
 
 // ---- gray x3 detection on the device (no host round trip) ------------------------------------------------------------
-namespace sstem {
-int launch_planes_equal(const float* in, int64_t B, int64_t C, int64_t plane, int* flag, cudaStream_t s);
-}
-
 extern "C" int sstem_sepconv_forward_detect(const float* input, const float* vertical, const float* horizontal,
                                             float* output, int64_t B, int64_t C, int64_t H, int64_t W,
                                             int32_t K, uint32_t flags, int32_t* gray_flag, void* stream) {

@@ -93,14 +93,17 @@ int launch_sepconv_bwd_input_k51(const float* g, const float* v, const float* h,
 int launch_sepconv_bwd_input_generic(const float* g, const float* v, const float* h, float* gi,
                                      int64_t B, int64_t C, int64_t H, int64_t W, int K, cudaStream_t s);
 
-// second / third generation 51-tap kernels (sepconv_k51_bwd2.cu, sepconv_k51_fwd3.cu); -1000 = path does not apply
-int workspace_alloc(void** p, size_t bytes, cudaStream_t s);
-int launch_repack_nhwc4(const float* in, float* ws, int64_t B, int C, int c0, int64_t IH, int64_t IW, cudaStream_t s);
-int try_launch_bwd_taps_k51_v2(const float* g, const float* in, const float* v, const float* h, float* gv, float* gh,
+// third-generation 51-tap kernels (sepconv_k51_bwd3.cu, sepconv_k51_fwd3.cu); -1000 = path does not apply
+int try_launch_bwd_taps_k51_v3(const float* g, const float* in, const float* v, const float* h, float* gv, float* gh,
                                int64_t B, int C, int c0, int H, int W, int accumulate, cudaStream_t s);
 int try_launch_fwd_k51_v3(const float* in, const float* v, const float* h, float* out,
                           int64_t B, int C, int c0, int H, int W, cudaStream_t s);
-int try_launch_fwd_k51_v3_c1(const float* in, const float* v, const float* h, float* out,
-                             int64_t B, int C, int c0, int H, int W, int replicas, cudaStream_t s);
+
+// layout kernels (sepconv_layout.cu): stream-ordered workspace, input repacks, gray x3 plane comparison
+int workspace_alloc(void** p, size_t bytes, cudaStream_t s);
+int launch_repack_nhwc4(const float* in, float* ws, int64_t B, int C, int c0, int64_t IH, int64_t IW, cudaStream_t s);
+int launch_repack_plane_pitch(const float* in, float* ws, int64_t B, int C, int c0, int64_t IH, int64_t IW, int64_t IWP,
+                              cudaStream_t s);
+int launch_planes_equal(const float* in, int64_t B, int64_t C, int64_t plane, int* flag, cudaStream_t s);
 
 }  // namespace sstem

@@ -71,8 +71,8 @@ int launch_bwd_all(const float* g, const float* in, const float* v, const float*
         const int acc = c0 > 0;
         int e;
         if (cc == 3) {
-            // second-generation kernel (TMA-staged, channel-interleaved window) when its layout rules hold
-            e = try_launch_bwd_taps_k51_v2(g, in, v, h, WV ? gv : nullptr, WH ? gh : nullptr, B, C, c0, H, W, acc, s);
+            // third-generation kernel (persistent warps, TMA-streamed, channel-interleaved window) when its layout rules hold
+            e = try_launch_bwd_taps_k51_v3(g, in, v, h, WV ? gv : nullptr, WH ? gh : nullptr, B, C, c0, H, W, acc, s);
             if (e == -1000) e = launch_bwd_chunk<3, WV, WH>(g, in, v, h, gv, gh, B, C, c0, H, W, acc, 1, s);
         }
         else if (cc == 2) e = launch_bwd_chunk<2, WV, WH>(g, in, v, h, gv, gh, B, C, c0, H, W, acc, 1, s);

@@ -35,10 +35,8 @@ int launch_sepconv_fwd_k51(const float* in, const float* v, const float* h, floa
                            int64_t B, int64_t C, int64_t H, int64_t W, bool gray, cudaStream_t s) {
     if (B > 65535 || (H + SSTEM_FWD_R - 1) / SSTEM_FWD_R > 65535)   // grid.y / grid.z limits
         return launch_sepconv_fwd_generic(in, v, h, out, B, C, H, W, 51, false, s);
-    if (gray && C > 1) {                                   // identical planes: compute one, write C copies
-        const int e = try_launch_fwd_k51_v3_c1(in, v, h, out, B, (int)C, 0, (int)H, (int)W, (int)C, s);
-        return e != -1000 ? e : launch_fwd_chunk<1>(in, v, h, out, B, (int)C, 0, (int)H, (int)W, (int)C, s);
-    }
+    if (gray && C > 1)                                     // identical planes: compute one, write C copies
+        return launch_fwd_chunk<1>(in, v, h, out, B, (int)C, 0, (int)H, (int)W, (int)C, s);
     int c0 = 0;
     while (c0 < C) {                                       // channels in chunks of <= 3 (taps re-read per chunk)
         const int cc = (C - c0) < 3 ? (int)(C - c0) : 3;
@@ -49,10 +47,7 @@ int launch_sepconv_fwd_k51(const float* in, const float* v, const float* h, floa
             if (e == -1000) e = launch_fwd_chunk<3>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
         }
         else if (cc == 2) e = launch_fwd_chunk<2>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
-        else {
-            e = try_launch_fwd_k51_v3_c1(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
-            if (e == -1000) e = launch_fwd_chunk<1>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
-        }
+        else e = launch_fwd_chunk<1>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
         if (e) return e;
         c0 += cc;
     }

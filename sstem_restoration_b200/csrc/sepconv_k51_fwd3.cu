@@ -1,7 +1,7 @@
 // Launchers of the third-generation forward kernel (device code in sepconv_k51_v3.cuh): copy the input into the layout
 // the window loads want (channel-interleaved for 3 channels, 16-byte pitch for 1) in a stream-ordered workspace, encode
-// the tensor maps, launch the persistent grid.  Also the tile-major tap layout of SURVEY 8f N2 (sstem_taps_to_tiled,
-// sstem_sepconv_forward_tiled).
+// the tensor maps, launch the persistent grid.  Also the forward on the tile-major tap layout of SURVEY 8f N2
+// (sstem_sepconv_forward_tiled; the layout conversion sstem_taps_to_tiled is in sepconv_layout.cu).
 #include "sepconv_k51_v3.cuh"
 
 #include <stdlib.h>
@@ -27,15 +27,7 @@ int launch_fwd_v3(const float* in, const float* v, const float* h, float* out,
     if (workspace_alloc(reinterpret_cast<void**>(&ws), ws_bytes + 256, s)) return -1000;
     int* counter = reinterpret_cast<int*>(reinterpret_cast<char*>(ws) + ws_bytes);   // dynamic tile scheduler ticket
     cudaMemsetAsync(counter, 0, 256, s);
-    int e = 0;
-    if (CC == 3) e = launch_repack_nhwc4(in, ws, B, C, c0, IH, IW, s);
-    else {
-        const int64_t total = B * IH * IWP;
-        const unsigned blocks = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)sm_count() * 16);
-        repack_plane_pitch_kernel<<<blocks, 256, 0, s>>>(in, ws, C, c0, (int)IH, (int)IW, (int)IWP, total, g_gate.ptr, g_gate.want);
-        count_launch();
-        e = finish_launch();
-    }
+    int e = CC == 3 ? launch_repack_nhwc4(in, ws, B, C, c0, IH, IW, s) : launch_repack_plane_pitch(in, ws, B, C, c0, IH, IW, IWP, s);
     CUtensorMap min, mv, mh;
     if (!e) {
         const int64_t row = CC == 3 ? 4 * IW : IWP;
@@ -68,62 +60,16 @@ int launch_fwd_v3(const float* in, const float* v, const float* h, float* out,
     return e;
 }
 
-bool fwd_gen3_enabled() {
-    static const int gen = getenv("SSTEM_FWD_GEN") ? atoi(getenv("SSTEM_FWD_GEN")) : 3;   // experiments: force generation 1
-    return gen >= 3;
-}
-
 }  // namespace
 
 int try_launch_fwd_k51_v3(const float* in, const float* v, const float* h, float* out,
                           int64_t B, int C, int c0, int H, int W, cudaStream_t s) {
-    if (!fwd_gen3_enabled()) return -1000;
     return launch_fwd_v3<3, false>(in, v, h, out, B, C, c0, H, W, 1, false, s);
-}
-
-// one channel (plane c0), written to `replicas` consecutive output planes (gray x3 shortcut: replicas = C)
-int try_launch_fwd_k51_v3_c1(const float* in, const float* v, const float* h, float* out,
-                             int64_t B, int C, int c0, int H, int W, int replicas, cudaStream_t s) {
-    // Measured (16x3x512^2 gray x3): generation 1 0.700 ms, this kernel 0.718 ms on [B,51,H,W] taps and 0.685 ms on tile-major
-    // taps -- at one channel a step has only 56 FFMA2 to hide its 21 LDS and the ring bookkeeping behind, so the
-    // persistent kernel pays off only with the cheaper tiled tap delivery.  Kept selectable for experiments.
-    static const bool on = getenv("SSTEM_FWD_C1_GEN") && atoi(getenv("SSTEM_FWD_C1_GEN")) >= 3;
-    if (!on || !fwd_gen3_enabled()) return -1000;
-    return launch_fwd_v3<1, false>(in, v, h, out, B, C, c0, H, W, replicas, false, s);
-}
-
-int launch_planes_equal(const float* in, int64_t B, int64_t C, int64_t plane, int* flag, cudaStream_t s) {
-    cudaError_t e = cudaMemsetAsync(flag, 1, sizeof(int), s);      // non-zero = "identical planes" until a mismatch clears it
-    if (e != cudaSuccess) return (int)e;
-    const int64_t total = B * plane;
-    const unsigned blocks = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)sm_count() * 16);
-    planes_equal_kernel<<<blocks, 256, 0, s>>>(in, (int)C, plane, total, flag);
-    count_launch();
-    return finish_launch();
 }
 
 }  // namespace sstem
 
 using namespace sstem;
-
-// ---- tile-major taps (SURVEY 8f N2) ---------------------------------------------------------------------------------
-extern "C" int64_t sstem_taps_tiled_elems(int64_t B, int64_t H, int64_t W) {
-    if (B <= 0 || H <= 0 || W <= 0) return 0;
-    return B * ((H + 7) / 8) * ((W + 7) / 8) * K51 * 64;
-}
-
-extern "C" int sstem_taps_to_tiled(const float* taps, float* tiled, int64_t B, int64_t H, int64_t W, void* stream) {
-    if (!taps || !tiled) return SSTEM_E_NULL;
-    if (B <= 0 || H <= 0 || W <= 0 || H > (1 << 24) || W > (1 << 24)) return SSTEM_E_SHAPE;
-    if (!aligned4(taps) || !aligned16(tiled)) return SSTEM_E_ALIGN;
-    DeviceGuard guard(tiled);
-    if (guard.err) return guard.err;
-    const int64_t total = sstem_taps_tiled_elems(B, H, W);
-    const unsigned blocks = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)sm_count() * 32);
-    taps_to_tiled_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(taps, tiled, (int)H, (int)W, (int)((H + 7) / 8), (int)((W + 7) / 8), total);
-    count_launch();
-    return finish_launch();
-}
 
 extern "C" int sstem_sepconv_forward_tiled(const float* input, const float* vertical_tiled, const float* horizontal_tiled,
                                            float* output, int64_t B, int64_t C, int64_t H, int64_t W,

@@ -1,15 +1,17 @@
 // Third-generation tap-gradient kernel: persistent warps fed entirely by TMA.
 //
-// Measured on the second generation (sepconv_k51_v2.cuh; ncu, profiles/): with the window and the vertical taps of a
-// tile arriving as two big TMA boxes the step loop itself became 15 % faster, but the tile's prologue -- waiting for
-// ~130 KB per tile to cross the SM's L2 port, then for the horizontal taps -- grew to 16 % of all warp time, because a
-// CTA cannot prefetch its next tile and only one other CTA is there to cover.  Here nothing waits:
+// Measured on a second generation (CTA per tile, removed; DESIGN §4.1 and §7): with the window and the vertical taps
+// of a tile arriving as two big TMA boxes the step loop itself became 15 % faster, but the tile's prologue -- waiting
+// for ~130 KB per tile to cross the SM's L2 port, then for the horizontal taps -- grew to 16 % of all warp time,
+// because a CTA cannot prefetch its next tile and only one other CTA is there to cover.  Here nothing waits:
 //
 //   * a WARP, not a CTA, owns a tile (8 columns x 4 rows) and walks a sequence of tiles (persistent grid, two
 //     4-warp CTAs per SM); warps never synchronise with each other, so they drift apart and cover each other's
 //     tile switches;
 //   * the window streams through a 3-slot ring in groups of 4 input rows: one TMA box {4 channels, 60 columns, 4 rows}
-//     of the channel-interleaved input (see v2) plus one box {8 columns, 4 rows, 4 planes} of vertical taps per group,
+//     of the input repacked channel-interleaved, [B][H+50][W+50][4] with the 4th lane zero (sepconv_layout.cu: its
+//     rows are 16-byte multiples and a lane reads all three channels of a tap with one LDS.128), plus one box
+//     {8 columns, 4 rows, 4 planes} of vertical taps per group,
 //     requested two groups (8 steps) ahead by lane 0, completion on the slot's mbarrier.  A step's vertical taps sit
 //     in the current or the previous group's slot at compile-time offsets; tap planes outside 0..50 and pixels
 //     outside the image are zero-filled by the TMA unit;
@@ -20,7 +22,8 @@
 // ring costs ~10 instructions per 4 steps.  The forward's operation order is that of generation 1 (bit-identical
 // results); grad_vertical sums its 13 tap terms in one chain instead of two (same tolerance against the oracle).
 #pragma once
-#include "sepconv_k51_v2.cuh"
+#include "sepconv_k51.cuh"
+#include "tma.cuh"
 #include <type_traits>
 
 namespace sstem {
@@ -30,11 +33,13 @@ constexpr int V3_COLS = 8;                                   // columns per warp
 constexpr int V3_WIN_COLS = 60;                              // 8 + 52 tap slots
 constexpr int V3_GROUP = 4;                                  // input rows per ring slot
 constexpr int V3_NGROUPS = 14;                               // 56 >= 54 input rows per tile
+constexpr int B3_R = 4;                                      // rows per warp tile of the tap-gradient kernel
+constexpr int B3_ROWS = B3_R + K51 - 1;                      // 54 input rows per tile
 constexpr unsigned V3_WIN_BYTES = V3_GROUP * V3_WIN_COLS * 16;   // 3840
-constexpr unsigned V3_V_BYTES = V3_GROUP * V2_R * V3_COLS * 4;   // 512: [plane][row][col]
+constexpr unsigned V3_V_BYTES = V3_GROUP * B3_R * V3_COLS * 4;   // 512: [plane][row][col]
 constexpr unsigned V3_SLOT_BYTES = V3_WIN_BYTES + V3_V_BYTES;    // 4352 = 34 * 128
-constexpr unsigned V3_H_BYTES = K51 * V2_R * V3_COLS * 4;        // 6528: [tap][row][col]
-constexpr unsigned V3_G_BYTES = 3 * V2_R * V3_COLS * 4;          // 384:  [channel][row][col]
+constexpr unsigned V3_H_BYTES = K51 * B3_R * V3_COLS * 4;        // 6528: [tap][row][col]
+constexpr unsigned V3_G_BYTES = 3 * B3_R * V3_COLS * 4;          // 384:  [channel][row][col]
 constexpr unsigned V3_OFF_H = 3 * V3_SLOT_BYTES;                 // 13056
 constexpr unsigned V3_OFF_G = V3_OFF_H + V3_H_BYTES;             // 19584
 constexpr unsigned V3_OFF_BAR = V3_OFF_G + V3_G_BYTES;           // 19968: full[3], hbar
@@ -62,11 +67,6 @@ __device__ __forceinline__ void mbar_wait_a(unsigned bar_addr, unsigned parity) 
 // pushed out by the 1.7 GB of taps streaming past it.  The taps keep the normal policy: a warp tile reads 32 bytes of
 // each 64-byte DRAM sector and its neighbour the other half -- marked evict-first the sector was often gone before
 // the neighbour asked (measured: +0.5 GB of DRAM reads per launch).
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
 __device__ __forceinline__ uint64_t l2_policy_evict_normal() {
     uint64_t p;
     asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
@@ -112,14 +112,9 @@ __device__ __forceinline__ float4 lds_f32x4(unsigned addr) {
     return v;
 }
 
-#ifndef SSTEM_V3_REREAD
-#define SSTEM_V3_REREAD 1
-#endif
-#ifndef SSTEM_BWD3_SPLIT
-#define SSTEM_BWD3_SPLIT 0                                 // 1: two gv partial sums per row pair (generation 1's operation order);
-                                                           // one chain measured 0.8 % faster here (4 fewer FADD per step)
-#endif
-// One input row; same arithmetic as bwd2_step, operands addressed by shared-memory byte addresses:
+// One input row: per tap slot t and row pair, t2 = sum_c g_c P_c, then gh += t2 v and gv += t2 h.  gv sums its 13 tap
+// terms in one chain (generation 1 uses two partial sums; one chain measured 0.8 % faster here, 4 fewer FADD per step).
+// Operands are addressed by shared-memory byte addresses:
 //   pa            window row of this step, already offset to the lane's first tap column
 //   va[p]         address of v[fy = s - p][row p][column of the lane]   (only read when the row is active)
 template <int S, bool WV, bool WH>
@@ -136,9 +131,8 @@ __device__ __forceinline__ void bwd3_step(unsigned pa, unsigned pa_last, const u
         v2[pp].x = (WH && a_ok) ? lds_f32(va[2 * pp]) : 0.f;
         v2[pp].y = (WH && b_ok) ? lds_f32(va[2 * pp + 1]) : 0.f;
     }
-    float2 gva[NP], gvb[NP];
 #pragma unroll
-    for (int pp = 0; pp < NP; ++pp) gva[pp] = gvb[pp] = make_float2(0.f, 0.f);
+    for (int pp = 0; pp < NP; ++pp) gvp[pp] = make_float2(0.f, 0.f);
     float2 t2[NT][NP];
     float4 P[NT];
 #pragma unroll
@@ -164,14 +158,8 @@ __device__ __forceinline__ void bwd3_step(unsigned pa, unsigned pa_last, const u
                 if (S - 2 * pp - 1 < 0) t2[t][pp].y = 0.f;
             }
             if (WH) gh2[pp][t] = __ffma2_rn(t2[t][pp], v2[pp], gh2[pp][t]);
-            if (WV) {
-                if (SSTEM_BWD3_SPLIT && (t & 1)) gvb[pp] = __ffma2_rn(t2[t][pp], h2[pp][t], gvb[pp]);
-                else gva[pp] = __ffma2_rn(t2[t][pp], h2[pp][t], gva[pp]);
-            }
+            if (WV) gvp[pp] = __ffma2_rn(t2[t][pp], h2[pp][t], gvp[pp]);
         }
-#pragma unroll
-    for (int pp = 0; pp < NP; ++pp)
-        gvp[pp] = SSTEM_BWD3_SPLIT ? make_float2(gva[pp].x + gvb[pp].x, gva[pp].y + gvb[pp].y) : gva[pp];
 }
 
 #ifndef SSTEM_BWD3_MINB
@@ -258,7 +246,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
     issue_group(s_nxt, b_nxt, tb, ty0, tx0, 1);
 
     const unsigned lane_win = (unsigned)(pg + g) * 16u;    // lane's first tap column inside a window row
-    const unsigned lane_last = lane_win + ((novalid && SSTEM_V3_REREAD) ? 11u : 12u) * 64u;   // its slot 12 (g == 3: tap 47 again, see the h copy)
+    const unsigned lane_last = lane_win + (novalid ? 11u : 12u) * 64u;   // its slot 12 (g == 3: tap 47 again, see the h copy)
     const unsigned lane_v = V3_WIN_BYTES + (unsigned)pg * 4u;
 
 #pragma unroll 1
@@ -321,7 +309,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
         auto run_step = [&](auto gi_tag, auto u_tag, int gi, unsigned wa, unsigned wl, unsigned vc, unsigned vp) {
             constexpr int GI = decltype(gi_tag)::value, U = decltype(u_tag)::value;
             constexpr int S = GI < 0 ? -1 : GI * V3_GROUP + U;            // compile-time step of the partial groups
-            if (GI >= 0 && GI * V3_GROUP + U >= V2_WIN_H) return;         // rows 54, 55 of the last group: nothing to do
+            if (GI >= 0 && GI * V3_GROUP + U >= B3_ROWS) return;          // rows 54, 55 of the last group: nothing to do
             unsigned va[4];
 #pragma unroll
             for (int p = 0; p < 4; ++p)                    // plane s - p: this group's slot or the previous one's

@@ -53,14 +53,15 @@ def test_tiled_forward_bit_identical_at_training_size_and_gray():
     general = pkg.SeparableConvolution.apply(gray, v, h)
     pkg.set_gray_replicated("assert")
     try:
-        assert torch.equal(pkg.SeparableConvolution.apply(gray, v, h), general)          # persistent one-channel kernel
-        assert torch.equal(pkg.sepconv_forward_tiled(gray, vt, ht), general)
+        assert torch.equal(pkg.SeparableConvolution.apply(gray, v, h), general)          # generation 1, one channel
+        assert torch.equal(pkg.sepconv_forward_tiled(gray, vt, ht), general)             # persistent one-channel kernel
     finally:
         pkg.set_gray_replicated("off")
 
 
 def test_one_channel_persistent_kernel_vs_oracle_order():
-    """C = 1 at a size that takes the persistent kernel: exact gather with one-hot taps + linearity-free oracle check on a crop."""
+    """C = 1 at 2x1024^2 on [B,51,H,W] taps (generation 1: the persistent one-channel kernel runs on tile-major taps only):
+    exact gather with one-hot taps + linearity-free oracle check on a crop."""
     dev = "cuda"
     B, H, W = 2, 1024, 1024
     torch.manual_seed(3)
