@@ -37,8 +37,11 @@ bool make_v3_maps(CUtensorMap* min, CUtensorMap* mv, CUtensorMap* mh, CUtensorMa
         if (!make_map_f32(mv, v, 4, tdims, tstrides, box)) return false;
     }
     if (h) {
-        const int box[4] = {V3_COLS, B3_R, K51, 1};
-        if (!make_map_f32(mh, h, 4, tdims, tstrides, box)) return false;
+        // tap and row dimensions swapped: the box lands as [row][tap][col], whose per-lane register copy hits 32 different
+        // banks (as [tap][row][col] the four tap groups of a column collide in one bank)
+        const int64_t rdims[4] = {W, K51, H, B}, rstrides[4] = {1, plane, W, (int64_t)K51 * plane};
+        const int box[4] = {V3_COLS, K51, B3_R, 1};
+        if (!make_map_f32(mh, h, 4, rdims, rstrides, box)) return false;
     }
     {
         const int64_t dims[4] = {W, H, 3, B}, strides[4] = {1, W, plane, C * plane};
@@ -85,3 +88,8 @@ int try_launch_bwd_taps_k51_v3(const float* g, const float* in, const float* v, 
 }
 
 }  // namespace sstem
+
+#ifdef SSTEM_V3_PHASES
+// diagnostic builds only (tools/v3_phases.py): clock64 ticks per tile phase, summed over the warps of every launch
+extern "C" int sstem_v3_phases_bwd(unsigned long long* out, int reset) { return sstem::v3_phases_read(out, reset); }
+#endif

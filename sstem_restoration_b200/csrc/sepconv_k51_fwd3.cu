@@ -35,9 +35,11 @@ int launch_fwd_v3(const float* in, const float* v, const float* h, float* out,
         const int box[3] = {(CC == 3 ? 4 : 1) * V3_WIN_COLS, V3_GROUP, 1};
         if (!make_map_f32(&min, ws, 3, dims, strides, box)) e = -1000;
         if (!e && !TILED) {
+            // h with its tap and row dimensions swapped: the box lands as [row][tap][col] (conflict-free register copy)
             const int64_t tdims[4] = {W, H, K51, B}, tstrides[4] = {1, W, plane, (int64_t)K51 * plane};
-            const int vbox[4] = {V3_COLS, F3_R, V3_GROUP, 1}, hbox[4] = {V3_COLS, F3_R, K51, 1};
-            if (!make_map_f32(&mv, v, 4, tdims, tstrides, vbox) || !make_map_f32(&mh, h, 4, tdims, tstrides, hbox)) e = -1000;
+            const int64_t rdims[4] = {W, K51, H, B}, rstrides[4] = {1, plane, W, (int64_t)K51 * plane};
+            const int vbox[4] = {V3_COLS, F3_R, V3_GROUP, 1}, hbox[4] = {V3_COLS, K51, F3_R, 1};
+            if (!make_map_f32(&mv, v, 4, tdims, tstrides, vbox) || !make_map_f32(&mh, h, 4, rdims, rstrides, hbox)) e = -1000;
         } else if (!e) {
             mv = min;                                      // unused by the kernel, but must be valid objects to copy
             mh = min;
@@ -97,3 +99,8 @@ extern "C" int sstem_sepconv_forward_tiled(const float* input, const float* vert
     }
     return e == -1000 ? SSTEM_E_SHAPE : e;
 }
+
+#ifdef SSTEM_V3_PHASES
+// diagnostic builds only (tools/v3_phases.py): clock64 ticks per tile phase, summed over the warps of every launch
+extern "C" int sstem_v3_phases_fwd(unsigned long long* out, int reset) { return sstem::v3_phases_read(out, reset); }
+#endif

@@ -38,7 +38,7 @@ constexpr int B3_ROWS = B3_R + K51 - 1;                      // 54 input rows pe
 constexpr unsigned V3_WIN_BYTES = V3_GROUP * V3_WIN_COLS * 16;   // 3840
 constexpr unsigned V3_V_BYTES = V3_GROUP * B3_R * V3_COLS * 4;   // 512: [plane][row][col]
 constexpr unsigned V3_SLOT_BYTES = V3_WIN_BYTES + V3_V_BYTES;    // 4352 = 34 * 128
-constexpr unsigned V3_H_BYTES = K51 * B3_R * V3_COLS * 4;        // 6528: [tap][row][col]
+constexpr unsigned V3_H_BYTES = K51 * B3_R * V3_COLS * 4;        // 6528: [row][tap][col]
 constexpr unsigned V3_G_BYTES = 3 * B3_R * V3_COLS * 4;          // 384:  [channel][row][col]
 constexpr unsigned V3_OFF_H = 3 * V3_SLOT_BYTES;                 // 13056
 constexpr unsigned V3_OFF_G = V3_OFF_H + V3_H_BYTES;             // 19584
@@ -111,6 +111,49 @@ __device__ __forceinline__ float4 lds_f32x4(unsigned addr) {
     asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
     return v;
 }
+
+// SSTEM_V3_PHASES (diagnostic builds only, off in the shipped library; tools/v3_phases.py): every warp adds the clock64
+// ticks it spends in each phase of a tile to counters in the unused tail of its barrier block (no extra registers but
+// the last timestamp), and lane 0 adds them to v3_phase_ticks when the warp leaves.  One array per translation unit:
+// the forward's in sepconv_k51_fwd3.cu, the tap gradients' in sepconv_k51_bwd3.cu.
+enum V3Phase { V3P_START, V3P_FIRST, V3P_STEADY, V3P_LAST, V3P_STORE, V3P_BARRIER, V3P_COUNT };
+#ifdef SSTEM_V3_PHASES
+__device__ unsigned long long v3_phase_ticks[V3P_COUNT];
+struct V3PhaseClock {
+    unsigned long long* acc;                               // V3P_COUNT counters in this warp's shared memory
+    long long last;
+    __device__ V3PhaseClock(unsigned char* warp_smem, unsigned off, bool lead) : acc(reinterpret_cast<unsigned long long*>(warp_smem + off)) {
+        if (lead)
+            for (int i = 0; i < V3P_COUNT; ++i) acc[i] = 0;
+        last = clock64();
+    }
+    __device__ __forceinline__ void mark(int phase, bool lead) {
+        const long long now = clock64();
+        if (lead) acc[phase] += (unsigned long long)(now - last);
+        last = now;
+    }
+    __device__ void flush(bool lead) {
+        if (lead)
+            for (int i = 0; i < V3P_COUNT; ++i) atomicAdd(&v3_phase_ticks[i], acc[i]);
+    }
+};
+// copies (and optionally clears) this translation unit's totals; 0 or a CUDA error
+inline int v3_phases_read(unsigned long long* out, int reset) {
+    if (cudaError_t e = cudaMemcpyFromSymbol(out, v3_phase_ticks, sizeof(v3_phase_ticks))) return (int)e;
+    if (reset) {
+        const unsigned long long zero[V3P_COUNT] = {};
+        if (cudaError_t e = cudaMemcpyToSymbol(v3_phase_ticks, zero, sizeof(zero))) return (int)e;
+    }
+    return 0;
+}
+#define V3_PHASE_INIT(warp_smem, off) V3PhaseClock v3_clock(warp_smem, off, lead)
+#define V3_PHASE(p) v3_clock.mark(p, lead)
+#define V3_PHASE_FLUSH() v3_clock.flush(lead)
+#else
+#define V3_PHASE_INIT(warp_smem, off) ((void)0)
+#define V3_PHASE(p) ((void)0)
+#define V3_PHASE_FLUSH() ((void)0)
+#endif
 
 // One input row: per tap slot t and row pair, t2 = sum_c g_c P_c, then gh += t2 v and gv += t2 h.  gv sums its 13 tap
 // terms in one chain (generation 1 uses two partial sums; one chain measured 0.8 % faster here, 4 fewer FADD per step).
@@ -228,7 +271,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
     auto issue_hg = [&](int b, int y0, int x0) {
         if (lead) {
             mbar_expect_tx_a(hbar, (WV ? V3_H_BYTES : 0u) + V3_G_BYTES);
-            if (WV) tma_load_4d_a(base + V3_OFF_H, &map_h, hbar, x0, y0, 0, b, pol_once);
+            if (WV) tma_load_4d_a(base + V3_OFF_H, &map_h, hbar, x0, 0, y0, b, pol_once);   // [row][tap][col]
             tma_load_4d_a(base + V3_OFF_G, &map_g, hbar, x0, y0, 0, b, pol_once);
         }
     };
@@ -248,6 +291,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
     const unsigned lane_win = (unsigned)(pg + g) * 16u;    // lane's first tap column inside a window row
     const unsigned lane_last = lane_win + (novalid ? 11u : 12u) * 64u;   // its slot 12 (g == 3: tap 47 again, see the h copy)
     const unsigned lane_v = V3_WIN_BYTES + (unsigned)pg * 4u;
+    V3_PHASE_INIT(smem_raw + (base - (unsigned)__cvta_generic_to_shared(smem_raw)), V3_OFF_BAR + 32);
 
 #pragma unroll 1
     for (;;) {
@@ -261,6 +305,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
         mbar_wait_a(hbar, p_h);
         p_h ^= 1;
         {
+            // [row][tap][col]: the lanes of one load sit in banks 8 * ((3 * row + g) mod 4) + pg, one wavefront
             const unsigned ha = base + V3_OFF_H + (unsigned)pg * 4u;
 #pragma unroll
             for (int t = 0; t < NT; ++t) {
@@ -268,8 +313,8 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
 #pragma unroll
                 for (int pp = 0; pp < NP; ++pp) {
                     gh2[pp][t] = make_float2(0.f, 0.f);
-                    h2[pp][t] = WV ? make_float2(lds_f32_ordered(ha + ((tap * R + 2 * pp) * V3_COLS) * 4),
-                                                 lds_f32_ordered(ha + ((tap * R + 2 * pp + 1) * V3_COLS) * 4))
+                    h2[pp][t] = WV ? make_float2(lds_f32_ordered(ha + ((2 * pp * K51 + tap) * V3_COLS) * 4),
+                                                 lds_f32_ordered(ha + (((2 * pp + 1) * K51 + tap) * V3_COLS) * 4))
                                    : make_float2(0.f, 0.f);
                     // tap 51 does not exist: its window value is tap 47's (finite whenever the lane's own taps are), its weight 0,
                     // its gh accumulator is never stored
@@ -283,6 +328,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
                 for (int pp = 0; pp < NP; ++pp)
                     g2[c][pp] = make_float2(lds_f32_ordered(ga + ((c * R + 2 * pp) * V3_COLS) * 4), lds_f32_ordered(ga + ((c * R + 2 * pp + 1) * V3_COLS) * 4));
         }
+        V3_PHASE(V3P_START);
         // The two buffers are refilled (next tile's taps) only after the first group below: they may be overwritten once
         // every lane's copy has ARRIVED in registers, not merely been issued -- the 64 loads queue behind the other warps'
         // shared-memory traffic, and a TMA write issued right here overtook them now and then (grad_vertical wrong in
@@ -336,15 +382,18 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
         run_group(std::integral_constant<int, 0>{}, 0);
         end_group(false, 2);
         if (has_next) issue_hg(nb, ny0, nx0);              // see above: h2 / g2 are in registers for sure by now
+        V3_PHASE(V3P_FIRST);
 #pragma unroll 1
         for (int gi = 1; gi < 12; ++gi) {                  // groups 1..11 = steps 4..47: every row active
             run_group(std::integral_constant<int, -1>{}, gi);
             end_group(false, gi + 2);
         }
+        V3_PHASE(V3P_STEADY);
         run_group(std::integral_constant<int, 12>{}, 12);  // steps 48..51
         end_group(true, 0);
         run_group(std::integral_constant<int, 13>{}, 13);  // steps 52, 53 (+ two rows nobody needs)
         end_group(true, 1);
+        V3_PHASE(V3P_LAST);
 
         // ---- gh: complete per lane (the sum over fy happened in registers)
         if (WH && col_ok) {
@@ -362,12 +411,15 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
                 }
             }
         }
+        V3_PHASE(V3P_STORE);
         if (!has_next) break;
         asm volatile("bar.sync 1, %0;" ::"n"(V3_WARPS * 32) : "memory");   // the CTA moves to its next tile together
         tile = ntile; tb = nb; ty0 = ny0; tx0 = nx0;
         ntile = 2 * nctas + *reinterpret_cast<volatile int*>(&s_ticket[tile_no & 1]);
         ++tile_no;
+        V3_PHASE(V3P_BARRIER);
     }
+    V3_PHASE_FLUSH();
 }
 
 // =====================================================================================================================
@@ -381,7 +433,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
 constexpr int F3_R = 8;
 constexpr int F3_ROWS = F3_R + K51 - 1;                          // 58
 constexpr unsigned F3_V_BYTES = V3_GROUP * F3_R * V3_COLS * 4;   // 1024: [plane][row][col]
-constexpr unsigned F3_H_BYTES = K51 * F3_R * V3_COLS * 4;        // 13056
+constexpr unsigned F3_H_BYTES = K51 * F3_R * V3_COLS * 4;        // 13056: [row][tap][col] ([tap][row][col] when TILED)
 constexpr unsigned F3_OFF_V = 2 * V3_WIN_BYTES;                  // 7680
 constexpr unsigned F3_OFF_H = F3_OFF_V + 4 * F3_V_BYTES;         // 11776
 constexpr unsigned F3_OFF_BAR = F3_OFF_H + F3_H_BYTES;           // 24832
@@ -504,7 +556,7 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
     auto issue_h = [&](int b, int y0, int x0) {
         if (lead) {
             mbar_expect_tx_a(hbar, F3_H_BYTES);
-            if (!TILED) tma_load_4d_a(base + F3_OFF_H, &map_h, hbar, x0, y0, 0, b, pol_once);
+            if (!TILED) tma_load_4d_a(base + F3_OFF_H, &map_h, hbar, x0, 0, y0, b, pol_once);   // [row][tap][col]
             else bulk_load_a(base + F3_OFF_H, tl.h + (((int64_t)b * tl.tiles_y8 + y0 / F3_R) * tl.tiles_x8 + x0 / V3_COLS) * (K51 * 64),
                              F3_H_BYTES, hbar);
         }
@@ -521,6 +573,7 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
     const unsigned lane_win = (unsigned)(pg + g) * PIX;
     const unsigned lane_last = lane_win + (novalid ? 11u : 12u) * 4u * PIX;
     const unsigned lane_v = (unsigned)pg * 4u;
+    V3_PHASE_INIT(smem_raw + (base - (unsigned)__cvta_generic_to_shared(smem_raw)), F3_OFF_BAR + 32);
 
 #pragma unroll 1
     for (;;) {
@@ -533,13 +586,16 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
         mbar_wait_a(hbar, p_h);
         p_h ^= 1;
         {
+            // NCHW taps land as [row][tap][col] (banks 8 * ((3 * row + g) mod 4) + pg: one wavefront per load); the tile-major
+            // layout is [tap][row][col], an external format (its loads are 4-way bank conflicts)
             const unsigned ha = base + F3_OFF_H + (unsigned)pg * 4u;
+            auto h_word = [](int row, int tap) { return TILED ? tap * R + row : row * K51 + tap; };
 #pragma unroll
             for (int t = 0; t < NT; ++t) {
                 const int tap = (t == NT - 1 && novalid) ? (G * (NT - 2) + g) : (G * t + g);
 #pragma unroll
                 for (int pp = 0; pp < NP; ++pp) {
-                    h2[pp][t] = make_float2(lds_f32_ordered(ha + ((tap * R + 2 * pp) * V3_COLS) * 4), lds_f32_ordered(ha + ((tap * R + 2 * pp + 1) * V3_COLS) * 4));
+                    h2[pp][t] = make_float2(lds_f32_ordered(ha + (h_word(2 * pp, tap) * V3_COLS) * 4), lds_f32_ordered(ha + (h_word(2 * pp + 1, tap) * V3_COLS) * 4));
                     if (t == NT - 1 && novalid) h2[pp][t] = make_float2(0.f, 0.f);   // tap 51 does not exist: weight 0 on tap 47's column
                 }
             }
@@ -548,6 +604,7 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
         for (int c = 0; c < CC; ++c)
 #pragma unroll
             for (int pp = 0; pp < NP; ++pp) acc[c][pp] = make_float2(0.f, 0.f);
+        V3_PHASE(V3P_START);
         // (the tap buffer is refilled after the second group: see the tap-gradient kernel)
 
         auto run_step = [&](auto gi_tag, auto u_tag, unsigned wa, unsigned wl, unsigned vc, unsigned vp1, unsigned vp2) {
@@ -590,17 +647,20 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
         run_group(std::integral_constant<int, 1>{});
         end_group(false, 3);
         if (has_next) issue_h(nb, ny0, nx0);               // all 8 rows have used their taps by step 7
+        V3_PHASE(V3P_FIRST);
 #pragma unroll 1
         for (int gi = 2; gi < 12; ++gi) {                  // groups 2..11 = steps 8..47: every row active
             run_group(std::integral_constant<int, -1>{});
             end_group(false, gi + 2);
         }
+        V3_PHASE(V3P_STEADY);
         run_group(std::integral_constant<int, 12>{});      // steps 48..51
         end_group(false, 14);
         run_group(std::integral_constant<int, 13>{});      // steps 52..55
         end_group(true, 0);
         run_group(std::integral_constant<int, 14>{});      // steps 56, 57
         end_group(true, 1);
+        V3_PHASE(V3P_LAST);
 
         // ---- sum the 4 tap groups of each pixel: lane g ends up with rows 2g, 2g+1 of every channel
         const int x = tx0 + pg;
@@ -624,12 +684,15 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
                 }
             }
         }
+        V3_PHASE(V3P_STORE);
         if (!has_next) break;
         asm volatile("bar.sync 1, %0;" ::"n"(V3_WARPS * 32) : "memory");   // the CTA moves to its next tile together
         tile = ntile; tb = nb; ty0 = ny0; tx0 = nx0;
         ntile = 2 * nctas + *reinterpret_cast<volatile int*>(&s_ticket[tile_no & 1]);
         ++tile_no;
+        V3_PHASE(V3P_BARRIER);
     }
+    V3_PHASE_FLUSH();
 }
 
 }  // namespace
