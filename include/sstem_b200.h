@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define SSTEM_ABI_VERSION 3
+#define SSTEM_ABI_VERSION 4
 
 /* argument errors (negative) */
 #define SSTEM_E_NULL      (-1)  /* a required pointer is NULL */
@@ -289,6 +289,25 @@ int sstem_taps_to_tiled(const float* taps, float* tiled, int64_t B, int64_t H, i
 int sstem_sepconv_forward_tiled(const float* input, const float* vertical_tiled, const float* horizontal_tiled,
                                 float* output, int64_t B, int64_t C, int64_t H, int64_t W,
                                 int32_t K, uint32_t flags, void* stream);
+
+/*
+ * Gradients of sstem_sepconv_forward_tiled given grad_output [B,C,H,W] (NCHW, as the forward's output).
+ *   grad_vertical_tiled / grad_horizontal_tiled: tile-major like the taps, EVERY element written; entries outside the
+ *     image are 0 (the forward never reads them)
+ *   grad_input [B,C,H+50,W+50] or NULL (computed as sstem_sepconv_backward does; not a tuned path here: the taps are
+ *     converted back to [B,51,H,W] in a stream-ordered workspace, 2 x 204 B per pixel, ~816 B per pixel of traffic)
+ * Any of the three outputs may be NULL; K must be 51; flags: SSTEM_SEPCONV_GRAY_REPLICATED (same meaning as for
+ * sstem_sepconv_backward: t = (sum_c g_c) * in_0).  Tiled pointers 16-byte aligned (SSTEM_E_ALIGN otherwise).
+ * With [B,51,H,W] taps that run the same (third-generation) kernel, the tap gradients are bit-identical to
+ * sstem_sepconv_backward's.
+ */
+int sstem_sepconv_backward_tiled(const float* grad_output, const float* input,
+                                 const float* vertical_tiled, const float* horizontal_tiled,
+                                 float* grad_input, float* grad_vertical_tiled, float* grad_horizontal_tiled,
+                                 int64_t B, int64_t C, int64_t H, int64_t W, int32_t K, uint32_t flags, void* stream);
+
+/* inverse of sstem_taps_to_tiled: tile-major -> [B,51,H,W] (the padding entries are ignored) */
+int sstem_taps_from_tiled(const float* tiled, float* taps, int64_t B, int64_t H, int64_t W, void* stream);
 
 /*
  * The one-plane frame the interpolation tail convolves when its taps are tile-major (mean_c sepconv(i_c) = sepconv(mean_c i_c);

@@ -16,7 +16,7 @@ from ._lib import SstemError, launch_count, fp32_peak_probe  # noqa: F401
 from .sepconv import (  # noqa: F401
     SeparableConvolution, FunctionSepconv, ModuleSepconv, set_strict_order, set_gray_replicated,
     interpolation_tail, ModuleInterpolationTail, taps_to_tiled, sepconv_forward_tiled,
-    interpolation_tail_tiled, frame_mean_pad,
+    interpolation_tail_tiled, frame_mean_pad, taps_from_tiled, SeparableConvolutionTiled, ModuleInterpolationTailTiled,
 )
 from .warp import SpatialTransformation, image_warp  # noqa: F401
 from .host import sepconv_forward_backward_host, join_host_pipeline  # noqa: F401
@@ -28,6 +28,7 @@ from . import shard, synth, sff_sim  # noqa: F401
 __all__ = [
     "SeparableConvolution", "FunctionSepconv", "ModuleSepconv", "set_strict_order", "set_gray_replicated",
     "interpolation_tail", "ModuleInterpolationTail", "taps_to_tiled", "sepconv_forward_tiled", "interpolation_tail_tiled", "frame_mean_pad",
+    "taps_from_tiled", "SeparableConvolutionTiled", "ModuleInterpolationTailTiled",
     "SpatialTransformation", "image_warp", "sepconv_forward_backward_host", "join_host_pipeline", "SstemError", "launch_count", "fp32_peak_probe",
     "sections_to_input", "prediction_to_uint8", "restore_stack", "warp_stitch", "warp_and_stitch",
     "tap_conv3x3", "pack_tap_conv_weight", "ModuleTapProducer", "shard", "synth", "sff_sim",

@@ -13,7 +13,7 @@ import threading
 from ._build import LIB_PATH as _DEFAULT_LIB_PATH, needs_build as _needs_build
 
 #: must equal SSTEM_ABI_VERSION of include/sstem_b200.h (checked against the loaded library in load())
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 #: SSTEM_LIB_PATH selects another build of the same library (kernel-tuning experiments)
 LIB_PATH = os.environ.get("SSTEM_LIB_PATH") or _DEFAULT_LIB_PATH
@@ -42,6 +42,7 @@ EXPORTED_SYMBOLS = (
     "sstem_warp_forward", "sstem_warp_backward", "sstem_image_warp", "sstem_sff_degrade", "sstem_sff_contrast",
     "sstem_sections_to_input", "sstem_prediction_to_u8", "sstem_warp_stitch_u8", "sstem_warp_stitch_forward",
     "sstem_taps_tiled_elems", "sstem_taps_to_tiled", "sstem_sepconv_forward_tiled", "sstem_frame_mean_pad",
+    "sstem_sepconv_backward_tiled", "sstem_taps_from_tiled",
     "sstem_sepconv_forward_detect", "sstem_sepconv_backward_detect",
     "sstem_tap_conv3x3_packed_elems", "sstem_tap_conv3x3_pack_weights", "sstem_tap_conv3x3",
     "sstem_fp32_peak_probe", "sstem_launch_count", "sstem_abi_version", "sstem_error_string",
@@ -100,6 +101,10 @@ def load() -> ctypes.CDLL:
         lib.sstem_taps_to_tiled.restype = ctypes.c_int
         lib.sstem_sepconv_forward_tiled.argtypes = [_c_p, _c_p, _c_p, _c_p, _c_i64, _c_i64, _c_i64, _c_i64, _c_i32, _c_u32, _c_p]
         lib.sstem_sepconv_forward_tiled.restype = ctypes.c_int
+        lib.sstem_sepconv_backward_tiled.argtypes = [_c_p] * 7 + [_c_i64] * 4 + [_c_i32, _c_u32, _c_p]
+        lib.sstem_sepconv_backward_tiled.restype = ctypes.c_int
+        lib.sstem_taps_from_tiled.argtypes = [_c_p, _c_p, _c_i64, _c_i64, _c_i64, _c_p]
+        lib.sstem_taps_from_tiled.restype = ctypes.c_int
         lib.sstem_frame_mean_pad.argtypes = [_c_p, _c_i64, _c_p, _c_i64, _c_i64, _c_i64, _c_i64, _c_i32, _c_u32, _c_p]
         lib.sstem_frame_mean_pad.restype = ctypes.c_int
         lib.sstem_sepconv_forward_detect.argtypes = [_c_p, _c_p, _c_p, _c_p, _c_i64, _c_i64, _c_i64, _c_i64, _c_i32, _c_u32, _c_p, _c_p]

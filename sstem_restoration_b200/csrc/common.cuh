@@ -105,5 +105,11 @@ int launch_repack_nhwc4(const float* in, float* ws, int64_t B, int C, int c0, in
 int launch_repack_plane_pitch(const float* in, float* ws, int64_t B, int C, int c0, int64_t IH, int64_t IW, int64_t IWP,
                               cudaStream_t s);
 int launch_planes_equal(const float* in, int64_t B, int64_t C, int64_t plane, int* flag, cudaStream_t s);
+// grad_output [B,C,H,W] -> out [B,nplanes,H,WP] (WP >= W a multiple of 4, zero pad columns): all C planes, or with `sum`
+// their channel sum as one plane
+int launch_stage_grad_planes(const float* g, float* out, int64_t B, int64_t C, int64_t H, int64_t W, int64_t WP, bool sum,
+                             cudaStream_t s);
+// tile-major taps -> [B,51,H,W]
+int launch_taps_from_tiled(const float* tiled, float* taps, int64_t B, int64_t H, int64_t W, cudaStream_t s);
 
 }  // namespace sstem

@@ -160,9 +160,11 @@ inline int v3_phases_read(unsigned long long* out, int reset) {
 // Operands are addressed by shared-memory byte addresses:
 //   pa            window row of this step, already offset to the lane's first tap column
 //   va[p]         address of v[fy = s - p][row p][column of the lane]   (only read when the row is active)
-template <int S, bool WV, bool WH>
+// CC = 3: channel-interleaved window, one LDS.128 per tap; CC = 1: one plane at a 16-byte row pitch, one LDS.32 per tap
+// and t2 = P g (26 products instead of 78 FFMA2).
+template <int S, bool WV, bool WH, int CC>
 __device__ __forceinline__ void bwd3_step(unsigned pa, unsigned pa_last, const unsigned (&va)[4],
-                                          const float2 (&g2)[3][2], const float2 (&h2)[2][13],
+                                          const float2 (&g2)[CC][2], const float2 (&h2)[2][13],
                                           float2 (&gh2)[2][13], float2 (&gvp)[2]) {
     constexpr int NP = 2, NT = 13;
     float2 v2[NP];
@@ -179,10 +181,12 @@ __device__ __forceinline__ void bwd3_step(unsigned pa, unsigned pa_last, const u
     float2 t2[NT][NP];
     float4 P[NT];
 #pragma unroll
-    for (int t = 0; t < NT; ++t)                           // channels x, y, z of column x + g + 4t; slot 12 of the lanes
-        P[t] = lds_f32x4(t == NT - 1 ? pa_last : pa + 64 * t);   // g == 3 (tap 51 does not exist) rereads tap 47, h = 0 there
+    for (int t = 0; t < NT; ++t) {                         // channels x, y, z of column x + g + 4t; slot 12 of the lanes
+        const unsigned a = t == NT - 1 ? pa_last : pa + (CC == 3 ? 64 : 16) * t;   // g == 3 (tap 51 does not exist) rereads
+        P[t] = CC == 3 ? lds_f32x4(a) : make_float4(lds_f32(a), 0.f, 0.f, 0.f);   // tap 47, h = 0 there
+    }
 #pragma unroll
-    for (int c = 0; c < 3; ++c)
+    for (int c = 0; c < CC; ++c)
 #pragma unroll
         for (int t = 0; t < NT; ++t)
 #pragma unroll
@@ -205,17 +209,32 @@ __device__ __forceinline__ void bwd3_step(unsigned pa, unsigned pa_last, const u
         }
 }
 
+__device__ __forceinline__ void tma_load_5d_a(unsigned dst, const CUtensorMap* map, unsigned bar, int c0, int c1, int c2, int c3,
+                                              int c4, uint64_t policy) {
+    asm volatile(
+        "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5, %6, %7}], [%2], %8;"
+        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "l"(policy) : "memory");
+}
+
 #ifndef SSTEM_BWD3_MINB
 #define SSTEM_BWD3_MINB 2
 #endif
-template <bool WV, bool WH, bool ACCUM>
-__global__ void __launch_bounds__(V3_WARPS * 32, SSTEM_BWD3_MINB)
-sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_constant__ CUtensorMap map_v,
-                               const __grid_constant__ CUtensorMap map_h, const __grid_constant__ CUtensorMap map_g,
-                               float* __restrict__ gv, float* __restrict__ gh, int* __restrict__ next_tile_counter,
-                               const V3Shape sh, const int* gate, int gate_want) {
+// The tap-gradient kernels' body.  CC = 3: channel-interleaved window [B][H+50][W+50][4], upstream gradient box
+// {8 columns, 4 rows, 3 channels}; CC = 1: one plane copied to a 16-byte row pitch, one gradient plane (the gray x3
+// shortcut with the channel-summed gradient, single remainder planes, the one-plane frames of the tiled tail).
+// TILED: the taps and their gradients are tile-major [B][H/8][W/8][51][8][8] (sstem_taps_to_tiled).  A warp tile is half
+// of an 8x8 tile; map_v / map_h are 5-D maps over that layout that land exactly as the [B,51,H,W] maps do
+// ([plane][row][col] and [row][tap][col]), so only the coordinates and the stores differ.  Every element of a tile inside
+// the tensor is written, entries outside the image as explicit zeros (g is zero there but the window may hold Inf).
+template <bool WV, bool WH, bool ACCUM, int CC, bool TILED>
+__device__ __forceinline__ void bwd3_taps_body(const CUtensorMap& map_in, const CUtensorMap& map_v, const CUtensorMap& map_h,
+                                               const CUtensorMap& map_g, float* __restrict__ gv, float* __restrict__ gh,
+                                               int* __restrict__ next_tile_counter, const V3Shape& sh, const int* gate, int gate_want) {
     SSTEM_GATE_RETURN(gate, gate_want);
     constexpr int G = 4, R = 4, NP = 2, NT = 13;
+    constexpr unsigned WIN_BYTES = CC == 3 ? V3_WIN_BYTES : V3_WIN_BYTES / 4;   // 4 rows x 60 pixels x (16 | 4) bytes
+    constexpr unsigned PIX = CC == 3 ? 16u : 4u;
+    constexpr unsigned G_BYTES = CC * B3_R * V3_COLS * 4;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     // the shuffle tells the compiler that `warp` -- and with it every ring / barrier address and TMA coordinate below --
     // is warp-uniform, so those live in uniform registers and a TMA issue needs no R2UR moves
@@ -251,6 +270,8 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
     const uint64_t pol_once = l2_policy_evict_normal(), pol_keep = l2_policy_evict_last();
 
     const int64_t plane = (int64_t)sh.H * sh.W;
+    // TILED: 8x8 tiles per row / column of the tile-major tensors (the row tiles of sh.tiles_y are half tiles)
+    const int tiles_x8 = TILED ? (sh.W + 7) >> 3 : 0, tiles_y8 = TILED ? (sh.H + 7) >> 3 : 0;
     auto decode = [&](int t, int& b, int& y0, int& x0) {
         const int tx = t % sh.tiles_x, r = t / sh.tiles_x;
         x0 = (tx * V3_WARPS + warp) * V3_COLS;
@@ -263,15 +284,23 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
     unsigned p_cur = 0, p_nxt = 0, p_prv = 0, p_h = 0;
     auto issue_group = [&](unsigned slot, unsigned bar, int b, int y0, int x0, int gi) {
         if (lead) {
-            mbar_expect_tx_a(bar, V3_WIN_BYTES + (WH ? V3_V_BYTES : 0u));
-            tma_load_3d_a(slot, &map_in, bar, 4 * x0, y0 + V3_GROUP * gi, b, pol_keep);   // rows of 60 pixels x 4 floats: 960 contiguous bytes
-            if (WH) tma_load_4d_a(slot + V3_WIN_BYTES, &map_v, bar, x0, y0, V3_GROUP * gi, b, pol_once);
+            mbar_expect_tx_a(bar, WIN_BYTES + (WH ? V3_V_BYTES : 0u));
+            // rows of 60 pixels x 4 floats (CC = 3: 960 contiguous bytes) or x 1 float
+            tma_load_3d_a(slot, &map_in, bar, (CC == 3 ? 4 : 1) * x0, y0 + V3_GROUP * gi, b, pol_keep);
+            if (WH) {
+                // tiled box {8 col, 4 row, 4 tap}: starts at column 0 and row 0 or 4 of its 8x8 tile (32-byte aligned)
+                if constexpr (TILED) tma_load_5d_a(slot + V3_WIN_BYTES, &map_v, bar, 0, y0 & 7, V3_GROUP * gi, x0 >> 3, b * tiles_y8 + (y0 >> 3), pol_once);
+                else tma_load_4d_a(slot + V3_WIN_BYTES, &map_v, bar, x0, y0, V3_GROUP * gi, b, pol_once);
+            }
         }
     };
     auto issue_hg = [&](int b, int y0, int x0) {
         if (lead) {
-            mbar_expect_tx_a(hbar, (WV ? V3_H_BYTES : 0u) + V3_G_BYTES);
-            if (WV) tma_load_4d_a(base + V3_OFF_H, &map_h, hbar, x0, 0, y0, b, pol_once);   // [row][tap][col]
+            mbar_expect_tx_a(hbar, (WV ? V3_H_BYTES : 0u) + G_BYTES);
+            if (WV) {                                      // [row][tap][col]
+                if constexpr (TILED) tma_load_5d_a(base + V3_OFF_H, &map_h, hbar, 0, 0, y0 & 7, x0 >> 3, b * tiles_y8 + (y0 >> 3), pol_once);
+                else tma_load_4d_a(base + V3_OFF_H, &map_h, hbar, x0, 0, y0, b, pol_once);
+            }
             tma_load_4d_a(base + V3_OFF_G, &map_g, hbar, x0, y0, 0, b, pol_once);
         }
     };
@@ -288,8 +317,8 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
     issue_group(s_cur, b_cur, tb, ty0, tx0, 0);
     issue_group(s_nxt, b_nxt, tb, ty0, tx0, 1);
 
-    const unsigned lane_win = (unsigned)(pg + g) * 16u;    // lane's first tap column inside a window row
-    const unsigned lane_last = lane_win + (novalid ? 11u : 12u) * 64u;   // its slot 12 (g == 3: tap 47 again, see the h copy)
+    const unsigned lane_win = (unsigned)(pg + g) * PIX;    // lane's first tap column inside a window row
+    const unsigned lane_last = lane_win + (novalid ? 11u : 12u) * 4u * PIX;   // its slot 12 (g == 3: tap 47 again, see the h copy)
     const unsigned lane_v = V3_WIN_BYTES + (unsigned)pg * 4u;
     V3_PHASE_INIT(smem_raw + (base - (unsigned)__cvta_generic_to_shared(smem_raw)), V3_OFF_BAR + 32);
 
@@ -301,7 +330,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
         if (has_next && warp == 0 && lead) s_ticket[tile_no & 1] = atomicAdd(next_tile_counter, 1);   // read after this tile's barrier
 
         // ---- this tile's horizontal taps and upstream gradient: shared memory -> registers
-        float2 h2[NP][NT], gh2[NP][NT], g2[3][NP];
+        float2 h2[NP][NT], gh2[NP][NT], g2[CC][NP];
         mbar_wait_a(hbar, p_h);
         p_h ^= 1;
         {
@@ -323,7 +352,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
             }
             const unsigned ga = base + V3_OFF_G + (unsigned)pg * 4u;
 #pragma unroll
-            for (int c = 0; c < 3; ++c)
+            for (int c = 0; c < CC; ++c)
 #pragma unroll
                 for (int pp = 0; pp < NP; ++pp)
                     g2[c][pp] = make_float2(lds_f32_ordered(ga + ((c * R + 2 * pp) * V3_COLS) * 4), lds_f32_ordered(ga + ((c * R + 2 * pp + 1) * V3_COLS) * 4));
@@ -336,8 +365,12 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
 
         const int x = tx0 + pg;
         const bool col_ok = x < sh.W;
-        float* gv_ptr = WV ? gv + (int64_t)tb * K51 * plane + (int64_t)min(ty0 + g, sh.H - 1) * sh.W + min(x, sh.W - 1) - (int64_t)g * plane
-                           : nullptr;
+        // TILED: this warp tile's 8x8 tile (none when the CTA tile reaches past the tensor's last tile column)
+        const bool tile_ok = !TILED || (tx0 >> 3) < tiles_x8;
+        const int64_t tile_base = TILED ? (((int64_t)tb * tiles_y8 + (ty0 >> 3)) * tiles_x8 + (tx0 >> 3)) * (K51 * 64) : 0;
+        float* gv_ptr = !WV ? nullptr
+                      : TILED ? gv + tile_base + ((ty0 & 7) + g) * V3_COLS + pg - g * 64   // plane fy = -g
+                              : gv + (int64_t)tb * K51 * plane + (int64_t)min(ty0 + g, sh.H - 1) * sh.W + min(x, sh.W - 1) - (int64_t)g * plane;
         const bool gv_row_ok = col_ok && (ty0 + g < sh.H);
         float2 gvp[NP];
         auto store_gv = [&](int fy) {                      // fy = s - g for this lane
@@ -346,8 +379,13 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
 #pragma unroll
                 for (int pp = 0; pp < NP; ++pp) { val[2 * pp] = gvp[pp].x; val[2 * pp + 1] = gvp[pp].y; }
                 group_reduce<G, R>(val, g);                // lane g now holds the total of row g
-                if (gv_row_ok && fy >= 0 && fy < K51) __stcs(gv_ptr, ACCUM ? (*gv_ptr + val[0]) : val[0]);
-                gv_ptr += plane;
+                if constexpr (TILED) {                     // a tap's 4 rows x 8 columns are 128 contiguous bytes
+                    if (tile_ok && fy >= 0 && fy < K51) __stcs(gv_ptr, gv_row_ok ? (ACCUM ? (*gv_ptr + val[0]) : val[0]) : 0.f);
+                    gv_ptr += 64;
+                } else {
+                    if (gv_row_ok && fy >= 0 && fy < K51) __stcs(gv_ptr, ACCUM ? (*gv_ptr + val[0]) : val[0]);
+                    gv_ptr += plane;
+                }
             }
         };
         // One group of 4 input rows.  GI >= 0: compile-time group index (first / last groups of the tile, whose steps
@@ -360,7 +398,7 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
 #pragma unroll
             for (int p = 0; p < 4; ++p)                    // plane s - p: this group's slot or the previous one's
                 va[p] = (U - p >= 0 ? vc + ((U - p) * R + p) * V3_COLS * 4 : vp + ((V3_GROUP + U - p) * R + p) * V3_COLS * 4);
-            bwd3_step<S, WV, WH>(wa + U * V3_WIN_COLS * 16, wl + U * V3_WIN_COLS * 16, va, g2, h2, gh2, gvp);
+            bwd3_step<S, WV, WH, CC>(wa + U * V3_WIN_COLS * PIX, wl + U * V3_WIN_COLS * PIX, va, g2, h2, gh2, gvp);
             store_gv(V3_GROUP * gi + U - g);
         };
         auto run_group = [&](auto gi_tag, int gi) {
@@ -396,7 +434,22 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
         V3_PHASE(V3P_LAST);
 
         // ---- gh: complete per lane (the sum over fy happened in registers)
-        if (WH && col_ok) {
+        if constexpr (TILED) if (WH && tile_ok) {
+            float* gp = gh + tile_base + g * 64 + (ty0 & 7) * V3_COLS + pg;
+#pragma unroll
+            for (int t = 0; t < NT; ++t) {
+                if (t == NT - 1 && novalid) break;
+#pragma unroll
+                for (int pp = 0; pp < NP; ++pp) {
+                    const bool a_ok = col_ok && ty0 + 2 * pp < sh.H, b_ok = col_ok && ty0 + 2 * pp + 1 < sh.H;
+                    float* da = gp + G * t * 64 + 2 * pp * V3_COLS;
+                    float* db = da + V3_COLS;
+                    __stcs(da, a_ok ? (ACCUM ? (*da + gh2[pp][t].x) : gh2[pp][t].x) : 0.f);
+                    __stcs(db, b_ok ? (ACCUM ? (*db + gh2[pp][t].y) : gh2[pp][t].y) : 0.f);
+                }
+            }
+        }
+        if constexpr (!TILED) if (WH && col_ok) {
             float* gp = gh + ((int64_t)tb * K51 + g) * plane + x;
 #pragma unroll
             for (int t = 0; t < NT; ++t) {
@@ -420,6 +473,26 @@ sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const
         V3_PHASE(V3P_BARRIER);
     }
     V3_PHASE_FLUSH();
+}
+
+// [B,51,H,W] taps, three channels
+template <bool WV, bool WH, bool ACCUM>
+__global__ void __launch_bounds__(V3_WARPS * 32, SSTEM_BWD3_MINB)
+sepconv_bwd_taps_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_constant__ CUtensorMap map_v,
+                               const __grid_constant__ CUtensorMap map_h, const __grid_constant__ CUtensorMap map_g,
+                               float* __restrict__ gv, float* __restrict__ gh, int* __restrict__ next_tile_counter,
+                               const V3Shape sh, const int* gate, int gate_want) {
+    bwd3_taps_body<WV, WH, ACCUM, 3, false>(map_in, map_v, map_h, map_g, gv, gh, next_tile_counter, sh, gate, gate_want);
+}
+
+// tile-major taps and tap gradients, three channels or one (sstem_sepconv_backward_tiled)
+template <bool WV, bool WH, bool ACCUM, int CC>
+__global__ void __launch_bounds__(V3_WARPS * 32, SSTEM_BWD3_MINB)
+sepconv_bwd_taps_k51_v3_tiled_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_constant__ CUtensorMap map_v,
+                                     const __grid_constant__ CUtensorMap map_h, const __grid_constant__ CUtensorMap map_g,
+                                     float* __restrict__ gv, float* __restrict__ gh, int* __restrict__ next_tile_counter,
+                                     const V3Shape sh, const int* gate, int gate_want) {
+    bwd3_taps_body<WV, WH, ACCUM, CC, true>(map_in, map_v, map_h, map_g, gv, gh, next_tile_counter, sh, gate, gate_want);
 }
 
 // =====================================================================================================================

@@ -1,6 +1,7 @@
 // Layout kernels around the 51-tap kernels, each compiled once: the input repacks that the third-generation kernels'
 // tensor maps read (sepconv_k51_fwd3.cu, sepconv_k51_bwd3.cu) in a stream-ordered workspace, the gray x3 plane
-// comparison (abi.cu) and the tile-major tap layout of SURVEY 8f N2 (sstem_taps_to_tiled).
+// comparison (abi.cu), the tile-major tap layout of SURVEY 8f N2 (sstem_taps_to_tiled, sstem_taps_from_tiled) and the
+// upstream-gradient staging of the tiled tap gradients (sepconv_k51_bwd3.cu).
 #include "sepconv_k51.cuh"
 
 namespace sstem {
@@ -82,6 +83,43 @@ taps_to_tiled_kernel(const float* __restrict__ taps, float* __restrict__ tiled, 
     }
 }
 
+// The inverse: tile-major -> [B,51,H,W] (the padding entries are not read).  One thread per output element.
+__global__ void __launch_bounds__(256)
+taps_from_tiled_kernel(const float* __restrict__ tiled, float* __restrict__ taps, int H, int W, int ty8, int tx8, int64_t total) {
+    const int64_t step = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += step) {
+        const int x = (int)(i % W);
+        int64_t r = i / W;
+        const int y = (int)(r % H); r /= H;
+        const int tap = (int)(r % K51);
+        const int64_t b = r / K51;
+        taps[i] = __ldg(tiled + (((b * ty8 + (y >> 3)) * tx8 + (x >> 3)) * K51 + tap) * 64 + (y & 7) * 8 + (x & 7));
+    }
+}
+
+// grad_output planes at a 16-byte row pitch for the tiled tap-gradient kernel's tensor map: out [B,nplanes,H,WP] holds the
+// C planes of g [B,C,H,W], or (sum) their channel sum, the gray x3 shortcut's upstream gradient.  Pad columns are zero.
+__global__ void __launch_bounds__(256)
+stage_grad_planes_kernel(const float* __restrict__ g, float* __restrict__ out, int C, int nplanes, int H, int W, int WP, int64_t total) {
+    const int64_t step = (int64_t)gridDim.x * blockDim.x;
+    const int64_t plane = (int64_t)H * W;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += step) {
+        const int x = (int)(i % WP);
+        int64_t r = i / WP;
+        const int y = (int)(r % H); r /= H;
+        const int p = (int)(r % nplanes);
+        const int64_t b = r / nplanes;
+        float v = 0.f;
+        if (x < W) {
+            const float* src = g + (b * C + (nplanes == C ? p : 0)) * plane + (int64_t)y * W + x;
+            v = __ldg(src);
+            if (nplanes != C)
+                for (int c = 1; c < C; ++c) v += __ldg(src + c * plane);
+        }
+        out[i] = v;
+    }
+}
+
 }  // namespace
 
 // Stream-ordered scratch memory (released with cudaFreeAsync on the same stream).  The device's default pool hands
@@ -128,6 +166,24 @@ int launch_repack_plane_pitch(const float* in, float* ws, int64_t B, int C, int 
     return finish_launch();
 }
 
+int launch_stage_grad_planes(const float* g, float* out, int64_t B, int64_t C, int64_t H, int64_t W, int64_t WP, bool sum,
+                             cudaStream_t s) {
+    const int nplanes = sum ? 1 : (int)C;
+    const int64_t total = B * nplanes * H * WP;
+    const unsigned blocks = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)sm_count() * 16);
+    stage_grad_planes_kernel<<<blocks, 256, 0, s>>>(g, out, (int)C, nplanes, (int)H, (int)W, (int)WP, total);
+    count_launch();
+    return finish_launch();
+}
+
+int launch_taps_from_tiled(const float* tiled, float* taps, int64_t B, int64_t H, int64_t W, cudaStream_t s) {
+    const int64_t total = B * K51 * H * W;
+    const unsigned blocks = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)sm_count() * 32);
+    taps_from_tiled_kernel<<<blocks, 256, 0, s>>>(tiled, taps, (int)H, (int)W, (int)((H + 7) / 8), (int)((W + 7) / 8), total);
+    count_launch();
+    return finish_launch();
+}
+
 int launch_planes_equal(const float* in, int64_t B, int64_t C, int64_t plane, int* flag, cudaStream_t s) {
     cudaError_t e = cudaMemsetAsync(flag, 1, sizeof(int), s);      // non-zero = "identical planes" until a mismatch clears it
     if (e != cudaSuccess) return (int)e;
@@ -159,4 +215,13 @@ extern "C" int sstem_taps_to_tiled(const float* taps, float* tiled, int64_t B, i
     taps_to_tiled_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(taps, tiled, (int)H, (int)W, (int)((H + 7) / 8), (int)((W + 7) / 8), total);
     count_launch();
     return finish_launch();
+}
+
+extern "C" int sstem_taps_from_tiled(const float* tiled, float* taps, int64_t B, int64_t H, int64_t W, void* stream) {
+    if (!tiled || !taps) return SSTEM_E_NULL;
+    if (B <= 0 || H <= 0 || W <= 0 || H > (1 << 24) || W > (1 << 24)) return SSTEM_E_SHAPE;
+    if (!aligned16(tiled) || !aligned4(taps)) return SSTEM_E_ALIGN;
+    DeviceGuard guard(taps);
+    if (guard.err) return guard.err;
+    return launch_taps_from_tiled(tiled, taps, B, H, W, (cudaStream_t)stream);
 }

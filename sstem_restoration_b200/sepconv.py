@@ -333,36 +333,106 @@ def taps_to_tiled(taps: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def sepconv_forward_tiled(input: torch.Tensor, vertical_tiled: torch.Tensor, horizontal_tiled: torch.Tensor, out=None,
-                          accumulate: bool = False) -> torch.Tensor:
-    """``SeparableConvolution.apply(input, vertical, horizontal)`` with both tap tensors in the tile-major layout of
-    :func:`taps_to_tiled`; forward only; bit-identical to the [B,51,H,W] path.  Follows :func:`set_gray_replicated`.
-    ``out`` / ``accumulate``: write into (add to) an existing [B,C,H,W] tensor -- the second frame of the interpolation
-    tail (the general path only: the gray shortcut writes its replicas from one register)."""
+def taps_from_tiled(tiled: torch.Tensor, H: int, W: int) -> torch.Tensor:
+    """Inverse of :func:`taps_to_tiled`: tile-major ``[B, ceil(H/8), ceil(W/8), 51, 8, 8]`` -> [B,51,H,W] (the entries
+    outside the image are not read)."""
+    if tiled.is_cuda == False:
+        raise NotImplementedError()
+    want = ((H + 7) // 8, (W + 7) // 8, 51, 8, 8)
+    if tiled.dtype != torch.float32 or tiled.dim() != 6 or tuple(tiled.shape[1:]) != want:
+        raise TypeError(f"taps_from_tiled: float32 [B,{','.join(map(str, want))}] required for H={H}, W={W}")
+    tiled = tiled.contiguous()
+    B = tiled.size(0)
+    out = torch.empty((B, 51, H, W), dtype=torch.float32, device=tiled.device)
+    if out.numel():
+        code = _lib.load().sstem_taps_from_tiled(tiled.data_ptr(), out.data_ptr(), B, H, W, _stream_ptr(tiled))
+        if code:
+            _lib.check(code, "sstem_taps_from_tiled")
+    return out
+
+
+def _check_tiled(what, input, vertical_tiled, horizontal_tiled):
     for t in (input, vertical_tiled, horizontal_tiled):
         if t.is_cuda == False:
             raise NotImplementedError()
         if t.dtype != torch.float32:
-            raise TypeError("sepconv_forward_tiled: float32 tensors required")
+            raise TypeError(f"{what}: float32 tensors required")
     assert (input.is_contiguous() == True) and (vertical_tiled.is_contiguous() == True) and (horizontal_tiled.is_contiguous() == True)
     B, C, IH, IW = input.shape
     H, W = IH - 50, IW - 50
     want = (B, (H + 7) // 8, (W + 7) // 8, 51, 8, 8)
     assert tuple(vertical_tiled.shape) == want and tuple(horizontal_tiled.shape) == want, f"tiled taps must be {want}"
-    if out is None:
-        if accumulate:
-            raise ValueError("sepconv_forward_tiled: accumulate needs an existing `out`")
-        out = torch.empty((B, C, H, W), dtype=torch.float32, device=input.device)
-    else:
-        assert tuple(out.shape) == (B, C, H, W) and out.dtype == torch.float32 and (out.is_contiguous() == True) and out.device == input.device
+    return B, C, H, W
+
+
+def _forward_tiled(input, vertical_tiled, horizontal_tiled, out, accumulate, gray):
+    B, C, H, W = out.shape
     if out.numel():
-        gray = (not accumulate) and _is_gray(input)
         flags = (_lib.SEPCONV_GRAY_REPLICATED if gray else 0) | (_lib.SEPCONV_ACCUMULATE if accumulate else 0)
         code = _lib.load().sstem_sepconv_forward_tiled(input.data_ptr(), vertical_tiled.data_ptr(), horizontal_tiled.data_ptr(),
                                                        out.data_ptr(), B, C, H, W, 51, flags, _stream_ptr(input))
         if code:
             _lib.check(code, "sstem_sepconv_forward_tiled")
     return out
+
+
+def _backward_tiled(grad_output, input, vertical_tiled, horizontal_tiled, need_in, need_v, need_h, gray):
+    """-> (grad_input, grad_vertical_tiled, grad_horizontal_tiled), None where not needed."""
+    B, C, IH, IW = input.shape
+    grad_output = _check_grad_output(grad_output, (B, C, IH - 50, IW - 50), input)
+    grad_input = torch.empty_like(input) if need_in else None
+    grad_v = torch.empty_like(vertical_tiled) if need_v else None
+    grad_h = torch.empty_like(horizontal_tiled) if need_h else None
+    if (need_in or need_v or need_h) and grad_output.numel() > 0:
+        code = _lib.load().sstem_sepconv_backward_tiled(
+            grad_output.data_ptr(), input.data_ptr(), vertical_tiled.data_ptr(), horizontal_tiled.data_ptr(),
+            grad_input.data_ptr() if need_in else None, grad_v.data_ptr() if need_v else None,
+            grad_h.data_ptr() if need_h else None, B, C, IH - 50, IW - 50, 51,
+            _lib.SEPCONV_GRAY_REPLICATED if gray else 0, _stream_ptr(input))
+        if code:
+            _lib.check(code, "sstem_sepconv_backward_tiled")
+    return grad_input, grad_v, grad_h
+
+
+def sepconv_forward_tiled(input: torch.Tensor, vertical_tiled: torch.Tensor, horizontal_tiled: torch.Tensor, out=None,
+                          accumulate: bool = False) -> torch.Tensor:
+    """``SeparableConvolution.apply(input, vertical, horizontal)`` with both tap tensors in the tile-major layout of
+    :func:`taps_to_tiled`; forward only (no autograd graph: use :class:`SeparableConvolutionTiled` for gradients);
+    bit-identical to the [B,51,H,W] path.  Follows :func:`set_gray_replicated`.
+    ``out`` / ``accumulate``: write into (add to) an existing [B,C,H,W] tensor -- the second frame of the interpolation
+    tail (the general path only: the gray shortcut writes its replicas from one register)."""
+    B, C, H, W = _check_tiled("sepconv_forward_tiled", input, vertical_tiled, horizontal_tiled)
+    if out is None:
+        if accumulate:
+            raise ValueError("sepconv_forward_tiled: accumulate needs an existing `out`")
+        out = torch.empty((B, C, H, W), dtype=torch.float32, device=input.device)
+    else:
+        assert tuple(out.shape) == (B, C, H, W) and out.dtype == torch.float32 and (out.is_contiguous() == True) and out.device == input.device
+    gray = out.numel() > 0 and (not accumulate) and _is_gray(input)
+    return _forward_tiled(input, vertical_tiled, horizontal_tiled, out, accumulate, gray)
+
+
+class SeparableConvolutionTiled(torch.autograd.Function):
+    """:class:`SeparableConvolution` with both tap tensors in the tile-major layout of :func:`taps_to_tiled`:
+    ``SeparableConvolutionTiled.apply(input, vertical_tiled, horizontal_tiled)`` -> [B,C,H,W].  The tap gradients come
+    out tile-major as well (zero outside the image); with taps that run the same kernel on the [B,51,H,W] path they are
+    bit-identical to :class:`SeparableConvolution`'s.  The gray x3 shortcut is decided once, on the host, in the forward
+    (:func:`set_gray_replicated`; ``"auto"`` does not pay a synchronisation for it) and reused by the backward."""
+
+    @staticmethod
+    def forward(ctx, input, vertical_tiled, horizontal_tiled):
+        B, C, H, W = _check_tiled("SeparableConvolutionTiled", input, vertical_tiled, horizontal_tiled)
+        out = torch.empty((B, C, H, W), dtype=torch.float32, device=input.device)
+        ctx.gray = out.numel() > 0 and _is_gray(input)
+        ctx.save_for_backward(input, vertical_tiled, horizontal_tiled)
+        return _forward_tiled(input, vertical_tiled, horizontal_tiled, out, False, ctx.gray)
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        input, vertical_tiled, horizontal_tiled = ctx.saved_tensors
+        if grad_output.is_cuda == False:
+            raise NotImplementedError()
+        return _backward_tiled(grad_output, input, vertical_tiled, horizontal_tiled, *ctx.needs_input_grad[:3], ctx.gray)
 
 
 def frame_mean_pad(frame: torch.Tensor, pad: int = 25, gray=None) -> torch.Tensor:
@@ -388,7 +458,8 @@ def frame_mean_pad(frame: torch.Tensor, pad: int = 25, gray=None) -> torch.Tenso
 
 def interpolation_tail_tiled(i1, i2, k1v_tiled, k1h_tiled, k2v_tiled, k2h_tiled) -> torch.Tensor:
     """:func:`interpolation_tail` for tap tensors in the tile-major layout (what :class:`ModuleTapProducer` emits): the whole
-    tail of ``IFNet.forward`` (model_interp.py:90-97) without a [B,51,H,W] tensor anywhere.  Forward only.
+    tail of ``IFNet.forward`` (model_interp.py:90-97) without a [B,51,H,W] tensor anywhere.  Forward only (no autograd
+    graph: :class:`ModuleInterpolationTailTiled` is the differentiable form).
 
     mean_c sepconv(pad(i_c)) = sepconv(pad(mean_c i_c)), so each frame is reduced to one replicate-padded plane
     (:func:`frame_mean_pad`) and convolved by the persistent one-channel kernel; the second frame accumulates into the first
@@ -396,3 +467,35 @@ def interpolation_tail_tiled(i1, i2, k1v_tiled, k1h_tiled, k2v_tiled, k2h_tiled)
     p2, p1 = frame_mean_pad(i2), frame_mean_pad(i1)
     out = sepconv_forward_tiled(p2, k2v_tiled, k2h_tiled)
     return sepconv_forward_tiled(p1, k1v_tiled, k1h_tiled, out=out, accumulate=True)
+
+
+class _InterpolationTailTiled(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, i1, i2, k1v, k1h, k2v, k2h):
+        p2, p1 = frame_mean_pad(i2), frame_mean_pad(i1)
+        out = sepconv_forward_tiled(p2, k2v, k2h)
+        ctx.save_for_backward(p1, p2, k1v, k1h, k2v, k2h)
+        return sepconv_forward_tiled(p1, k1v, k1h, out=out, accumulate=True)
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
+            raise NotImplementedError("interpolation_tail_tiled: the frames are data; no gradient w.r.t. them "
+                                      "(use SeparableConvolutionTiled on the padded frames for that)")
+        if grad_output.is_cuda == False:
+            raise NotImplementedError()
+        p1, p2, k1v, k1h, k2v, k2h = ctx.saved_tensors
+        n1v, n1h, n2v, n2h = ctx.needs_input_grad[2:6]
+        # out = sepconv(p2, k2) + sepconv(p1, k1) on the one-plane mean frames: each frame's taps see grad_output as is
+        _, g2v, g2h = _backward_tiled(grad_output, p2, k2v, k2h, False, n2v, n2h, False)
+        _, g1v, g1h = _backward_tiled(grad_output, p1, k1v, k1h, False, n1v, n1h, False)
+        return None, None, g1v, g1h, g2v, g2h
+
+
+class ModuleInterpolationTailTiled(torch.nn.Module):
+    """Differentiable :func:`interpolation_tail_tiled` (stateless): the same forward, and the four tap gradients in the
+    tile-major layout, two one-plane tiled backward calls on the padded mean frames.  The frames get no gradient
+    (``NotImplementedError`` if one is asked for, as :func:`interpolation_tail`)."""
+
+    def forward(self, i1, i2, k1v_tiled, k1h_tiled, k2v_tiled, k2h_tiled):
+        return _InterpolationTailTiled.apply(i1, i2, k1v_tiled, k1h_tiled, k2v_tiled, k2h_tiled)

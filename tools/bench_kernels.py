@@ -1,5 +1,5 @@
 """Quick kernel-level timing of the sepconv / warp entry points (CUDA events, inputs > L2 rotated).
-Usage: python tools/bench_kernels.py [fwd] [bwd] [warp] [gi]"""
+Usage: python tools/bench_kernels.py [fwd] [bwd] [warp] [gi] [tiled] [gray] [tail] [tiledbwd]"""
 import os
 import sys
 import json
@@ -65,6 +65,34 @@ def main():
                 print(json.dumps({"op": nm, "shape": [B, C, H, W], "ms_tiled": round(ms, 4), "ms_nchw": round(ms0, 4),
                                   "gpix_s_tiled": round(px / ms / 1e6, 3), "tap_GBs_tiled": round(px * 408 / ms / 1e6, 1), "tap_GBs_nchw": round(px * 408 / ms0 / 1e6, 1)}))
             del vt, ht
+        if "tiledbwd" in what and C == 3 and (B, H, W) in ((16, 512, 512), (1, 2048, 2048)):
+            # tap gradients on tile-major taps vs [B,51,H,W], general and gray x3; then the tail's tap gradients (both frames)
+            vt, ht = pkg.taps_to_tiled(v), pkg.taps_to_tiled(h)
+            gv, gh, gvt, ght = torch.empty_like(v), torch.empty_like(h), torch.empty_like(vt), torch.empty_like(ht)
+            res = {"op": "tiledbwd", "shape": [B, C, H, W]}
+            for flag, nm in ((0, "general"), (2, "gray")):
+                if flag:
+                    inp[:, 1:] = inp[:, :1]
+                res["ms_tiled_" + nm] = round(timeit(lambda: lib.sstem_sepconv_backward_tiled(
+                    g.data_ptr(), inp.data_ptr(), vt.data_ptr(), ht.data_ptr(), None, gvt.data_ptr(), ght.data_ptr(), B, C, H, W, K, flag, st), reps=3, warm=1), 4)
+                res["ms_nchw_" + nm] = round(timeit(lambda: lib.sstem_sepconv_backward(
+                    g.data_ptr(), inp.data_ptr(), v.data_ptr(), h.data_ptr(), None, gv.data_ptr(), gh.data_ptr(), B, C, H, W, K, flag, st), reps=3, warm=1), 4)
+            f1, f2 = (torch.rand((B, 3, H, W), device=dev) for _ in range(2))
+            p1, p2 = pkg.frame_mean_pad(f1), pkg.frame_mean_pad(f2)
+            go = torch.rand((B, 1, H, W), device=dev) - 0.5
+            gts = [torch.empty_like(vt) for _ in range(4)]
+            gns = [torch.empty_like(v) for _ in range(4)]
+
+            def tail_tiled():                              # what ModuleInterpolationTailTiled's backward launches
+                for p, t in ((p2, gts[2:]), (p1, gts[:2])):
+                    lib.sstem_sepconv_backward_tiled(go.data_ptr(), p.data_ptr(), vt.data_ptr(), ht.data_ptr(), None, t[0].data_ptr(), t[1].data_ptr(),
+                                                     B, 1, H, W, K, 0, st)
+            res["ms_tail_bwd_tiled"] = round(timeit(tail_tiled, reps=3, warm=1), 4)
+            res["ms_tail_bwd_nchw"] = round(timeit(lambda: lib.sstem_interp_tail_backward(
+                go.data_ptr(), f1.data_ptr(), f2.data_ptr(), 3 * H * W, v.data_ptr(), h.data_ptr(), v.data_ptr(), h.data_ptr(),
+                *[t.data_ptr() for t in gns], B, 3, H, W, K, 0, st), reps=3, warm=1), 4)
+            print(json.dumps(res))
+            del vt, ht, gv, gh, gvt, ght, f1, f2, p1, p2, go, gts, gns
         if "gray" in what and C == 3:
             gv, gh = torch.empty_like(v), torch.empty_like(h)
             inp[:, 1:] = inp[:, :1]
