@@ -1,7 +1,6 @@
 // C-ABI entry points for the sepconv path (argument checks + dispatch) and the
 // small ABI utilities.  See include/sstem_b200.h for the contract.
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace sstem {
 std::atomic<int64_t> g_launches{0};
@@ -58,8 +57,7 @@ extern "C" int sstem_sepconv_backward(const float* grad_output, const float* inp
         if (e) return e;
     }
     if (grad_input) {
-        static const bool gi_generic = getenv("SSTEM_GI_GENERIC") != nullptr;   // experiments
-        if (K == 51 && !gi_generic) e = launch_sepconv_bwd_input_k51(grad_output, vertical, horizontal, grad_input, B, C, H, W, s);
+        if (K == 51) e = launch_sepconv_bwd_input_k51(grad_output, vertical, horizontal, grad_input, B, C, H, W, s);
         else e = launch_sepconv_bwd_input_generic(grad_output, vertical, horizontal, grad_input, B, C, H, W, K, s);
     }
     return e;

@@ -93,7 +93,12 @@ int launch_sepconv_bwd_input_k51(const float* g, const float* v, const float* h,
 int launch_sepconv_bwd_input_generic(const float* g, const float* v, const float* h, float* gi,
                                      int64_t B, int64_t C, int64_t H, int64_t W, int K, cudaStream_t s);
 
-// third-generation 51-tap kernels (sepconv_k51_bwd3.cu, sepconv_k51_fwd3.cu); -1000 = path does not apply
+// Returned by a try_launch_* launcher whose fast path does not apply to the call; the caller runs its general kernel.
+// Distinct from every CUDA error (positive) and SSTEM_E_* code, and never returned through the C ABI.
+constexpr int PATH_NOT_APPLICABLE = INT32_MIN;
+
+// third-generation 51-tap kernels on a 3-channel chunk of [B,51,H,W] taps (sepconv_k51_bwd3.cu, sepconv_k51_fwd3.cu):
+// 0, a CUDA error, or PATH_NOT_APPLICABLE (the caller runs generation 1)
 int try_launch_bwd_taps_k51_v3(const float* g, const float* in, const float* v, const float* h, float* gv, float* gh,
                                int64_t B, int C, int c0, int H, int W, int accumulate, cudaStream_t s);
 int try_launch_fwd_k51_v3(const float* in, const float* v, const float* h, float* out,

@@ -73,7 +73,7 @@ int launch_bwd_all(const float* g, const float* in, const float* v, const float*
         if (cc == 3) {
             // third-generation kernel (persistent warps, TMA-streamed, channel-interleaved window) when its layout rules hold
             e = try_launch_bwd_taps_k51_v3(g, in, v, h, WV ? gv : nullptr, WH ? gh : nullptr, B, C, c0, H, W, acc, s);
-            if (e == -1000) e = launch_bwd_chunk<3, WV, WH>(g, in, v, h, gv, gh, B, C, c0, H, W, acc, 1, s);
+            if (e == PATH_NOT_APPLICABLE) e = launch_bwd_chunk<3, WV, WH>(g, in, v, h, gv, gh, B, C, c0, H, W, acc, 1, s);
         }
         else if (cc == 2) e = launch_bwd_chunk<2, WV, WH>(g, in, v, h, gv, gh, B, C, c0, H, W, acc, 1, s);
         else e = launch_bwd_chunk<1, WV, WH>(g, in, v, h, gv, gh, B, C, c0, H, W, acc, 1, s);

@@ -44,7 +44,7 @@ int launch_sepconv_fwd_k51(const float* in, const float* v, const float* h, floa
         if (cc == 3) {
             // third-generation kernel (persistent warps, TMA-streamed, channel-interleaved window) when its layout rules hold
             e = try_launch_fwd_k51_v3(in, v, h, out, B, (int)C, c0, (int)H, (int)W, s);
-            if (e == -1000) e = launch_fwd_chunk<3>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
+            if (e == PATH_NOT_APPLICABLE) e = launch_fwd_chunk<3>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
         }
         else if (cc == 2) e = launch_fwd_chunk<2>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);
         else e = launch_fwd_chunk<1>(in, v, h, out, B, (int)C, c0, (int)H, (int)W, 1, s);

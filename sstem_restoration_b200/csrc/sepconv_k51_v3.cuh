@@ -24,6 +24,7 @@
 #pragma once
 #include "sepconv_k51.cuh"
 #include "tma.cuh"
+#include <stdlib.h>
 #include <type_traits>
 
 namespace sstem {
@@ -766,6 +767,92 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
         V3_PHASE(V3P_BARRIER);
     }
     V3_PHASE_FLUSH();
+}
+
+// =====================================================================================================================
+// Host side, shared by the launchers in sepconv_k51_fwd3.cu and sepconv_k51_bwd3.cu.
+// =====================================================================================================================
+
+// Tile grid of a persistent launch: CTA tiles of V3_WARPS warp tiles side by side, `tiles_y` warp-tile rows per image.
+// false when there are too many tiles for the int tile tickets.
+inline bool v3_shape(V3Shape& sh, int64_t B, int C, int c0, int H, int W, int64_t tiles_y) {
+    const int64_t tiles_x = (W + V3_COLS * V3_WARPS - 1) / (V3_COLS * V3_WARPS);
+    if (tiles_x * tiles_y * B > INT32_MAX / 2) return false;
+    sh = V3Shape{H, W, (int)tiles_x, (int)tiles_y, (int)(tiles_x * tiles_y * B), C, c0};
+    return true;
+}
+
+// The window of one persistent launch, in a stream-ordered workspace: channels sh.c0.. of the input [B,C,H+50,W+50]
+// copied to the layout the window boxes read (CC = 3: channel-interleaved [B][H+50][W+50][4]; CC = 1: one plane at a
+// 16-byte row pitch), then the dynamic tile scheduler's ticket counter, and the tensor map of the copy.  The workspace
+// goes back to the pool on the stream when the object goes out of scope, after the work enqueued on it.
+// err: 0, cudaErrorMemoryAllocation when there is no workspace, a CUDA error of the memset or the copy, or SSTEM_E_SHAPE
+// when the map cannot be encoded.
+template <int CC>
+struct V3Window {
+    cudaStream_t s;
+    float* ws = nullptr;
+    int* counter = nullptr;
+    CUtensorMap map;
+    int err = 0;
+    V3Window(const float* in, int64_t B, const V3Shape& sh, cudaStream_t s_) : s(s_) {
+        const int64_t IH = sh.H + K51 - 1, IW = sh.W + K51 - 1, IWP = (IW + 3) & ~(int64_t)3;
+        const int64_t row = CC == 3 ? 4 * IW : IWP;        // floats per window row
+        const size_t bytes = (size_t)(B * IH * row) * 4;
+        if (workspace_alloc(reinterpret_cast<void**>(&ws), bytes + 256, s)) { err = cudaErrorMemoryAllocation; return; }
+        counter = reinterpret_cast<int*>(reinterpret_cast<char*>(ws) + bytes);
+        if (cudaError_t e = cudaMemsetAsync(counter, 0, 256, s)) { cudaGetLastError(); err = (int)e; return; }
+        err = CC == 3 ? launch_repack_nhwc4(in, ws, B, sh.C, sh.c0, IH, IW, s)
+                      : launch_repack_plane_pitch(in, ws, B, sh.C, sh.c0, IH, IW, IWP, s);
+        if (err) return;
+        // CC = 3: the box's inner extent is a whole 960-byte row segment (an inner extent of one pixel = 16 bytes makes
+        // the TMA unit issue 240 tiny requests per box: measured 1.5x slower)
+        const int64_t dims[3] = {row, IH, B}, strides[3] = {1, row, row * IH};
+        const int box[3] = {(CC == 3 ? 4 : 1) * V3_WIN_COLS, V3_GROUP, 1};
+        if (!make_map_f32(&map, ws, 3, dims, strides, box)) err = SSTEM_E_SHAPE;
+    }
+    ~V3Window() { if (ws) cudaFreeAsync(ws, s); }
+};
+
+// Tensor maps of [B,51,H,W] taps for warp tiles of `rows` rows: v in boxes {8 columns, rows, 4 planes}, landing as
+// [plane][row][col].  h is described with its tap and row dimensions swapped, {W, 51, H, B}, so that its box
+// {8 columns, 51 taps, rows} lands as [row][tap][col]: the per-lane register copy of the taps then hits 32 different
+// banks, where as [tap][row][col] the four tap groups of a column collide in one bank.
+inline bool make_v3_tap_maps(CUtensorMap* mv, CUtensorMap* mh, const float* v, const float* h, int64_t B, int H, int W, int rows) {
+    const int64_t plane = (int64_t)H * W;
+    const int64_t vdims[4] = {W, H, K51, B}, vstrides[4] = {1, W, plane, K51 * plane};
+    const int64_t hdims[4] = {W, K51, H, B}, hstrides[4] = {1, plane, W, K51 * plane};
+    const int vbox[4] = {V3_COLS, rows, V3_GROUP, 1}, hbox[4] = {V3_COLS, K51, rows, 1};
+    return make_map_f32(mv, v, 4, vdims, vstrides, vbox) && make_map_f32(mh, h, 4, hdims, hstrides, hbox);
+}
+
+// Launches a persistent grid of Kern: two CTAs per SM, fewer when there are fewer CTA tiles.  Templated on the kernel
+// itself, not its type: every kernel needs its own PerDeviceOnce, or only the first would get its shared-memory size.
+template <auto Kern, class... Args>
+int launch_persistent(size_t smem, int ntiles, cudaStream_t s, const Args&... args) {
+    static PerDeviceOnce done;
+    if (int e = set_smem_once(Kern, smem, done)) return e;
+    const int ctas = (int)std::min<int64_t>(2 * (int64_t)sm_count(), (int64_t)ntiles);
+    Kern<<<ctas, V3_WARPS * 32, smem, s>>>(args..., g_gate.ptr, g_gate.want);
+    count_launch();
+    return finish_launch();
+}
+
+// When a 3-channel chunk on [B,51,H,W] taps runs on generation 3: `launch(sh)` runs it, or the caller gets
+// PATH_NOT_APPLICABLE and runs generation 1.  The tensor maps need W % 4 == 0 and the tensors they read 16-byte aligned
+// (`aligned`), the tile tickets must fit an int, and a persistent grid needs several CTA tiles per CTA to balance:
+// `min_tiles`, the measured crossover, unless SSTEM_V3_MIN_TILES gives another (A/B runs, tools/sweep_small.py).  A
+// launch that returns cudaErrorMemoryAllocation (no workspace; nothing of the chunk has run) or SSTEM_E_SHAPE (a tensor
+// map cannot be encoded) falls back too.
+template <class Launch>
+int try_v3(bool aligned, int64_t B, int C, int c0, int H, int W, int rows, int64_t min_tiles, Launch launch) {
+    static const char* env = getenv("SSTEM_V3_MIN_TILES");
+    if (env) min_tiles = atoll(env);
+    V3Shape sh;
+    if ((W & 3) || !aligned || !v3_shape(sh, B, C, c0, H, W, (H + rows - 1) / rows) || sh.ntiles < min_tiles * 2 * sm_count())
+        return PATH_NOT_APPLICABLE;
+    const int e = launch(sh);
+    return e == cudaErrorMemoryAllocation || e == SSTEM_E_SHAPE ? PATH_NOT_APPLICABLE : e;
 }
 
 }  // namespace

@@ -474,18 +474,18 @@ static bool make_map3(CUtensorMap* m, const float* base, int64_t W, int64_t H, i
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// returns 0 on launch, >0 cuda error, -1000 when the TMA path does not apply (caller falls back)
+// returns 0 on launch, >0 cuda error, PATH_NOT_APPLICABLE when the TMA path does not apply (caller falls back)
 template <int CT, bool STITCH = false>
 static int try_launch_warp_tma(const float* moving, const float* flow, const int64_t* fs, float* out,
                                int64_t B, int64_t H, int64_t W, cudaStream_t s, WarpStitch st = WarpStitch{nullptr, nullptr, nullptr}) {
-    if ((W & 3) || fs[2] != 1 || !aligned16(moving) || !aligned16(flow) || (!STITCH && !aligned16(out))) return -1000;
-    if ((fs[0] & 3) || (fs[1] & 3) || (fs[3] & 3) || fs[1] < W || B > 65535 || (H + WT_TH - 1) / WT_TH > 65535) return -1000;
+    if ((W & 3) || fs[2] != 1 || !aligned16(moving) || !aligned16(flow) || (!STITCH && !aligned16(out))) return PATH_NOT_APPLICABLE;
+    if ((fs[0] & 3) || (fs[1] & 3) || (fs[3] & 3) || fs[1] < W || B > 65535 || (H + WT_TH - 1) / WT_TH > 65535) return PATH_NOT_APPLICABLE;
     CUtensorMap mfx, mfy, mim, mims, mimm;
-    if (!make_map3(&mfx, flow, W, H, B, fs[1], fs[0], WT_TW, WT_TH, 1)) return -1000;
-    if (!make_map3(&mfy, flow + fs[3], W, H, B, fs[1], fs[0], WT_TW, WT_TH, 1)) return -1000;
-    if (!make_map3(&mim, moving, W, H, B * CT, W, H * W, WT_BW, WT_BH, CT)) return -1000;
-    if (!make_map3(&mims, moving, W, H, B * CT, W, H * W, WT_SW, WT_SH, CT)) return -1000;
-    if (!make_map3(&mimm, moving, W, H, B * CT, W, H * W, WT_MW, WT_MH, CT)) return -1000;
+    if (!make_map3(&mfx, flow, W, H, B, fs[1], fs[0], WT_TW, WT_TH, 1)) return PATH_NOT_APPLICABLE;
+    if (!make_map3(&mfy, flow + fs[3], W, H, B, fs[1], fs[0], WT_TW, WT_TH, 1)) return PATH_NOT_APPLICABLE;
+    if (!make_map3(&mim, moving, W, H, B * CT, W, H * W, WT_BW, WT_BH, CT)) return PATH_NOT_APPLICABLE;
+    if (!make_map3(&mims, moving, W, H, B * CT, W, H * W, WT_SW, WT_SH, CT)) return PATH_NOT_APPLICABLE;
+    if (!make_map3(&mimm, moving, W, H, B * CT, W, H * W, WT_MW, WT_MH, CT)) return PATH_NOT_APPLICABLE;
     const size_t smem = (size_t)(CT * WT_BH * WT_BW + 2 * WT_TH * WT_TW) * sizeof(float) + 64;   // 2 barriers + 7 ints of tile statistics
     static PerDeviceOnce done;
     int dev = 0;
@@ -622,7 +622,7 @@ extern "C" int sstem_warp_forward(const float* moving, const float* flow, const 
     if (out_layout == SSTEM_LAYOUT_NCHW && (C == 1 || C == 3) && !no_tma) {
         const int r = (C == 3) ? try_launch_warp_tma<3>(moving, flow, flow_strides, out, B, H, W, s)
                                : try_launch_warp_tma<1>(moving, flow, flow_strides, out, B, H, W, s);
-        if (r != -1000) return r;
+        if (r != PATH_NOT_APPLICABLE) return r;
     }
     constexpr int PX = SSTEM_WARP_PX;
     const int gpr = (int)((W + PX - 1) / PX);
@@ -729,7 +729,7 @@ extern "C" int sstem_warp_stitch_forward(const float* moving, const float* flow,
     const WarpStitch st{interp, gray_out, stitch_out};
     const int r = (C == 3) ? try_launch_warp_tma<3, true>(moving, flow, flow_strides, nullptr, B, H, W, s, st)
                            : try_launch_warp_tma<1, true>(moving, flow, flow_strides, nullptr, B, H, W, s, st);
-    if (r != -1000) return r;
+    if (r != PATH_NOT_APPLICABLE) return r;
     // shapes the TMA kernel does not take: the two steps one after the other through a stream-ordered scratch image
     float* tmp = nullptr;
     if (workspace_alloc(reinterpret_cast<void**>(&tmp), (size_t)(B * C * H * W) * sizeof(float), s)) return (int)cudaErrorMemoryAllocation;
