@@ -376,12 +376,15 @@ warp_torch_tma_kernel(const __grid_constant__ CUtensorMap map_fx, const __grid_c
         float2 wa2[2], wb2[2], wc2[2], wd2[2];          // pixels (0,1) and (2,3) side by side for the packed FP32 ops
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
-            a00[q] = offa[q];
-            a01[q] = offa[q] + dxs[q];
-            a10[q] = offa[q] + dys[q] * pitch;
-            a11[q] = a10[q] + dxs[q];
             const int i = i0 + warp + WT_HALF * (q >> 1), j = j00 + lane + 32 * (q & 1);
             ok[q] = i < H && j < W;
+            // A pixel outside the image (last tile row / column of a ragged shape) is not in the box, so its taps can lie
+            // anywhere -- far outside the window and the CTA's shared memory when the flow moves the tile's taps far.  It
+            // reads the window's first words instead; its result is never stored.
+            a00[q] = ok[q] ? offa[q] : 0;
+            a01[q] = a00[q] + dxs[q];
+            a10[q] = a00[q] + dys[q] * pitch;
+            a11[q] = a10[q] + dxs[q];
             ooff[q] = (unsigned)(i * W + j);
         }
 #pragma unroll

@@ -86,6 +86,7 @@ def test_spatial_transformation_backward_matches_reference_autograd(golden_dir):
         if name + "_gm" not in ref:
             continue
         g = torch.from_numpy(upstream(name, mv.shape)).cuda()
+        om, of = oracle.warp_torch_backward_restated(mv, fl, g.cpu().numpy())
         for variant in ("interleaved", "planar_view", "nhwc"):
             m = torch.from_numpy(mv).cuda().requires_grad_(True)
             if variant == "planar_view":
@@ -96,10 +97,25 @@ def test_spatial_transformation_backward_matches_reference_autograd(golden_dir):
             out = SpatialTransformation(True, nhwc_memory=(variant == "nhwc"))(m, f)
             out.backward(g)
             gf = base.grad.permute(0, 2, 3, 1) if variant == "planar_view" else base.grad
-            for got, want in ((m.grad, ref[name + "_gm"]), (gf, ref[name + "_gf"])):
+            for got, want in ((m.grad, ref[name + "_gm"]), (gf, ref[name + "_gf"]), (m.grad, om), (gf, of)):
                 assert np.abs(got.cpu().numpy() - want).max() <= 2e-5 * max(1.0, np.abs(want).max()), (name, variant)
-        om, of = oracle.warp_torch_backward_restated(mv, fl, g.cpu().numpy())
-        assert np.abs(m.grad.cpu().numpy() - om).max() <= 2e-5 * max(1.0, np.abs(om).max())
+
+
+@pytest.mark.parametrize("kind", ["fold", "noise2"])
+def test_spatial_transformation_backward_through_a_planar_view_at_512(kind):
+    """Both gradients at 1x3x512^2 through the planar flow view every reference call site passes, against the oracle."""
+    from sstem_restoration_b200 import SpatialTransformation, synth
+    H = W = 512
+    fl = (synth.random_fold_flow(H, W, 555)[0] if kind == "fold" else synth.noise_flow(H, W, 2.0, seed=7))[None]
+    r = np.random.default_rng(512)
+    mv = r.random((1, 3, H, W), dtype=np.float32)
+    g = r.standard_normal((1, 3, H, W)).astype(np.float32)
+    m = torch.from_numpy(mv).cuda().requires_grad_(True)
+    base = torch.from_numpy(np.ascontiguousarray(fl.transpose(0, 3, 1, 2))).cuda().requires_grad_(True)
+    SpatialTransformation(True)(m, base.permute(0, 2, 3, 1)).backward(torch.from_numpy(g).cuda())
+    om, of = oracle.warp_torch_backward_restated(mv, fl, g)
+    for got, want in ((m.grad, om), (base.grad.permute(0, 2, 3, 1), of)):
+        assert np.abs(got.cpu().numpy() - want).max() <= 2e-5 * max(1.0, np.abs(want).max())
 
 
 def test_spatial_transformation_backward_only_what_is_needed():
