@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define SSTEM_ABI_VERSION 4
+#define SSTEM_ABI_VERSION 5
 
 /* argument errors (negative) */
 #define SSTEM_E_NULL      (-1)  /* a required pointer is NULL */
@@ -342,6 +342,28 @@ int64_t sstem_tap_conv3x3_packed_elems(void);
 int sstem_tap_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream);
 int sstem_tap_conv3x3(const float* x, const float* packed_weight, const float* bias, float* out,
                       int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream);
+
+/*
+ * Backward of the tap producer, y = conv3x3(up(x), W) + b as in sstem_tap_conv3x3 (for training IFNet with the producer
+ * in the graph).  grad_out is [B,cout,H,W], or tile-major with SSTEM_TAPCONV_TILED (cout == 51: the tap gradients
+ * sstem_sepconv_backward_tiled returns; entries outside the image are never read).  Each non-NULL output is overwritten:
+ *
+ *   grad_x       [B, cin, h, w]      up^T(conv3x3(grad_out, W')), W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]: the forward's
+ *                                    tcgen05 convolution on W' (packed by sstem_tap_conv3x3_pack_weights_adjoint into
+ *                                    sstem_tap_conv3x3_packed_elems() floats), then the adjoint of the align_corners upsample
+ *                                    as a gather with the forward's float32 indices and weights (no atomics)
+ *   grad_weight  [cout, cin, 3, 3]   sum over pixels of grad_out x up(x) shifted per tap: a persistent tcgen05 TF32 kernel
+ *   grad_bias    [cout]              fp32 sum of grad_out over pixels
+ *
+ * packed_adjoint may be NULL when grad_x is.  cin <= 52, cout <= 52, (cin or cout) * H * W < 2^31.  Operands are rounded to
+ * TF32, sums accumulated in fp32; every gradient is run-to-run bit-identical on a given device, and identical for the
+ * two layouts of grad_out.  Stream-ordered workspaces: B*cin*H*W floats (grad_x with the upsample) and
+ * min(tiles, SMs) * (cout*cin*9 + cout) floats (grad_weight / grad_bias).
+ */
+int sstem_tap_conv3x3_pack_weights_adjoint(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream);
+int sstem_tap_conv3x3_backward(const float* grad_out, const float* x, const float* packed_adjoint,
+                               float* grad_x, float* grad_weight, float* grad_bias,
+                               int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream);
 
 /*
  * Gray x3 detection on the device, without a host round trip.  Every reference caller feeds sepconv a grayscale section

@@ -13,7 +13,7 @@ import threading
 from ._build import LIB_PATH as _DEFAULT_LIB_PATH, needs_build as _needs_build
 
 #: must equal SSTEM_ABI_VERSION of include/sstem_b200.h (checked against the loaded library in load())
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 #: SSTEM_LIB_PATH selects another build of the same library (kernel-tuning experiments)
 LIB_PATH = os.environ.get("SSTEM_LIB_PATH") or _DEFAULT_LIB_PATH
@@ -45,6 +45,7 @@ EXPORTED_SYMBOLS = (
     "sstem_sepconv_backward_tiled", "sstem_taps_from_tiled",
     "sstem_sepconv_forward_detect", "sstem_sepconv_backward_detect",
     "sstem_tap_conv3x3_packed_elems", "sstem_tap_conv3x3_pack_weights", "sstem_tap_conv3x3",
+    "sstem_tap_conv3x3_pack_weights_adjoint", "sstem_tap_conv3x3_backward",
     "sstem_fp32_peak_probe", "sstem_launch_count", "sstem_abi_version", "sstem_error_string",
 )
 
@@ -117,6 +118,10 @@ def load() -> ctypes.CDLL:
         lib.sstem_tap_conv3x3_pack_weights.restype = ctypes.c_int
         lib.sstem_tap_conv3x3.argtypes = [_c_p, _c_p, _c_p, _c_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i64, _c_u32, _c_p]
         lib.sstem_tap_conv3x3.restype = ctypes.c_int
+        lib.sstem_tap_conv3x3_pack_weights_adjoint.argtypes = [_c_p, _c_p, _c_i32, _c_i32, _c_p]
+        lib.sstem_tap_conv3x3_pack_weights_adjoint.restype = ctypes.c_int
+        lib.sstem_tap_conv3x3_backward.argtypes = [_c_p] * 6 + [_c_i64, _c_i32, _c_i32, _c_i64, _c_i64, _c_u32, _c_p]
+        lib.sstem_tap_conv3x3_backward.restype = ctypes.c_int
         lib.sstem_fp32_peak_probe.argtypes = [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
         lib.sstem_fp32_peak_probe.restype = ctypes.c_int
         lib.sstem_launch_count.argtypes = []

@@ -22,6 +22,8 @@
 //     mbarriers between them, a persistent grid of one CTA per SM.
 // Shared memory bandwidth bounds the kernel (each MMA reads 4 KB of A and 2 KB of W for 65 536 FMAs); see DESIGN 4.11
 // and profiles/tapconv_r2.md.
+// The backward (sstem_tap_conv3x3_backward, DESIGN 4.11b) is at the end of this file: the input gradient reuses this kernel
+// on the adjoint weights, the weight gradient is tap_conv3x3_wgrad_kernel.
 #include <string.h>
 
 #include <algorithm>
@@ -118,9 +120,13 @@ __device__ __forceinline__ float lds_f32(unsigned addr) {
     return v;
 }
 
-// UPS: fold the x2 upsample into the producer.  WVEC (UPS only): w % 4 == 0 and x is 16-byte aligned, so the source
-// window is fetched with 16-byte loads; otherwise element by element.
-// FULL: cin is 49..52, i.e. all 13 chunks exist -- the MMA and blend loops then have no per-chunk checks.
+// UPS: fold the x2 upsample into the producer.  WVEC with UPS: w % 4 == 0 and x is 16-byte aligned, so the source
+// window is fetched with 16-byte loads; otherwise element by element.  WVEC without UPS: x is tile-major,
+// [B][ceil(h/8)][ceil(w/8)][51][8][8] (cin == 51; the tap gradients of the tiled consumer, read by the input gradient of
+// sstem_tap_conv3x3_backward); entries outside the image are never read.  The one flag serves both so that the
+// existing instantiations keep their symbols and code.
+// TILED: the output is tile-major.  FULL: cin is 49..52, i.e. all 13 chunks exist -- the MMA and blend loops then have
+// no per-chunk checks.
 template <bool UPS, bool TILED, bool WVEC, bool FULL>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacked,
@@ -324,7 +330,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
         // WVEC: which 16-byte piece this thread fetches in round k does not depend on the tile: its channel offset (elements;
         // the host checks cin * h * w < 2^31), window row and column piece are computed once
         int f_choff[WVEC ? NFILL : 1], f_wy[WVEC ? NFILL : 1], f_c4[WVEC ? NFILL : 1], f_dst[WVEC ? NFILL : 1];
-        if (WVEC) {
+        if (UPS && WVEC) {
 #pragma unroll
             for (int k = 0; k < NFILL; ++k) {
                 const int i = ptid + k * TC_PROD_THREADS;
@@ -428,7 +434,25 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
             } else {
                 const float* xb = x + (int64_t)b * sh.cin * src_plane;
                 tc_wait(b_aempty + 8 * s, ph ^ 1);
-                if (has_pixel) {
+                if (WVEC && has_pixel) {                   // tile-major input: channel stride 64, cin == 51 (13 chunks)
+                    const int Yc = min(max(Y, 0), sh.H - 1), Xc = min(max(X, 0), sh.W - 1);
+                    const float* xp = x + ((((int64_t)b * ((sh.H + 7) >> 3) + (Yc >> 3)) * ((sh.W + 7) >> 3) + (Xc >> 3)) * (51 * 64) +
+                                           (Yc & 7) * 8 + (Xc & 7));
+#pragma unroll 1
+                    for (int ck0 = half; ck0 < nchunks; ck0 += 8) {
+                        const unsigned dst0 = a_dst - half_dst;
+                        float q[16];
+#pragma unroll
+                        for (int j = 0; j < 16; ++j) {
+                            const int ch = (ck0 + 2 * (j >> 2)) * 4 + (j & 3);
+                            q[j] = (inside && ch < sh.cin) ? __ldg(xp + ch * 64) : 0.f;
+                        }
+#pragma unroll
+                        for (int c4 = 0; c4 < 4; ++c4)
+                            if (ck0 + 2 * c4 < nchunks)
+                                sts128(dst0 + (ck0 + 2 * c4) * TC_NPIX * 16, to_tf32(q[4 * c4]), to_tf32(q[4 * c4 + 1]), to_tf32(q[4 * c4 + 2]), to_tf32(q[4 * c4 + 3]));
+                    }
+                } else if (has_pixel) {
                     const float* xp = xb + (int64_t)min(max(Y, 0), sh.H - 1) * sh.W + min(max(X, 0), sh.W - 1);
 #pragma unroll 1
                     for (int ck0 = half; ck0 < nchunks; ck0 += 8) {    // chunks half, half + 2, ...: 16 independent loads in flight per thread
@@ -478,6 +502,289 @@ int launch_tap_conv(const float* x, const float* wpacked, const float* bias, flo
     }
     const int ctas = std::min(sh.ntiles, sm_count());
     kern<<<ctas, TC_THREADS, TC_SMEM, s>>>(x, wpacked, bias, out, sh);
+    count_launch();
+    return finish_launch();
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Backward of y = conv3x3(up(x), W) + b (sstem_tap_conv3x3_backward).
+//
+// grad_x = up^T(conv3x3(gy, W')), W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]: the convolution is tap_conv3x3_kernel on its
+// no-upsample path (weights packed by tap_conv3x3_pack_adjoint_kernel), up^T is the gather below.
+
+// W [cout][cin][3][3] -> the packed image of W' (a convolution from cout to cin channels), rounded to TF32
+__global__ void tap_conv3x3_pack_adjoint_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int)(TC_W_BYTES / 4)) return;
+    if (i >= (int)(TC_W_ZERO_OFF / 4)) { packed[i] = 0.f; return; }
+    const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % TC_WCHUNKS, tap = (i >> 2) / TC_N / TC_WCHUNKS;
+    const int co = ck * 4 + j;                             // input channel of the adjoint = output channel of the layer
+    packed[i] = (n < cin && co < cout) ? to_tf32(w[((int64_t)co * cin + n) * 9 + (8 - tap)]) : 0.f;
+}
+
+// Weight with which output row (column) Y of the align_corners upsample reads source row i: ATen's float32 index and
+// fraction, as the forward producer computes them.  At the last row the neighbour is the row itself (both weights land
+// on it); with one source row the scale is 0 and every output row reads row 0.
+__device__ __forceinline__ float up_adjoint_weight(int Y, int i, int n_in, int n_out, float r) {
+    if (Y < 0 || Y >= n_out) return 0.f;
+    const float fr = r * (float)Y;
+    const int i0 = (int)fr, i1 = i0 + (i0 < n_in - 1 ? 1 : 0);
+    const float l1 = fr - (float)i0, l0 = 1.f - l1;
+    return (i0 == i ? l0 : 0.f) + (i1 == i ? l1 : 0.f);
+}
+
+// grad_x[p][i][j] = sum_Y sum_X wy(Y, i) wx(X, j) gU[p][Y][X] as a gather (no atomics: deterministic).  The output rows that
+// read source row i lie in [2i - 3, 2i + 4] (the scale (h - 1) / (2h - 1) is just below 1/2); weights of rows that do not
+// read it are 0 and skip their loads.
+__global__ void __launch_bounds__(256)
+upsample2x_adjoint_kernel(const float* __restrict__ gU, float* __restrict__ gx, int64_t n, int h, int w, int H, int W,
+                          float ry, float rx) {
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= n) return;
+    const int j = (int)(idx % w), i = (int)(idx / w % h);
+    const float* g = gU + idx / ((int64_t)h * w) * ((int64_t)H * W);
+    float wx[8];
+#pragma unroll
+    for (int d = 0; d < 8; ++d) wx[d] = up_adjoint_weight(2 * j - 3 + d, j, w, W, rx);
+    float acc = 0.f;
+#pragma unroll
+    for (int dy = 0; dy < 8; ++dy) {
+        const int Y = 2 * i - 3 + dy;
+        const float wy = up_adjoint_weight(Y, i, h, H, ry);
+        if (wy == 0.f) continue;
+        float row = 0.f;
+#pragma unroll
+        for (int dx = 0; dx < 8; ++dx)
+            if (wx[dx] != 0.f) row += wx[dx] * __ldg(g + (int64_t)Y * W + (2 * j - 3 + dx));
+        acc += wy * row;
+    }
+    gx[idx] = acc;
+}
+
+// grad_weight / grad_bias.  Per output tile of 16 x 8 pixels and tap (dy, dx):
+//     D_tap[co][ci] += sum_{pixels p} gy[co][p] * U[ci][p + (dy, dx)]            (U = up(x), zero padded by 1)
+// as tcgen05.mma kind::tf32, M = 64 (co, padded), N = 56 (ci, padded), K = 8 = one row of the tile: 16 K-steps x 9 taps =
+// 144 MMAs per tile, the nine accumulators (9 x 56 = 504 TMEM columns) resident for the whole tile loop.  Both operands
+// are K-major, no swizzle (the encoding tapconv's forward and tools/microbench/umma_probe.cu pin down):
+//   * A = gy of the tile: [tile row][K half][co group of 8][8 co][4 pixels], one K-step = one tile row (2 KB);
+//   * B = the upsampled, TF32-rounded 18 x 10 patch, recomputed from x, as three copies shifted by dx = 0, 1, 2 columns:
+//     [dx][patch row][K half][ci group of 8][8 ci][4 pixels].  Tap (dy, dx), K-step ky reads copy dx at patch row
+//     ky + dy: a start-address shift of one 1792-byte row per dy.
+// One stage: all 12 warps stage a tile, warp 0 issues its 144 MMAs, and the staging of the next tile waits for their
+// completion (tcgen05.commit).  gy is summed per output channel on the way (grad_bias).  Each CTA writes one partial of
+// both gradients at the end; tap_conv3x3_wgrad_reduce_kernel sums the partials over CTAs in a fixed order, so the result
+// is run-to-run bit-identical.
+constexpr int WG_THREADS = 384;
+constexpr int WG_M = 64, WG_N = 56;
+constexpr int WG_CO_PER_THREAD = 18;                       // output channels cgrp, cgrp + 3, ..., cgrp + 51 (cout <= 52)
+constexpr unsigned WG_A_ROW = 2 * (WG_M / 8) * 128;        // 2048
+constexpr unsigned WG_A_BYTES = TC_TH * WG_A_ROW;          // 32768
+constexpr unsigned WG_B_ROW = 2 * (WG_N / 8) * 128;        // 1792
+constexpr unsigned WG_B_COPY = TC_PH * WG_B_ROW;           // 32256
+constexpr unsigned WG_OFF_B = WG_A_BYTES;
+constexpr unsigned WG_OFF_BAR = WG_OFF_B + 3 * WG_B_COPY;  // 129536
+constexpr unsigned WG_SMEM = WG_OFF_BAR + 16 + 128;
+constexpr unsigned WG_TMEM_COLS = 512;
+static_assert(9 * WG_N <= (int)WG_TMEM_COLS, "nine accumulators in tensor memory");
+static_assert(WG_THREADS * WG_CO_PER_THREAD * 4 <= WG_OFF_BAR, "the bias reduction reuses the operand buffers");
+
+template <bool UPS, bool TILED>
+__global__ void __launch_bounds__(WG_THREADS, 1)
+tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__ x, float* __restrict__ part_w,
+                         float* __restrict__ part_b, const TapConvShape sh) {
+    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
+    const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
+    unsigned char* gen = tc_smem_raw + (base - (unsigned)__cvta_generic_to_shared(tc_smem_raw));
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const unsigned bar = base + WG_OFF_BAR;
+    volatile unsigned* tmem_slot = reinterpret_cast<volatile unsigned*>(gen + WG_OFF_BAR + 8);
+    if (tid == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
+        mbar_fence_init();
+    }
+    // padding rows / columns of both operands stay zero
+    for (unsigned i = tid; i < WG_OFF_BAR / 16; i += WG_THREADS) sts128(base + i * 16, 0.f, 0.f, 0.f, 0.f);
+    if (warp == 0) {
+        __syncwarp();
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(bar + 8), "n"(WG_TMEM_COLS));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const unsigned tmem = *tmem_slot;
+
+    // A staging: thread = (tile pixel, output-channel class); B staging: thread = (patch pixel, input-channel half)
+    const int apx = tid & 127, acg = tid >> 7, ay = apx >> 3, ax = apx & 7;
+    const unsigned a_dst = base + (unsigned)(ay * 2 + (ax >> 2)) * 8 * 128 + (ax & 3) * 4;
+    const bool bitem = tid < 2 * TC_NPIX;
+    const int bhalf = tid >= TC_NPIX ? 1 : 0, bpix = tid - bhalf * TC_NPIX, bpy = bpix / TC_PW, bpx = bpix % TC_PW;
+    const int64_t plane = (int64_t)sh.H * sh.W, src_plane = (int64_t)sh.h * sh.w;
+    const int tiles_y8 = (sh.H + 7) / 8, tiles_x8 = (sh.W + 7) / 8;
+    float bacc[WG_CO_PER_THREAD];
+#pragma unroll
+    for (int k = 0; k < WG_CO_PER_THREAD; ++k) bacc[k] = 0.f;
+    // D = f32, A = B = tf32, both K-major, N = 56, M = 64
+    constexpr unsigned idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(WG_N >> 3) << 17) | ((unsigned)(WG_M >> 4) << 24);
+
+    int it = 0;
+    for (int tile = blockIdx.x; tile < sh.ntiles; tile += gridDim.x, ++it) {
+        const int r = tile / sh.tiles_x, tx = tile - r * sh.tiles_x, b = r / sh.tiles_y, ty = r - b * sh.tiles_y;
+        const int Y0 = ty * TC_TH, X0 = tx * TC_TW;
+        if (it > 0) {
+            tc_wait(bar, (it - 1) & 1);                    // the MMAs of the previous tile have read the operands
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        }
+        {   // A: gy of the tile, and its per-channel sum
+            const int Y = Y0 + ay, X = X0 + ax;
+            const bool inside = Y < sh.H && X < sh.W;
+            const float* g = TILED ? gy + ((((int64_t)b * tiles_y8 + (Y >> 3)) * tiles_x8 + (X >> 3)) * (51 * 64) + (Y & 7) * 8 + (X & 7))
+                                   : gy + (int64_t)b * sh.cout * plane + (int64_t)Y * sh.W + X;
+            const int64_t cstride = TILED ? 64 : plane;
+#pragma unroll
+            for (int k = 0; k < WG_CO_PER_THREAD; ++k) {
+                const int co = acg + 3 * k;
+                const float v = (inside && co < sh.cout) ? __ldg(g + co * cstride) : 0.f;
+                bacc[k] += v;
+                if (co < WG_M) asm volatile("st.shared.f32 [%0], %1;" ::"r"(a_dst + (co >> 3) * 128 + (co & 7) * 16), "f"(to_tf32(v)) : "memory");
+            }
+        }
+        if (bitem) {   // B: the upsampled patch pixel, written into the (up to) three shifted copies that hold it
+            const int Y = Y0 - 1 + bpy, X = X0 - 1 + bpx;
+            const bool inside = Y >= 0 && Y < sh.H && X >= 0 && X < sh.W;
+            int o00 = 0, o01 = 0, o10 = 0, o11 = 0;
+            float wa = 0.f, wb = 0.f, wc = 0.f, wd = 0.f;
+            if (UPS && inside) {
+                const float h1r = sh.ry * (float)Y, w1r = sh.rx * (float)X;
+                const int h1 = (int)h1r, w1 = (int)w1r;
+                const int h1p = h1 < sh.h - 1 ? 1 : 0, w1p = w1 < sh.w - 1 ? 1 : 0;
+                const float h1l = h1r - (float)h1, h0l = 1.f - h1l, w1l = w1r - (float)w1, w0l = 1.f - w1l;
+                wa = h0l * w0l; wb = h0l * w1l; wc = h1l * w0l; wd = h1l * w1l;
+                o00 = h1 * sh.w + w1; o01 = o00 + w1p; o10 = o00 + h1p * sh.w; o11 = o10 + w1p;
+            } else if (inside) {
+                o00 = Y * sh.w + X;
+            }
+            const float* xb = x + (int64_t)b * sh.cin * src_plane;
+            const unsigned bdst = base + WG_OFF_B + bpy * WG_B_ROW;
+#pragma unroll 4
+            for (int k = 0; k < WG_N / 2; ++k) {
+                const int ci = bhalf * (WG_N / 2) + k;
+                float v = 0.f;
+                if (inside && ci < sh.cin) {
+                    const float* p = xb + ci * src_plane;
+                    v = UPS ? wa * __ldg(p + o00) + wb * __ldg(p + o01) + wc * __ldg(p + o10) + wd * __ldg(p + o11) : __ldg(p + o00);
+                }
+                v = to_tf32(v);
+#pragma unroll
+                for (int dx = 0; dx < 3; ++dx) {
+                    const int c = bpx - dx;
+                    if (c >= 0 && c < TC_TW)
+                        asm volatile("st.shared.f32 [%0], %1;" ::"r"(bdst + dx * WG_B_COPY + ((c >> 2) * (WG_N / 8) + (ci >> 3)) * 128 + (ci & 7) * 16 + (c & 3) * 4),
+                                     "f"(v) : "memory");
+                }
+            }
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy stores -> visible to the tensor core
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncthreads();
+        if (warp == 0) {
+            // the whole warp walks the loop (descriptors in uniform registers), one lane issues
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const uint64_t da0 = tc_desc(base, WG_A_ROW / 2, 128);
+            const uint64_t db0 = tc_desc(base + WG_OFF_B, WG_B_ROW / 2, 128);
+#pragma unroll 1
+            for (int tap = 0; tap < 9; ++tap) {
+                const int dy = tap / 3, dx = tap % 3;
+                const unsigned d_tmem = tmem + tap * WG_N;
+#pragma unroll
+                for (int ky = 0; ky < TC_TH; ++ky) {
+                    const uint64_t da = da0 + (uint64_t)((ky * WG_A_ROW) >> 4);
+                    const uint64_t db = db0 + (uint64_t)((dx * WG_B_COPY + (ky + dy) * WG_B_ROW) >> 4);
+                    if (lane == 0)
+                        asm volatile(
+                            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+                            "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+                            ::"r"(d_tmem), "l"(da), "l"(db), "r"(idesc), "r"((unsigned)((it | ky) != 0)) : "memory");
+                }
+            }
+            __syncwarp();
+            if (lane == 0) tc_commit(bar);
+            __syncwarp();
+        }
+    }
+    if (it > 0) {
+        tc_wait(bar, (it - 1) & 1);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    }
+    __syncthreads();
+
+    const int nw = sh.cout * sh.cin * 9;
+    if (warp < 4) {
+        // M = 64: row m of D is TMEM lane 32 (m / 16) + m % 16 (tools/microbench/umma_probe.cu, mode m64), so warp q reads
+        // rows 16 q .. 16 q + 15 in its lanes 0..15
+        const int co = warp * 16 + lane;
+        const bool mine = lane < 16 && co < sh.cout;
+        float* pw = part_w + (int64_t)blockIdx.x * nw + (int64_t)co * sh.cin * 9;
+#pragma unroll 1
+        for (int tap = 0; tap < 9; ++tap) {
+#pragma unroll 1
+            for (int c8 = 0; c8 < WG_N; c8 += 8) {
+                unsigned v[8];
+                asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                             : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+                             : "r"(tmem + ((unsigned)(warp * 32) << 16) + tap * WG_N + c8));
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                if (mine) {
+#pragma unroll
+                    for (int j = 0; j < 8; ++j)
+                        if (c8 + j < sh.cin) pw[(c8 + j) * 9 + tap] = __uint_as_float(v[j]);
+                }
+            }
+        }
+    }
+    // grad_bias partial: thread sums in shared memory (the operand buffers are free), then per channel in pixel order
+    float* red = reinterpret_cast<float*>(gen);
+#pragma unroll
+    for (int k = 0; k < WG_CO_PER_THREAD; ++k) red[tid * WG_CO_PER_THREAD + k] = bacc[k];
+    __syncthreads();
+    if (tid < sh.cout) {
+        const int cg = tid % 3, k = tid / 3;
+        float sum = 0.f;
+        for (int p = 0; p < 128; ++p) sum += red[(cg * 128 + p) * WG_CO_PER_THREAD + k];
+        part_b[(int64_t)blockIdx.x * sh.cout + tid] = sum;
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(WG_TMEM_COLS));
+}
+
+// sum of the per-CTA partials in CTA order (deterministic); out[i] for i < n, NULL outputs skipped
+__global__ void tap_conv3x3_wgrad_reduce_kernel(const float* __restrict__ part_w, const float* __restrict__ part_b,
+                                                float* __restrict__ gw, float* __restrict__ gb, int nw, int nb, int parts) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const float* src;
+    float* dst;
+    int n;
+    if (i < nw) { src = part_w + i; dst = gw ? gw + i : nullptr; n = nw; }
+    else if (i < nw + nb) { src = part_b + (i - nw); dst = gb ? gb + (i - nw) : nullptr; n = nb; }
+    else return;
+    if (!dst) return;
+    float s = 0.f;
+    for (int c = 0; c < parts; ++c) s += src[(int64_t)c * n];
+    *dst = s;
+}
+
+template <bool UPS, bool TILED>
+int launch_wgrad(const float* gy, const float* x, float* part_w, float* part_b, const TapConvShape& sh, int ctas, cudaStream_t s) {
+    static PerDeviceOnce done;
+    auto kern = tap_conv3x3_wgrad_kernel<UPS, TILED>;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (!done.test(dev)) {
+        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WG_SMEM) != cudaSuccess) return (int)cudaGetLastError();
+        done.set(dev);
+    }
+    kern<<<ctas, WG_THREADS, WG_SMEM, s>>>(gy, x, part_w, part_b, sh);
     count_launch();
     return finish_launch();
 }
@@ -538,4 +845,86 @@ extern "C" int sstem_tap_conv3x3(const float* x, const float* packed_weight, con
     }
     SSTEM_TC_LAUNCH(false, false);
 #undef SSTEM_TC_LAUNCH
+}
+
+extern "C" int sstem_tap_conv3x3_pack_weights_adjoint(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
+    if (!weight || !packed) return SSTEM_E_NULL;
+    if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > TC_MAXC) return SSTEM_E_SHAPE;
+    if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
+    DeviceGuard guard(packed);
+    if (guard.err) return guard.err;
+    const int total = (int)(TC_W_BYTES / 4);
+    tap_conv3x3_pack_adjoint_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(weight, packed, cin, cout);
+    count_launch();
+    return finish_launch();
+}
+
+extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x, const float* packed_adjoint,
+                                          float* grad_x, float* grad_weight, float* grad_bias,
+                                          int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream) {
+    if (!grad_out || !x || (grad_x && !packed_adjoint)) return SSTEM_E_NULL;
+    if (flags & ~(SSTEM_TAPCONV_UPSAMPLE2X | SSTEM_TAPCONV_TILED)) return SSTEM_E_FLAG;
+    const bool ups = flags & SSTEM_TAPCONV_UPSAMPLE2X, tiled = flags & SSTEM_TAPCONV_TILED;
+    if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
+    if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > TC_MAXC) return SSTEM_E_SHAPE;
+    if (tiled && cout != 51) return SSTEM_E_SHAPE;
+    if (!aligned4(grad_out) || !aligned4(x) || (packed_adjoint && !aligned16(packed_adjoint)) || (grad_x && !aligned4(grad_x)) ||
+        (grad_weight && !aligned4(grad_weight)) || (grad_bias && !aligned4(grad_bias)))
+        return SSTEM_E_ALIGN;
+    const int64_t H = ups ? 2 * h : h, W = ups ? 2 * w : w;
+    const int64_t nt = ((W + TC_TW - 1) / TC_TW) * ((H + TC_TH - 1) / TC_TH) * B;
+    if (nt > INT32_MAX / 2 || (int64_t)cout * H * W > INT32_MAX || (int64_t)cin * H * W > INT32_MAX) return SSTEM_E_SHAPE;
+    if (!grad_x && !grad_weight && !grad_bias) return 0;
+    DeviceGuard guard(grad_out);
+    if (guard.err) return guard.err;
+    cudaStream_t s = (cudaStream_t)stream;
+    TapConvShape sh;
+    sh.B = (int)B; sh.H = (int)H; sh.W = (int)W;
+    sh.tiles_x = (int)((W + TC_TW - 1) / TC_TW);
+    sh.tiles_y = (int)((H + TC_TH - 1) / TC_TH);
+    sh.ntiles = (int)nt;
+    sh.ry = ups && H > 1 ? (float)(h - 1) / (float)(H - 1) : 0.f;
+    sh.rx = ups && W > 1 ? (float)(w - 1) / (float)(W - 1) : 0.f;
+
+    if (grad_x) {
+        // gU = conv3x3(gy, W'), cout -> cin channels at full resolution; with the upsample into a workspace, then up^T
+        TapConvShape sd = sh;
+        sd.cin = cout; sd.cout = cin; sd.h = (int)H; sd.w = (int)W;
+        sd.k_steps = (cout + 7) / 8;
+        float* gU = grad_x;
+        if (ups && workspace_alloc(reinterpret_cast<void**>(&gU), (size_t)(B * cin * H * W) * sizeof(float), s)) return cudaErrorMemoryAllocation;
+        int e;
+        if (tiled) e = launch_tap_conv<false, false, true, true>(grad_out, packed_adjoint, nullptr, gU, sd, s);
+        else if (cout > 48) e = launch_tap_conv<false, false, false, true>(grad_out, packed_adjoint, nullptr, gU, sd, s);
+        else e = launch_tap_conv<false, false, false, false>(grad_out, packed_adjoint, nullptr, gU, sd, s);
+        if (!e && ups) {
+            const int64_t n = B * cin * h * w;
+            upsample2x_adjoint_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(gU, grad_x, n, (int)h, (int)w, (int)H, (int)W, sh.ry, sh.rx);
+            count_launch();
+            e = finish_launch();
+        }
+        if (ups) cudaFreeAsync(gU, s);
+        if (e) return e;
+    }
+    if (grad_weight || grad_bias) {
+        sh.cin = cin; sh.cout = cout; sh.h = (int)h; sh.w = (int)w;
+        sh.k_steps = 0;
+        const int ctas = std::min(sh.ntiles, sm_count());
+        const int nw = cout * cin * 9;
+        float* part = nullptr;
+        if (workspace_alloc(reinterpret_cast<void**>(&part), (size_t)ctas * (nw + cout) * sizeof(float), s)) return cudaErrorMemoryAllocation;
+        float* part_b = part + (size_t)ctas * nw;
+        int e = ups ? (tiled ? launch_wgrad<true, true>(grad_out, x, part, part_b, sh, ctas, s)
+                             : launch_wgrad<true, false>(grad_out, x, part, part_b, sh, ctas, s))
+                    : (tiled ? launch_wgrad<false, true>(grad_out, x, part, part_b, sh, ctas, s)
+                             : launch_wgrad<false, false>(grad_out, x, part, part_b, sh, ctas, s));
+        if (!e) {
+            tap_conv3x3_wgrad_reduce_kernel<<<(nw + cout + 255) / 256, 256, 0, s>>>(part, part_b, grad_weight, grad_bias, nw, cout, ctas);
+            count_launch();
+            e = finish_launch();
+        }
+        cudaFreeAsync(part, s);
+        if (e) return e;
+    }
+    return 0;
 }

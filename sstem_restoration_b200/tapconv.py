@@ -4,8 +4,9 @@
 
 (sff_scripts_interp/model/model_interp.py:18, 130-137; four instances, :34-37, run at :86-89) as one sm_100a kernel
 (csrc/tapconv.cu: tcgen05 TF32 implicit GEMM, the upsample folded into the operand producer), writing the taps in the
-layout of ``Conv2d`` or directly tile-major for :func:`sstem_restoration_b200.sepconv_forward_tiled`.  Forward only
-(the stack-restoration path, c5); no CPU / PyTorch fallback.
+layout of ``Conv2d`` or directly tile-major for :func:`sstem_restoration_b200.sepconv_forward_tiled`.
+:func:`tap_conv3x3` is forward only (the stack-restoration path, c5); :class:`TapConv3x3Function` and
+``ModuleTapProducer(trainable=True)`` add the backward (tcgen05 kernels as well) for training.  No CPU / PyTorch fallback.
 """
 import torch
 
@@ -32,6 +33,24 @@ def pack_tap_conv_weight(weight: torch.Tensor) -> torch.Tensor:
     if code:
         _lib.check(code, "sstem_tap_conv3x3_pack_weights")
     packed._sstem_cin_cout = (int(cin), int(cout))
+    return packed
+
+
+def pack_tap_conv_weight_adjoint(weight: torch.Tensor) -> torch.Tensor:
+    """``Conv2d.weight`` ``[cout<=52, cin<=52, 3, 3]`` -> the resident image of the adjoint convolution's weight
+    ``W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]`` (cout -> cin channels), which the input gradient runs."""
+    if weight.is_cuda == False:
+        raise NotImplementedError()
+    if weight.dtype != torch.float32 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3):
+        raise TypeError("pack_tap_conv_weight_adjoint: float32 [cout, cin, 3, 3] required")
+    cout, cin = weight.shape[:2]
+    if cin > 52 or cout > 52:
+        raise ValueError("pack_tap_conv_weight_adjoint: cin <= 52 and cout <= 52 required")
+    lib = _lib.load()
+    packed = torch.empty(lib.sstem_tap_conv3x3_packed_elems(), dtype=torch.float32, device=weight.device)
+    code = lib.sstem_tap_conv3x3_pack_weights_adjoint(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
+    if code:
+        _lib.check(code, "sstem_tap_conv3x3_pack_weights_adjoint")
     return packed
 
 
@@ -71,22 +90,76 @@ def tap_conv3x3(x: torch.Tensor, packed_weight: torch.Tensor, bias=None, cin=Non
     return out
 
 
+class TapConv3x3Function(torch.autograd.Function):
+    """``conv2d(upsample2x(x), weight, bias, padding 1)`` with its backward, over the raw ``Conv2d`` ``weight`` ``[cout, cin, 3,
+    3]`` (cin, cout <= 52) and ``bias`` (or None):
+
+        TapConv3x3Function.apply(x, weight, bias, upsample=True, tiled=False, packed=None, packed_adjoint=None)
+
+    ``tiled=True`` (cout == 51) returns the tile-major taps of :func:`tap_conv3x3`, and the backward then takes their
+    gradient tile-major, as :class:`SeparableConvolutionTiled` / :class:`ModuleInterpolationTailTiled` return it.
+    ``packed`` / ``packed_adjoint``: images of ``weight`` from :func:`pack_tap_conv_weight` /
+    :func:`pack_tap_conv_weight_adjoint`, packed here when not given.  The gradients are TF32 (the reference layer's
+    precision under torch's default ``allow_tf32``), deterministic; inputs that need none get ``None``."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias=None, upsample=True, tiled=False, packed=None, packed_adjoint=None):
+        if packed is None:
+            packed = pack_tap_conv_weight(weight.detach())
+        if packed_adjoint is None and ctx.needs_input_grad[0]:
+            packed_adjoint = pack_tap_conv_weight_adjoint(weight.detach())
+        cout, cin = weight.shape[:2]
+        y = tap_conv3x3(x, packed, None if bias is None else bias.detach(), cin=cin, cout=cout, upsample=upsample, tiled=tiled)
+        ctx.save_for_backward(x)
+        ctx.packed_adjoint, ctx.upsample, ctx.tiled, ctx.cin_cout, ctx.has_bias = packed_adjoint, upsample, tiled, (cin, cout), bias is not None
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        (x,) = ctx.saved_tensors
+        cin, cout = ctx.cin_cout
+        need_x, need_w, need_b = ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.has_bias and ctx.needs_input_grad[2]
+        gx = torch.empty_like(x) if need_x else None
+        gw = torch.empty((cout, cin, 3, 3), dtype=torch.float32, device=x.device) if need_w else None
+        gb = torch.empty(cout, dtype=torch.float32, device=x.device) if need_b else None
+        if (need_x or need_w or need_b) and x.numel():
+            gy = gy.contiguous()
+            B, _, h, w = x.shape
+            flags = (_lib.TAPCONV_UPSAMPLE2X if ctx.upsample else 0) | (_lib.TAPCONV_TILED if ctx.tiled else 0)
+            ptr = lambda t: None if t is None else t.data_ptr()
+            code = _lib.load().sstem_tap_conv3x3_backward(gy.data_ptr(), x.data_ptr(), ptr(ctx.packed_adjoint) if need_x else None,
+                                                          ptr(gx), ptr(gw), ptr(gb), B, cin, cout, h, w, flags, _stream_ptr(x))
+            if code:
+                _lib.check(code, "sstem_tap_conv3x3_backward")
+        return gx, gw, gb, None, None, None, None
+
+
 class ModuleTapProducer(torch.nn.Module):
     """Drop-in for the tail ``nn.Sequential(upsample, Conv2d(51, 51, 3, 1, 1))`` of ``_kernel_module``: holds ``weight`` /
     ``bias`` under the names of ``nn.Conv2d`` (so the reference layer's state_dict loads), packs the weight on first use
-    and whenever it changes."""
+    and whenever it changes.  Forward only by default (an input that requires grad raises); ``trainable=True`` runs
+    :class:`TapConv3x3Function`, so gradients reach ``x``, ``weight`` and ``bias``."""
 
-    def __init__(self, in_channels=51, out_channels=51, upsample=True, tiled=False):
+    def __init__(self, in_channels=51, out_channels=51, upsample=True, tiled=False, trainable=False):
         super().__init__()
         self.weight = torch.nn.Parameter(torch.empty(out_channels, in_channels, 3, 3))
         self.bias = torch.nn.Parameter(torch.zeros(out_channels))
         torch.nn.init.kaiming_uniform_(self.weight, a=5 ** 0.5)
-        self.upsample, self.tiled = upsample, tiled
+        self.upsample, self.tiled, self.trainable = upsample, tiled, trainable
         self._packed, self._packed_version = None, None
+        self._packed_adjoint, self._packed_adjoint_version = None, None
 
     def forward(self, x):
         key = (self.weight._version, self.weight.data_ptr())
         if self._packed is None or self._packed_version != key or self._packed.device != x.device:
             self._packed = pack_tap_conv_weight(self.weight.detach())
             self._packed_version = key
-        return tap_conv3x3(x, self._packed, self.bias.detach(), upsample=self.upsample, tiled=self.tiled)
+        if not self.trainable:
+            return tap_conv3x3(x, self._packed, self.bias.detach(), upsample=self.upsample, tiled=self.tiled)
+        adjoint = None
+        if torch.is_grad_enabled() and x.requires_grad:
+            if self._packed_adjoint is None or self._packed_adjoint_version != key or self._packed_adjoint.device != x.device:
+                self._packed_adjoint = pack_tap_conv_weight_adjoint(self.weight.detach())
+                self._packed_adjoint_version = key
+            adjoint = self._packed_adjoint
+        return TapConv3x3Function.apply(x, self.weight, self.bias, self.upsample, self.tiled, self._packed, adjoint)
