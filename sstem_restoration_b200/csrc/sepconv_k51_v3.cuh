@@ -52,18 +52,6 @@ struct V3Shape {
     int H, W, tiles_x, tiles_y, ntiles, C, c0;
 };
 
-__device__ __forceinline__ void mbar_expect_tx_a(unsigned bar_addr, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_addr), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_a(unsigned bar_addr, unsigned parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE;\n\t"
-        "bra WAIT_LOOP;\n\t"
-        "DONE:\n\t}" ::"r"(bar_addr), "r"(parity) : "memory");
-}
 // L2 policies: a window row is read by ~14 tile rows within a few tens of microseconds (evict last) and must not be
 // pushed out by the 1.7 GB of taps streaming past it.  The taps keep the normal policy: a warp tile reads 32 bytes of
 // each 64-byte DRAM sector and its neighbour the other half -- marked evict-first the sector was often gone before
@@ -88,16 +76,6 @@ __device__ __forceinline__ void tma_load_3d_a(unsigned dst, const CUtensorMap* m
     asm volatile(
         "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], [%2], %6;"
         ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "l"(policy) : "memory");
-}
-// 1-D bulk copy global -> shared (16-byte aligned, size a multiple of 16), completion on an mbarrier
-__device__ __forceinline__ void bulk_load_a(unsigned dst, const void* src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ float lds_f32(unsigned addr) {
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
-    return v;
 }
 // Ordered variant for the tile-start copies of the tap / gradient buffers: the "memory" clobber keeps the compiler from
 // sinking the load below the TMA request that refills the buffer (it did: the values are first used deep inside the
@@ -264,7 +242,7 @@ __device__ __forceinline__ void bwd3_taps_body(const CUtensorMap& map_in, const 
     if (lead) {
 #pragma unroll
         for (int i = 0; i < 4; ++i)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar0 + 8 * i), "r"(1));
+            mbar_init(bar0 + 8 * i, 1);
         mbar_fence_init();
     }
     __syncwarp();
@@ -285,7 +263,7 @@ __device__ __forceinline__ void bwd3_taps_body(const CUtensorMap& map_in, const 
     unsigned p_cur = 0, p_nxt = 0, p_prv = 0, p_h = 0;
     auto issue_group = [&](unsigned slot, unsigned bar, int b, int y0, int x0, int gi) {
         if (lead) {
-            mbar_expect_tx_a(bar, WIN_BYTES + (WH ? V3_V_BYTES : 0u));
+            mbar_expect_tx(bar, WIN_BYTES + (WH ? V3_V_BYTES : 0u));
             // rows of 60 pixels x 4 floats (CC = 3: 960 contiguous bytes) or x 1 float
             tma_load_3d_a(slot, &map_in, bar, (CC == 3 ? 4 : 1) * x0, y0 + V3_GROUP * gi, b, pol_keep);
             if (WH) {
@@ -297,7 +275,7 @@ __device__ __forceinline__ void bwd3_taps_body(const CUtensorMap& map_in, const 
     };
     auto issue_hg = [&](int b, int y0, int x0) {
         if (lead) {
-            mbar_expect_tx_a(hbar, (WV ? V3_H_BYTES : 0u) + G_BYTES);
+            mbar_expect_tx(hbar, (WV ? V3_H_BYTES : 0u) + G_BYTES);
             if (WV) {                                      // [row][tap][col]
                 if constexpr (TILED) tma_load_5d_a(base + V3_OFF_H, &map_h, hbar, 0, 0, y0 & 7, x0 >> 3, b * tiles_y8 + (y0 >> 3), pol_once);
                 else tma_load_4d_a(base + V3_OFF_H, &map_h, hbar, x0, 0, y0, b, pol_once);
@@ -332,7 +310,7 @@ __device__ __forceinline__ void bwd3_taps_body(const CUtensorMap& map_in, const 
 
         // ---- this tile's horizontal taps and upstream gradient: shared memory -> registers
         float2 h2[NP][NT], gh2[NP][NT], g2[CC][NP];
-        mbar_wait_a(hbar, p_h);
+        mbar_wait(hbar, p_h);
         p_h ^= 1;
         {
             // [row][tap][col]: the lanes of one load sit in banks 8 * ((3 * row + g) mod 4) + pg, one wavefront
@@ -403,7 +381,7 @@ __device__ __forceinline__ void bwd3_taps_body(const CUtensorMap& map_in, const 
             store_gv(V3_GROUP * gi + U - g);
         };
         auto run_group = [&](auto gi_tag, int gi) {
-            mbar_wait_a(b_cur, p_cur);
+            mbar_wait(b_cur, p_cur);
             p_cur ^= 1;
             const unsigned wa = s_cur + lane_win, wl = s_cur + lane_last, vc = s_cur + lane_v, vp = s_prv + lane_v;
             run_step(gi_tag, std::integral_constant<int, 0>{}, gi, wa, wl, vc, vp);
@@ -594,7 +572,7 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
     if (lead) {
 #pragma unroll
         for (int i = 0; i < 3; ++i)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar0 + 8 * i), "r"(1));
+            mbar_init(bar0 + 8 * i, 1);
         mbar_fence_init();
     }
     __syncwarp();
@@ -618,21 +596,21 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
             // tiled: planes 4gi .. 4gi+3 of this warp tile are contiguous (256 bytes each); planes past the 51st do not exist
             // (nothing reads them: rows with fy > 50 are masked at compile time)
             const int nplanes = TILED ? max(0, min(V3_GROUP, K51 - V3_GROUP * gi)) : V3_GROUP;
-            mbar_expect_tx_a(bar, WIN_BYTES + (unsigned)nplanes * (F3_V_BYTES / V3_GROUP));
+            mbar_expect_tx(bar, WIN_BYTES + (unsigned)nplanes * (F3_V_BYTES / V3_GROUP));
             tma_load_3d_a(wslot, &map_in, bar, (CC == 3 ? 4 : 1) * x0, y0 + V3_GROUP * gi, b, pol_keep);
             if (!TILED) tma_load_4d_a(vslot, &map_v, bar, x0, y0, V3_GROUP * gi, b, pol_once);
             else if (nplanes > 0) {
                 const float* src = tl.v + (((int64_t)b * tl.tiles_y8 + y0 / F3_R) * tl.tiles_x8 + x0 / V3_COLS) * (K51 * 64) + gi * (V3_GROUP * 64);
-                bulk_load_a(vslot, src, (unsigned)nplanes * (F3_V_BYTES / V3_GROUP), bar);
+                bulk_load(vslot, src, (unsigned)nplanes * (F3_V_BYTES / V3_GROUP), bar);
             }
         }
     };
     auto issue_h = [&](int b, int y0, int x0) {
         if (lead) {
-            mbar_expect_tx_a(hbar, F3_H_BYTES);
+            mbar_expect_tx(hbar, F3_H_BYTES);
             if (!TILED) tma_load_4d_a(base + F3_OFF_H, &map_h, hbar, x0, 0, y0, b, pol_once);   // [row][tap][col]
-            else bulk_load_a(base + F3_OFF_H, tl.h + (((int64_t)b * tl.tiles_y8 + y0 / F3_R) * tl.tiles_x8 + x0 / V3_COLS) * (K51 * 64),
-                             F3_H_BYTES, hbar);
+            else bulk_load(base + F3_OFF_H, tl.h + (((int64_t)b * tl.tiles_y8 + y0 / F3_R) * tl.tiles_x8 + x0 / V3_COLS) * (K51 * 64),
+                           F3_H_BYTES, hbar);
         }
     };
 
@@ -657,7 +635,7 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
         if (has_next && warp == 0 && lead) s_ticket[tile_no & 1] = atomicAdd(next_tile_counter, 1);
 
         float2 h2[NP][NT], acc[CC][NP];
-        mbar_wait_a(hbar, p_h);
+        mbar_wait(hbar, p_h);
         p_h ^= 1;
         {
             // NCHW taps land as [row][tap][col] (banks 8 * ((3 * row + g) mod 4) + pg: one wavefront per load); the tile-major
@@ -696,7 +674,7 @@ sepconv_fwd_k51_v3_kernel(const __grid_constant__ CUtensorMap map_in, const __gr
             fwd3_step<S, CC>(wa + U * V3_WIN_COLS * PIX, wl + U * V3_WIN_COLS * PIX, va, h2, acc);
         };
         auto run_group = [&](auto gi_tag) {
-            mbar_wait_a(b_a, p_a);
+            mbar_wait(b_a, p_a);
             p_a ^= 1;
             const unsigned wa = w_a + lane_win, wl = w_a + lane_last, vc = v_c + lane_v, vp1 = v_p1 + lane_v, vp2 = v_p2 + lane_v;
             run_step(gi_tag, std::integral_constant<int, 0>{}, wa, wl, vc, vp1, vp2);

@@ -29,11 +29,7 @@
 #include <algorithm>
 
 #include "common.cuh"
-#include "tma.cuh"   // mbar_fence_init
-
-#ifndef SSTEM_TC_DIAG
-#define SSTEM_TC_DIAG 0                                    // kernel-tuning experiments: 1 = no blend, 2 = no output stores, 4 = no MMAs
-#endif
+#include "tma.cuh"
 
 namespace sstem {
 namespace {
@@ -102,9 +98,35 @@ __device__ __forceinline__ uint64_t tc_desc(unsigned addr, unsigned lbo, unsigne
     return (uint64_t)((addr >> 4) & 0x3fffu) | ((uint64_t)((lbo >> 4) & 0x3fffu) << 16) |
            ((uint64_t)((sbo >> 4) & 0x3fffu) << 32) | ((uint64_t)1 << 46);
 }
-__device__ __forceinline__ void tc_bulk_load(unsigned dst, const void* src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+// instruction descriptor of tcgen05.mma kind::tf32: D = f32, A = B = tf32, both K-major, M x N
+__host__ __device__ constexpr unsigned tc_idesc_tf32(int m, int n) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(n >> 3) << 17) | ((unsigned)(m >> 4) << 24);
+}
+// D[tmem] (+)= A * B, the accumulate flag as the instruction's predicate
+__device__ __forceinline__ void tc_mma(unsigned d_tmem, uint64_t da, uint64_t db, unsigned idesc, bool accumulate) {
+    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+                 ::"r"(d_tmem), "l"(da), "l"(db), "r"(idesc), "r"((unsigned)accumulate) : "memory");
+}
+// Warp 0 allocates NCOLS columns of tensor memory and writes their address to shared memory at `slot`; every thread
+// returns it after the block-wide barrier.
+template <unsigned NCOLS>
+__device__ __forceinline__ unsigned tmem_alloc(unsigned slot, int warp) {
+    if (warp == 0) {
+        __syncwarp();
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "n"(NCOLS));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    return *reinterpret_cast<volatile unsigned*>(__cvta_shared_to_generic(slot));
+}
+template <unsigned NCOLS>
+__device__ __forceinline__ void tmem_dealloc(unsigned tmem, int warp) {   // after every thread's last tensor-memory access
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(NCOLS));
 }
 __device__ __forceinline__ float to_tf32(float x) {        // round to nearest (the tensor core itself would truncate)
     unsigned u;
@@ -114,23 +136,23 @@ __device__ __forceinline__ float to_tf32(float x) {        // round to nearest (
 __device__ __forceinline__ void sts128(unsigned addr, float a, float b, float c, float d) {
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
-__device__ __forceinline__ float lds_f32(unsigned addr) {
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
-    return v;
-}
 
-// UPS: fold the x2 upsample into the producer.  WVEC with UPS: w % 4 == 0 and x is 16-byte aligned, so the source
-// window is fetched with 16-byte loads; otherwise element by element.  WVEC without UPS: x is tile-major,
-// [B][ceil(h/8)][ceil(w/8)][51][8][8] (cin == 51; the tap gradients of the tiled consumer, read by the input gradient of
-// sstem_tap_conv3x3_backward); entries outside the image are never read.  The one flag serves both so that the
-// existing instantiations keep their symbols and code.
-// TILED: the output is tile-major.  FULL: cin is 49..52, i.e. all 13 chunks exist -- the MMA and blend loops then have
-// no per-chunk checks.
-template <bool UPS, bool TILED, bool WVEC, bool FULL>
+// How the producers read x.
+enum class TapSrc {
+    NCHW,        // [B][cin][h][w], no upsample
+    TILE_MAJOR,  // [B][ceil(h/8)][ceil(w/8)][51][8][8], no upsample (cin == 51: the tap gradients of the tiled consumer, read
+                 // by the input gradient of sstem_tap_conv3x3_backward); entries outside the image are never read
+    UP,          // NCHW, x2 upsample folded into the producer, source window fetched element by element
+    UP_VEC,      // the same with 16-byte loads: w % 4 == 0 and x 16-byte aligned
+};
+
+// TILED_OUT: the output is tile-major.  FULL: cin is 49..52, i.e. all 13 chunks exist -- the MMA and blend loops then
+// have no per-chunk checks.
+template <TapSrc SRC, bool TILED_OUT, bool FULL>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacked,
                    const float* __restrict__ bias, float* __restrict__ out, const TapConvShape sh) {
+    constexpr bool UPS = SRC == TapSrc::UP || SRC == TapSrc::UP_VEC, VEC = SRC == TapSrc::UP_VEC;
     extern __shared__ __align__(128) unsigned char tc_smem_raw[];
     const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
     unsigned char* gen = tc_smem_raw + (base - (unsigned)__cvta_generic_to_shared(tc_smem_raw));
@@ -138,15 +160,14 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
     // barriers: 0 weights, 1-2 a_full, 3-4 a_empty, 5-6 acc_full, 7-8 acc_empty; the TMEM base address after them
     const unsigned bar = base + TC_OFF_BAR;
     const unsigned b_w = bar, b_afull = bar + 8, b_aempty = bar + 24, b_accfull = bar + 40, b_accempty = bar + 56;
-    volatile unsigned* tmem_slot = reinterpret_cast<volatile unsigned*>(gen + TC_OFF_BAR + 96);
 
     if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(b_w));
+        mbar_init(b_w, 1);
         for (int s = 0; s < 2; ++s) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(b_afull + 8 * s), "r"(TC_PROD_THREADS));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(b_aempty + 8 * s));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(b_accfull + 8 * s));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(b_accempty + 8 * s), "r"(TC_EPI_WARPS * 32));
+            mbar_init(b_afull + 8 * s, TC_PROD_THREADS);
+            mbar_init(b_aempty + 8 * s, 1);
+            mbar_init(b_accfull + 8 * s, 1);
+            mbar_init(b_accempty + 8 * s, TC_EPI_WARPS * 32);
         }
         mbar_fence_init();
     }
@@ -154,15 +175,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
     for (unsigned i = tid; i < 2 * TC_A_BYTES / 16; i += TC_THREADS) sts128(base + TC_OFF_A + i * 16, 0.f, 0.f, 0.f, 0.f);
         if (tid < TC_N) reinterpret_cast<float*>(gen + TC_OFF_BIAS)[tid] = (bias != nullptr && tid < sh.cout) ? bias[tid] : 0.f;
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    if (warp == 0) {
-        __syncwarp();
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(bar + 96), "n"(TC_TMEM_COLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const unsigned tmem = *tmem_slot;
+    const unsigned tmem = tmem_alloc<TC_TMEM_COLS>(bar + 96, warp);
 
     // A CTA walks tiles blockIdx.x, + gridDim.x, ...; the tile coordinates advance by a fixed (column, row) step, so
     // the loop needs no division (two 32-bit divisions per tile and warp were 15 % of all instructions issued).
@@ -219,8 +232,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             tc_arrive(b_accempty + 8 * as);                // the accumulator stage is free: the MMAs of tile it + 2 may start
             const int Y = Y0 + r, X = X0 + c;
-            if (SSTEM_TC_DIAG & 2) continue;
-            if (TILED) {
+            if (TILED_OUT) {
                 // the 16 x 8 tile is two 8 x 8 blocks of the tile-major layout; a warp writes 32 consecutive floats per tap
                 // (cout == 51 here).  Pad pixels of an existing block (ragged H / W) are written as zeros.
                 if ((Y >> 3) < tiles_y8) {
@@ -254,15 +266,14 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
         const unsigned tmem_u = __shfl_sync(0xffffffffu, tmem, 0);
         if (lane == 0) {
             // weights: resident for the life of the CTA
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(b_w), "r"(TC_W_BYTES) : "memory");
+            mbar_expect_tx(b_w, TC_W_BYTES);
             for (int t = 0; t < 9; ++t)
-                tc_bulk_load(base + t * TC_W_TAP_BYTES, reinterpret_cast<const char*>(wpacked) + (size_t)t * TC_W_TAP_BYTES, TC_W_TAP_BYTES, b_w);
-            tc_bulk_load(base + TC_W_ZERO_OFF, reinterpret_cast<const char*>(wpacked) + TC_W_ZERO_OFF, TC_N * 16, b_w);
+                bulk_load(base + t * TC_W_TAP_BYTES, reinterpret_cast<const char*>(wpacked) + (size_t)t * TC_W_TAP_BYTES, TC_W_TAP_BYTES, b_w);
+            bulk_load(base + TC_W_ZERO_OFF, reinterpret_cast<const char*>(wpacked) + TC_W_ZERO_OFF, TC_N * 16, b_w);
         }
         __syncwarp();
         tc_wait(b_w, 0);
-        // instruction descriptor: D = f32, A = B = tf32, both K-major, N = 64, M = 128
-        constexpr unsigned idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(TC_N >> 3) << 17) | ((unsigned)(128 >> 4) << 24);
+        constexpr unsigned idesc = tc_idesc_tf32(128, TC_N);
         // Descriptors differ only in their start-address field (units of 16 bytes, no carry out of the field: shared memory
         // addresses are < 2^18): per tap + (dy * 10 + dx) pixels for the patch, + 13 chunks for the weights; per K-step
         // + 2 chunks each.  The last K-step's second weight chunk is the zero chunk all taps share: its leading-byte
@@ -276,25 +287,18 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
             tc_wait(b_accempty + 8 * s, ph ^ 1);           // accumulator stage drained by the epilogue (passes at once the first time)
             tc_wait(b_afull + 8 * s, ph);                  // patch written and fenced by the producers
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint64_t da0 = (SSTEM_TC_DIAG & 32) ? tc_desc(base + TC_OFF_A, 3072, 256)       // timing experiment: 128-byte aligned core matrices
-                                                      : tc_desc(base + TC_OFF_A + s * TC_A_BYTES, TC_NPIX * 16, TC_PW * 16);
+            const uint64_t da0 = tc_desc(base + TC_OFF_A + s * TC_A_BYTES, TC_NPIX * 16, TC_PW * 16);
             const unsigned d_tmem = tmem_u + s * TC_N;
 #pragma unroll
             for (int tap = 0; tap < 9; ++tap) {
 #pragma unroll
                 for (int ks = 0; ks < TC_CHUNKS / 2; ++ks) {
-                    if ((SSTEM_TC_DIAG & 4) || ks >= k_steps) break;
-                    const uint64_t da = (SSTEM_TC_DIAG & 32) ? da0 + (uint64_t)((tap / 3) * 16 + ks * 2 * 192)
-                                      : (SSTEM_TC_DIAG & 16) ? da0 + (uint64_t)((tap / 3) * TC_PW + ks * 2 * TC_NPIX)
-                                                             : da0 + (uint64_t)((tap / 3) * TC_PW + (tap % 3) + ks * 2 * TC_NPIX);
+                    if (ks >= k_steps) break;
+                    const uint64_t da = da0 + (uint64_t)((tap / 3) * TC_PW + (tap % 3) + ks * 2 * TC_NPIX);
                     uint64_t db = db0 + (uint64_t)((tap * TC_W_TAP_BYTES + ks * 2 * TC_N * 16) >> 4);
                     if (2 * ks + 1 >= TC_WCHUNKS)
                         db += (uint64_t)(((TC_W_ZERO_OFF - tap * TC_W_TAP_BYTES - ks * 2 * TC_N * 16) >> 4) - TC_N) << 16;
-                    if (lane == 0)
-                        asm volatile(
-                            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                            "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-                            ::"r"(d_tmem), "l"(da), "l"(db), "r"(idesc), "r"((unsigned)((tap | ks) != 0)) : "memory");
+                    if (lane == 0) tc_mma(d_tmem, da, db, idesc, (tap | ks) != 0);
                 }
             }
             __syncwarp();
@@ -323,14 +327,14 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
         // box per channel group was tried first: its 48-byte rows cost ~2 us per box and shared memory has no room for a
         // second window, so half of that latency stayed exposed (0.85 ms vs the register prefetch, see DESIGN 4.11).
         constexpr int ROW4 = TC_WIN_W / 4;                 // 16-byte pieces per window row: 3
-        constexpr int NFILL = WVEC ? (TC_MAXC * TC_WIN_H * ROW4 + TC_PROD_THREADS - 1) / TC_PROD_THREADS      // 5 x float4
+        constexpr int NFILL = VEC ? (TC_MAXC * TC_WIN_H * ROW4 + TC_PROD_THREADS - 1) / TC_PROD_THREADS      // 5 x float4
                                    : (TC_MAXC * TC_WIN_CH + TC_PROD_THREADS - 1) / TC_PROD_THREADS;          // 18 x float
-        float4 pre4[WVEC ? NFILL : 1];
-        float pre[WVEC ? 1 : NFILL];
-        // WVEC: which 16-byte piece this thread fetches in round k does not depend on the tile: its channel offset (elements;
+        float4 pre4[VEC ? NFILL : 1];
+        float pre[VEC ? 1 : NFILL];
+        // VEC: which 16-byte piece this thread fetches in round k does not depend on the tile: its channel offset (elements;
         // the host checks cin * h * w < 2^31), window row and column piece are computed once
-        int f_choff[WVEC ? NFILL : 1], f_wy[WVEC ? NFILL : 1], f_c4[WVEC ? NFILL : 1], f_dst[WVEC ? NFILL : 1];
-        if (UPS && WVEC) {
+        int f_choff[VEC ? NFILL : 1], f_wy[VEC ? NFILL : 1], f_c4[VEC ? NFILL : 1], f_dst[VEC ? NFILL : 1];
+        if (VEC) {
 #pragma unroll
             for (int k = 0; k < NFILL; ++k) {
                 const int i = ptid + k * TC_PROD_THREADS;
@@ -349,7 +353,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
 #pragma unroll
             for (int k = 0; k < NFILL; ++k) {
                 const int i = ptid + k * TC_PROD_THREADS;
-                if (WVEC) {
+                if (VEC) {
                     const int gy = min(sy0 + f_wy[k], sh.h - 1), gx = sx0 + f_c4[k];   // columns past the edge are never blended in
                     pre4[k] = (f_choff[k] >= 0 && gx < sh.w) ? __ldg(reinterpret_cast<const float4*>(xb + (f_choff[k] + gy * sh.w + gx)))
                                                              : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -365,7 +369,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
 #pragma unroll
             for (int k = 0; k < NFILL; ++k) {
                 const int i = ptid + k * TC_PROD_THREADS;
-                if (WVEC) {
+                if (VEC) {
                     if (f_dst[k] >= 0) sts128(win + f_dst[k], pre4[k].x, pre4[k].y, pre4[k].z, pre4[k].w);
                 } else {
                     const int ch = i / TC_WIN_CH, p = i - ch * TC_WIN_CH;
@@ -408,7 +412,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
                 tc_wait(b_aempty + 8 * s, ph ^ 1);         // the MMAs that read this patch stage two tiles ago are complete
 #pragma unroll
                 for (int g = 0; g < TC_WIN_GROUPS; ++g) {
-                    if (has_pixel && !(SSTEM_TC_DIAG & 1)) {
+                    if (has_pixel) {
                         // this thread's chunks of the group: 7 g + half + 2 k.  With 13 chunks (cin 49..52, FULL) that is
                         // k < 3, plus k = 3 for the even chunks of group 0; otherwise each chunk is checked against cin.
 #pragma unroll
@@ -434,26 +438,12 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
             } else {
                 const float* xb = x + (int64_t)b * sh.cin * src_plane;
                 tc_wait(b_aempty + 8 * s, ph ^ 1);
-                if (WVEC && has_pixel) {                   // tile-major input: channel stride 64, cin == 51 (13 chunks)
+                if (has_pixel) {
+                    // the pixel's channels: tile-major (cin == 51, 13 chunks) at a stride of 64, NCHW at a stride of one plane
                     const int Yc = min(max(Y, 0), sh.H - 1), Xc = min(max(X, 0), sh.W - 1);
-                    const float* xp = x + ((((int64_t)b * ((sh.H + 7) >> 3) + (Yc >> 3)) * ((sh.W + 7) >> 3) + (Xc >> 3)) * (51 * 64) +
-                                           (Yc & 7) * 8 + (Xc & 7));
-#pragma unroll 1
-                    for (int ck0 = half; ck0 < nchunks; ck0 += 8) {
-                        const unsigned dst0 = a_dst - half_dst;
-                        float q[16];
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            const int ch = (ck0 + 2 * (j >> 2)) * 4 + (j & 3);
-                            q[j] = (inside && ch < sh.cin) ? __ldg(xp + ch * 64) : 0.f;
-                        }
-#pragma unroll
-                        for (int c4 = 0; c4 < 4; ++c4)
-                            if (ck0 + 2 * c4 < nchunks)
-                                sts128(dst0 + (ck0 + 2 * c4) * TC_NPIX * 16, to_tf32(q[4 * c4]), to_tf32(q[4 * c4 + 1]), to_tf32(q[4 * c4 + 2]), to_tf32(q[4 * c4 + 3]));
-                    }
-                } else if (has_pixel) {
-                    const float* xp = xb + (int64_t)min(max(Y, 0), sh.H - 1) * sh.W + min(max(X, 0), sh.W - 1);
+                    const float* xp = SRC == TapSrc::TILE_MAJOR
+                        ? x + ((((int64_t)b * ((sh.H + 7) >> 3) + (Yc >> 3)) * ((sh.W + 7) >> 3) + (Xc >> 3)) * (51 * 64) + (Yc & 7) * 8 + (Xc & 7))
+                        : xb + (int64_t)Yc * sh.W + Xc;
 #pragma unroll 1
                     for (int ck0 = half; ck0 < nchunks; ck0 += 8) {    // chunks half, half + 2, ...: 16 independent loads in flight per thread
                         const unsigned dst0 = a_dst - half_dst;
@@ -461,7 +451,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
 #pragma unroll
                         for (int j = 0; j < 16; ++j) {
                             const int ch = (ck0 + 2 * (j >> 2)) * 4 + (j & 3);
-                            q[j] = (inside && ch < sh.cin) ? __ldg(xp + (int64_t)ch * src_plane) : 0.f;
+                            q[j] = (inside && ch < sh.cin) ? __ldg(xp + (SRC == TapSrc::TILE_MAJOR ? ch * 64 : (int64_t)ch * src_plane)) : 0.f;
                         }
 #pragma unroll
                         for (int c4 = 0; c4 < 4; ++c4)
@@ -475,52 +465,70 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(TC_TMEM_COLS));
+    tmem_dealloc<TC_TMEM_COLS>(tmem, warp);
 }
 
-// weights [cout][cin][3][3] -> [tap][chunk < 13][n = 64][4] + one zero chunk, zero padded, rounded to TF32
+// weights [cout][cin][3][3] -> [tap][chunk < 13][n = 64][4] + one zero chunk, zero padded, rounded to TF32.  ADJOINT:
+// the image of W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx] instead, the convolution from cout to cin channels that the
+// input gradient runs.
+template <bool ADJOINT>
 __global__ void tap_conv3x3_pack_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (int)(TC_W_BYTES / 4)) return;
     if (i >= (int)(TC_W_ZERO_OFF / 4)) { packed[i] = 0.f; return; }
     const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % TC_WCHUNKS, tap = (i >> 2) / TC_N / TC_WCHUNKS;
-    const int ch = ck * 4 + j;
-    packed[i] = (n < cout && ch < cin) ? to_tf32(w[((int64_t)n * cin + ch) * 9 + tap]) : 0.f;
+    const int ch = ck * 4 + j;                             // input channel of the packed convolution
+    if (ADJOINT)                                           // W'[n][ch][tap] = W[ch][n][8 - tap]
+        packed[i] = (n < cin && ch < cout) ? to_tf32(w[((int64_t)ch * cin + n) * 9 + (8 - tap)]) : 0.f;
+    else
+        packed[i] = (n < cout && ch < cin) ? to_tf32(w[((int64_t)n * cin + ch) * 9 + tap]) : 0.f;
 }
 
-template <bool UPS, bool TILED, bool WVEC, bool FULL>
-int launch_tap_conv(const float* x, const float* wpacked, const float* bias, float* out, const TapConvShape& sh, cudaStream_t s) {
+// One persistent launch.  Templated on the kernel itself: every kernel needs its own PerDeviceOnce, or only the first
+// would get its shared-memory size.
+template <auto Kern, class... Args>
+int launch_tc(unsigned smem, int threads, int ctas, cudaStream_t s, const Args&... args) {
     static PerDeviceOnce done;
-    auto kern = tap_conv3x3_kernel<UPS, TILED, WVEC, FULL>;
     int dev = 0;
     cudaGetDevice(&dev);
     if (!done.test(dev)) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM) != cudaSuccess) return (int)cudaGetLastError();
+        if (cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return (int)cudaGetLastError();
         done.set(dev);
     }
-    const int ctas = std::min(sh.ntiles, sm_count());
-    kern<<<ctas, TC_THREADS, TC_SMEM, s>>>(x, wpacked, bias, out, sh);
+    Kern<<<ctas, threads, smem, s>>>(args...);
     count_launch();
     return finish_launch();
+}
+
+template <TapSrc SRC>
+int launch_tap_conv(bool tiled_out, bool full, const float* x, const float* wpacked, const float* bias, float* out,
+                    const TapConvShape& sh, cudaStream_t s) {
+    const int ctas = std::min(sh.ntiles, sm_count());
+    if (tiled_out)
+        return full ? launch_tc<tap_conv3x3_kernel<SRC, true, true>>(TC_SMEM, TC_THREADS, ctas, s, x, wpacked, bias, out, sh)
+                    : launch_tc<tap_conv3x3_kernel<SRC, true, false>>(TC_SMEM, TC_THREADS, ctas, s, x, wpacked, bias, out, sh);
+    return full ? launch_tc<tap_conv3x3_kernel<SRC, false, true>>(TC_SMEM, TC_THREADS, ctas, s, x, wpacked, bias, out, sh)
+                : launch_tc<tap_conv3x3_kernel<SRC, false, false>>(TC_SMEM, TC_THREADS, ctas, s, x, wpacked, bias, out, sh);
+}
+
+// tap_conv3x3_kernel for (source layout, output layout, all 13 chunks).  A tile-major source is only the input
+// gradient's: 51 channels (FULL), NCHW output.
+int launch_tap_conv(TapSrc src, bool tiled_out, bool full, const float* x, const float* wpacked, const float* bias, float* out,
+                    const TapConvShape& sh, cudaStream_t s) {
+    switch (src) {
+    case TapSrc::NCHW: return launch_tap_conv<TapSrc::NCHW>(tiled_out, full, x, wpacked, bias, out, sh, s);
+    case TapSrc::UP: return launch_tap_conv<TapSrc::UP>(tiled_out, full, x, wpacked, bias, out, sh, s);
+    case TapSrc::UP_VEC: return launch_tap_conv<TapSrc::UP_VEC>(tiled_out, full, x, wpacked, bias, out, sh, s);
+    default: return launch_tc<tap_conv3x3_kernel<TapSrc::TILE_MAJOR, false, true>>(TC_SMEM, TC_THREADS, std::min(sh.ntiles, sm_count()),
+                                                                                   s, x, wpacked, bias, out, sh);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Backward of y = conv3x3(up(x), W) + b (sstem_tap_conv3x3_backward).
 //
 // grad_x = up^T(conv3x3(gy, W')), W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]: the convolution is tap_conv3x3_kernel on its
-// no-upsample path (weights packed by tap_conv3x3_pack_adjoint_kernel), up^T is the gather below.
-
-// W [cout][cin][3][3] -> the packed image of W' (a convolution from cout to cin channels), rounded to TF32
-__global__ void tap_conv3x3_pack_adjoint_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (int)(TC_W_BYTES / 4)) return;
-    if (i >= (int)(TC_W_ZERO_OFF / 4)) { packed[i] = 0.f; return; }
-    const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % TC_WCHUNKS, tap = (i >> 2) / TC_N / TC_WCHUNKS;
-    const int co = ck * 4 + j;                             // input channel of the adjoint = output channel of the layer
-    packed[i] = (n < cin && co < cout) ? to_tf32(w[((int64_t)co * cin + n) * 9 + (8 - tap)]) : 0.f;
-}
+// no-upsample path (weights packed by tap_conv3x3_pack_kernel<true>), up^T is the gather below.
 
 // Weight with which output row (column) Y of the align_corners upsample reads source row i: ATen's float32 index and
 // fraction, as the forward producer computes them.  At the last row the neighbour is the row itself (both weights land
@@ -588,7 +596,8 @@ constexpr unsigned WG_TMEM_COLS = 512;
 static_assert(9 * WG_N <= (int)WG_TMEM_COLS, "nine accumulators in tensor memory");
 static_assert(WG_THREADS * WG_CO_PER_THREAD * 4 <= WG_OFF_BAR, "the bias reduction reuses the operand buffers");
 
-template <bool UPS, bool TILED>
+// GY_TILED: gy is tile-major (cout == 51)
+template <bool UPS, bool GY_TILED>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__ x, float* __restrict__ part_w,
                          float* __restrict__ part_b, const TapConvShape sh) {
@@ -597,22 +606,13 @@ tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__
     unsigned char* gen = tc_smem_raw + (base - (unsigned)__cvta_generic_to_shared(tc_smem_raw));
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const unsigned bar = base + WG_OFF_BAR;
-    volatile unsigned* tmem_slot = reinterpret_cast<volatile unsigned*>(gen + WG_OFF_BAR + 8);
     if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
+        mbar_init(bar, 1);
         mbar_fence_init();
     }
     // padding rows / columns of both operands stay zero
     for (unsigned i = tid; i < WG_OFF_BAR / 16; i += WG_THREADS) sts128(base + i * 16, 0.f, 0.f, 0.f, 0.f);
-    if (warp == 0) {
-        __syncwarp();
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(bar + 8), "n"(WG_TMEM_COLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const unsigned tmem = *tmem_slot;
+    const unsigned tmem = tmem_alloc<WG_TMEM_COLS>(bar + 8, warp);
 
     // A staging: thread = (tile pixel, output-channel class); B staging: thread = (patch pixel, input-channel half)
     const int apx = tid & 127, acg = tid >> 7, ay = apx >> 3, ax = apx & 7;
@@ -624,8 +624,7 @@ tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__
     float bacc[WG_CO_PER_THREAD];
 #pragma unroll
     for (int k = 0; k < WG_CO_PER_THREAD; ++k) bacc[k] = 0.f;
-    // D = f32, A = B = tf32, both K-major, N = 56, M = 64
-    constexpr unsigned idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(WG_N >> 3) << 17) | ((unsigned)(WG_M >> 4) << 24);
+    constexpr unsigned idesc = tc_idesc_tf32(WG_M, WG_N);
 
     int it = 0;
     for (int tile = blockIdx.x; tile < sh.ntiles; tile += gridDim.x, ++it) {
@@ -638,9 +637,9 @@ tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__
         {   // A: gy of the tile, and its per-channel sum
             const int Y = Y0 + ay, X = X0 + ax;
             const bool inside = Y < sh.H && X < sh.W;
-            const float* g = TILED ? gy + ((((int64_t)b * tiles_y8 + (Y >> 3)) * tiles_x8 + (X >> 3)) * (51 * 64) + (Y & 7) * 8 + (X & 7))
+            const float* g = GY_TILED ? gy + ((((int64_t)b * tiles_y8 + (Y >> 3)) * tiles_x8 + (X >> 3)) * (51 * 64) + (Y & 7) * 8 + (X & 7))
                                    : gy + (int64_t)b * sh.cout * plane + (int64_t)Y * sh.W + X;
-            const int64_t cstride = TILED ? 64 : plane;
+            const int64_t cstride = GY_TILED ? 64 : plane;
 #pragma unroll
             for (int k = 0; k < WG_CO_PER_THREAD; ++k) {
                 const int co = acg + 3 * k;
@@ -700,11 +699,7 @@ tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__
                 for (int ky = 0; ky < TC_TH; ++ky) {
                     const uint64_t da = da0 + (uint64_t)((ky * WG_A_ROW) >> 4);
                     const uint64_t db = db0 + (uint64_t)((dx * WG_B_COPY + (ky + dy) * WG_B_ROW) >> 4);
-                    if (lane == 0)
-                        asm volatile(
-                            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                            "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-                            ::"r"(d_tmem), "l"(da), "l"(db), "r"(idesc), "r"((unsigned)((it | ky) != 0)) : "memory");
+                    if (lane == 0) tc_mma(d_tmem, da, db, idesc, (it | ky) != 0);
                 }
             }
             __syncwarp();
@@ -753,9 +748,7 @@ tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__
         for (int p = 0; p < 128; ++p) sum += red[(cg * 128 + p) * WG_CO_PER_THREAD + k];
         part_b[(int64_t)blockIdx.x * sh.cout + tid] = sum;
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(WG_TMEM_COLS));
+    tmem_dealloc<WG_TMEM_COLS>(tmem, warp);
 }
 
 // sum of the per-CTA partials in CTA order (deterministic); out[i] for i < n, NULL outputs skipped
@@ -774,17 +767,30 @@ __global__ void tap_conv3x3_wgrad_reduce_kernel(const float* __restrict__ part_w
     *dst = s;
 }
 
-template <bool UPS, bool TILED>
-int launch_wgrad(const float* gy, const float* x, float* part_w, float* part_b, const TapConvShape& sh, int ctas, cudaStream_t s) {
-    static PerDeviceOnce done;
-    auto kern = tap_conv3x3_wgrad_kernel<UPS, TILED>;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!done.test(dev)) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WG_SMEM) != cudaSuccess) return (int)cudaGetLastError();
-        done.set(dev);
-    }
-    kern<<<ctas, WG_THREADS, WG_SMEM, s>>>(gy, x, part_w, part_b, sh);
+// (h, w): the source; the output is (2h, 2w) with the upsample.  The callers have checked that the tile count fits.
+TapConvShape tap_conv_shape(int64_t B, int cin, int cout, int64_t h, int64_t w, bool ups) {
+    TapConvShape sh;
+    sh.B = (int)B; sh.cin = cin; sh.cout = cout; sh.h = (int)h; sh.w = (int)w;
+    sh.H = ups ? 2 * (int)h : (int)h;
+    sh.W = ups ? 2 * (int)w : (int)w;
+    sh.tiles_x = (sh.W + TC_TW - 1) / TC_TW;
+    sh.tiles_y = (sh.H + TC_TH - 1) / TC_TH;
+    sh.ntiles = (int)((int64_t)sh.tiles_x * sh.tiles_y * B);
+    sh.k_steps = (cin + 7) / 8;
+    sh.ry = sh.H > 1 ? (float)(sh.h - 1) / (float)(sh.H - 1) : 0.f;
+    sh.rx = sh.W > 1 ? (float)(sh.w - 1) / (float)(sh.W - 1) : 0.f;
+    return sh;
+}
+
+template <bool ADJOINT>
+int pack_weights(const float* weight, float* packed, int cin, int cout, int max_cout, cudaStream_t s) {
+    if (!weight || !packed) return SSTEM_E_NULL;
+    if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > max_cout) return SSTEM_E_SHAPE;
+    if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
+    DeviceGuard guard(packed);
+    if (guard.err) return guard.err;
+    const int total = (int)(TC_W_BYTES / 4);
+    tap_conv3x3_pack_kernel<ADJOINT><<<(total + 255) / 256, 256, 0, s>>>(weight, packed, cin, cout);
     count_launch();
     return finish_launch();
 }
@@ -798,15 +804,7 @@ using namespace sstem;
 extern "C" int64_t sstem_tap_conv3x3_packed_elems(void) { return (int64_t)TC_W_BYTES / 4; }
 
 extern "C" int sstem_tap_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
-    if (!weight || !packed) return SSTEM_E_NULL;
-    if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
-    if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
-    DeviceGuard guard(packed);
-    if (guard.err) return guard.err;
-    const int total = (int)(TC_W_BYTES / 4);
-    tap_conv3x3_pack_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(weight, packed, cin, cout);
-    count_launch();
-    return finish_launch();
+    return pack_weights<false>(weight, packed, cin, cout, TC_N, (cudaStream_t)stream);
 }
 
 extern "C" int sstem_tap_conv3x3(const float* x, const float* packed_weight, const float* bias, float* out,
@@ -820,43 +818,15 @@ extern "C" int sstem_tap_conv3x3(const float* x, const float* packed_weight, con
     if (!aligned4(x) || !aligned16(packed_weight) || !aligned4(out) || (bias && !aligned4(bias))) return SSTEM_E_ALIGN;
     DeviceGuard guard(out);
     if (guard.err) return guard.err;
-    TapConvShape sh;
-    sh.B = (int)B; sh.cin = cin; sh.cout = cout; sh.h = (int)h; sh.w = (int)w;
-    sh.H = ups ? 2 * (int)h : (int)h;
-    sh.W = ups ? 2 * (int)w : (int)w;
-    sh.tiles_x = (sh.W + TC_TW - 1) / TC_TW;
-    sh.tiles_y = (sh.H + TC_TH - 1) / TC_TH;
-    const int64_t nt = (int64_t)sh.tiles_x * sh.tiles_y * B;
-    if (nt > INT32_MAX / 2 || (int64_t)cin * h * w > INT32_MAX) return SSTEM_E_SHAPE;
-    sh.ntiles = (int)nt;
-    sh.k_steps = (cin + 7) / 8;
-    sh.ry = sh.H > 1 ? (float)(sh.h - 1) / (float)(sh.H - 1) : 0.f;
-    sh.rx = sh.W > 1 ? (float)(sh.w - 1) / (float)(sh.W - 1) : 0.f;
-    cudaStream_t s = (cudaStream_t)stream;
+    const TapConvShape sh = tap_conv_shape(B, cin, cout, h, w, ups);
+    if ((int64_t)sh.tiles_x * sh.tiles_y * B > INT32_MAX / 2 || (int64_t)cin * h * w > INT32_MAX) return SSTEM_E_SHAPE;
+    const TapSrc src = !ups ? TapSrc::NCHW : (w % 4 == 0 && aligned16(x)) ? TapSrc::UP_VEC : TapSrc::UP;
     const bool full = cin > 48;                            // all 13 channel chunks exist: the common (51-channel) case, no per-chunk checks
-#define SSTEM_TC_LAUNCH(UPS_, WVEC_)                                                                                       \
-    return full ? (tiled ? launch_tap_conv<UPS_, true, WVEC_, true>(x, packed_weight, bias, out, sh, s)                    \
-                         : launch_tap_conv<UPS_, false, WVEC_, true>(x, packed_weight, bias, out, sh, s))                  \
-                : (tiled ? launch_tap_conv<UPS_, true, WVEC_, false>(x, packed_weight, bias, out, sh, s)                   \
-                         : launch_tap_conv<UPS_, false, WVEC_, false>(x, packed_weight, bias, out, sh, s))
-    if (ups) {
-        if ((w % 4 == 0) && aligned16(x)) { SSTEM_TC_LAUNCH(true, true); }
-        SSTEM_TC_LAUNCH(true, false);
-    }
-    SSTEM_TC_LAUNCH(false, false);
-#undef SSTEM_TC_LAUNCH
+    return launch_tap_conv(src, tiled, full, x, packed_weight, bias, out, sh, (cudaStream_t)stream);
 }
 
 extern "C" int sstem_tap_conv3x3_pack_weights_adjoint(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
-    if (!weight || !packed) return SSTEM_E_NULL;
-    if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > TC_MAXC) return SSTEM_E_SHAPE;
-    if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
-    DeviceGuard guard(packed);
-    if (guard.err) return guard.err;
-    const int total = (int)(TC_W_BYTES / 4);
-    tap_conv3x3_pack_adjoint_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(weight, packed, cin, cout);
-    count_launch();
-    return finish_launch();
+    return pack_weights<true>(weight, packed, cin, cout, TC_MAXC, (cudaStream_t)stream);
 }
 
 extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x, const float* packed_adjoint,
@@ -878,25 +848,14 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
     DeviceGuard guard(grad_out);
     if (guard.err) return guard.err;
     cudaStream_t s = (cudaStream_t)stream;
-    TapConvShape sh;
-    sh.B = (int)B; sh.H = (int)H; sh.W = (int)W;
-    sh.tiles_x = (int)((W + TC_TW - 1) / TC_TW);
-    sh.tiles_y = (int)((H + TC_TH - 1) / TC_TH);
-    sh.ntiles = (int)nt;
-    sh.ry = ups && H > 1 ? (float)(h - 1) / (float)(H - 1) : 0.f;
-    sh.rx = ups && W > 1 ? (float)(w - 1) / (float)(W - 1) : 0.f;
+    const TapConvShape sh = tap_conv_shape(B, cin, cout, h, w, ups);
 
     if (grad_x) {
         // gU = conv3x3(gy, W'), cout -> cin channels at full resolution; with the upsample into a workspace, then up^T
-        TapConvShape sd = sh;
-        sd.cin = cout; sd.cout = cin; sd.h = (int)H; sd.w = (int)W;
-        sd.k_steps = (cout + 7) / 8;
+        const TapConvShape sd = tap_conv_shape(B, cout, cin, H, W, false);
         float* gU = grad_x;
         if (ups && workspace_alloc(reinterpret_cast<void**>(&gU), (size_t)(B * cin * H * W) * sizeof(float), s)) return cudaErrorMemoryAllocation;
-        int e;
-        if (tiled) e = launch_tap_conv<false, false, true, true>(grad_out, packed_adjoint, nullptr, gU, sd, s);
-        else if (cout > 48) e = launch_tap_conv<false, false, false, true>(grad_out, packed_adjoint, nullptr, gU, sd, s);
-        else e = launch_tap_conv<false, false, false, false>(grad_out, packed_adjoint, nullptr, gU, sd, s);
+        int e = launch_tap_conv(tiled ? TapSrc::TILE_MAJOR : TapSrc::NCHW, false, cout > 48, grad_out, packed_adjoint, nullptr, gU, sd, s);
         if (!e && ups) {
             const int64_t n = B * cin * h * w;
             upsample2x_adjoint_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(gU, grad_x, n, (int)h, (int)w, (int)H, (int)W, sh.ry, sh.rx);
@@ -907,17 +866,15 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
         if (e) return e;
     }
     if (grad_weight || grad_bias) {
-        sh.cin = cin; sh.cout = cout; sh.h = (int)h; sh.w = (int)w;
-        sh.k_steps = 0;
         const int ctas = std::min(sh.ntiles, sm_count());
         const int nw = cout * cin * 9;
         float* part = nullptr;
         if (workspace_alloc(reinterpret_cast<void**>(&part), (size_t)ctas * (nw + cout) * sizeof(float), s)) return cudaErrorMemoryAllocation;
         float* part_b = part + (size_t)ctas * nw;
-        int e = ups ? (tiled ? launch_wgrad<true, true>(grad_out, x, part, part_b, sh, ctas, s)
-                             : launch_wgrad<true, false>(grad_out, x, part, part_b, sh, ctas, s))
-                    : (tiled ? launch_wgrad<false, true>(grad_out, x, part, part_b, sh, ctas, s)
-                             : launch_wgrad<false, false>(grad_out, x, part, part_b, sh, ctas, s));
+        int e = ups ? (tiled ? launch_tc<tap_conv3x3_wgrad_kernel<true, true>>(WG_SMEM, WG_THREADS, ctas, s, grad_out, x, part, part_b, sh)
+                             : launch_tc<tap_conv3x3_wgrad_kernel<true, false>>(WG_SMEM, WG_THREADS, ctas, s, grad_out, x, part, part_b, sh))
+                    : (tiled ? launch_tc<tap_conv3x3_wgrad_kernel<false, true>>(WG_SMEM, WG_THREADS, ctas, s, grad_out, x, part, part_b, sh)
+                             : launch_tc<tap_conv3x3_wgrad_kernel<false, false>>(WG_SMEM, WG_THREADS, ctas, s, grad_out, x, part, part_b, sh));
         if (!e) {
             tap_conv3x3_wgrad_reduce_kernel<<<(nw + cout + 255) / 256, 256, 0, s>>>(part, part_b, grad_weight, grad_bias, nw, cout, ctas);
             count_launch();

@@ -1,5 +1,5 @@
-// TMA (cp.async.bulk.tensor) + mbarrier helpers shared by the warp and sepconv kernels, and the host-side
-// tensor-map encoder (driver entry point resolved through the runtime: no link-time dependency on libcuda).
+// TMA (cp.async.bulk.tensor), bulk-copy, mbarrier and shared-memory load helpers shared by the warp, sepconv and
+// tap-producer kernels, and the host-side tensor-map encoder (driver entry point resolved through the runtime: no link-time dependency on libcuda).
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -7,22 +7,35 @@
 
 namespace sstem {
 
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(count));
+// Shared-space (unsigned) addresses are the primary form; the pointer forms convert and forward.
+__device__ __forceinline__ void mbar_init(unsigned bar, int count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
 }
 __device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(bytes) : "memory");
+__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
-    const unsigned a = (unsigned)__cvta_generic_to_shared(bar);
+__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {   // unbounded: spins until the phase completes
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "WAIT_LOOP:\n\t"
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
         "@p bra DONE;\n\t"
         "bra WAIT_LOOP;\n\t"
-        "DONE:\n\t}" ::"r"(a), "r"(parity) : "memory");
+        "DONE:\n\t}" ::"r"(bar), "r"(parity) : "memory");
+}
+__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) { mbar_init((unsigned)__cvta_generic_to_shared(bar), count); }
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, unsigned bytes) { mbar_expect_tx((unsigned)__cvta_generic_to_shared(bar), bytes); }
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) { mbar_wait((unsigned)__cvta_generic_to_shared(bar), parity); }
+// 1-D bulk copy global -> shared (16-byte aligned, size a multiple of 16), completion on an mbarrier
+__device__ __forceinline__ void bulk_load(unsigned dst, const void* src, unsigned bytes, unsigned bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+__device__ __forceinline__ float lds_f32(unsigned addr) {
+    float v;
+    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
+    return v;
 }
 __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
     asm volatile(

@@ -17,41 +17,36 @@ def _stream_ptr(t: torch.Tensor) -> int:
     return torch.cuda.current_stream(t.device).cuda_stream
 
 
-def pack_tap_conv_weight(weight: torch.Tensor) -> torch.Tensor:
-    """``Conv2d.weight`` ``[cout<=64, cin<=52, 3, 3]`` -> the kernel's resident image (118 KB, TF32-rounded).  Pack once per
-    layer, reuse for every call."""
+def _pack(weight: torch.Tensor, adjoint: bool) -> torch.Tensor:
+    name, entry, max_cout = (("pack_tap_conv_weight_adjoint", "sstem_tap_conv3x3_pack_weights_adjoint", 52) if adjoint
+                             else ("pack_tap_conv_weight", "sstem_tap_conv3x3_pack_weights", 64))
     if weight.is_cuda == False:
         raise NotImplementedError()
     if weight.dtype != torch.float32 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3):
-        raise TypeError("pack_tap_conv_weight: float32 [cout, cin, 3, 3] required")
+        raise TypeError(f"{name}: float32 [cout, cin, 3, 3] required")
     cout, cin = weight.shape[:2]
-    if cin > 52 or cout > 64:
-        raise ValueError("pack_tap_conv_weight: cin <= 52 and cout <= 64 required")
+    if cin > 52 or cout > max_cout:
+        raise ValueError(f"{name}: cin <= 52 and cout <= {max_cout} required")
     lib = _lib.load()
     packed = torch.empty(lib.sstem_tap_conv3x3_packed_elems(), dtype=torch.float32, device=weight.device)
-    code = lib.sstem_tap_conv3x3_pack_weights(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
+    code = getattr(lib, entry)(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
     if code:
-        _lib.check(code, "sstem_tap_conv3x3_pack_weights")
-    packed._sstem_cin_cout = (int(cin), int(cout))
+        _lib.check(code, entry)
+    return packed
+
+
+def pack_tap_conv_weight(weight: torch.Tensor) -> torch.Tensor:
+    """``Conv2d.weight`` ``[cout<=64, cin<=52, 3, 3]`` -> the kernel's resident image (118 KB, TF32-rounded).  Pack once per
+    layer, reuse for every call."""
+    packed = _pack(weight, adjoint=False)
+    packed._sstem_cin_cout = (int(weight.shape[1]), int(weight.shape[0]))
     return packed
 
 
 def pack_tap_conv_weight_adjoint(weight: torch.Tensor) -> torch.Tensor:
     """``Conv2d.weight`` ``[cout<=52, cin<=52, 3, 3]`` -> the resident image of the adjoint convolution's weight
     ``W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]`` (cout -> cin channels), which the input gradient runs."""
-    if weight.is_cuda == False:
-        raise NotImplementedError()
-    if weight.dtype != torch.float32 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3):
-        raise TypeError("pack_tap_conv_weight_adjoint: float32 [cout, cin, 3, 3] required")
-    cout, cin = weight.shape[:2]
-    if cin > 52 or cout > 52:
-        raise ValueError("pack_tap_conv_weight_adjoint: cin <= 52 and cout <= 52 required")
-    lib = _lib.load()
-    packed = torch.empty(lib.sstem_tap_conv3x3_packed_elems(), dtype=torch.float32, device=weight.device)
-    code = lib.sstem_tap_conv3x3_pack_weights_adjoint(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
-    if code:
-        _lib.check(code, "sstem_tap_conv3x3_pack_weights_adjoint")
-    return packed
+    return _pack(weight, adjoint=True)
 
 
 def tap_conv3x3(x: torch.Tensor, packed_weight: torch.Tensor, bias=None, cin=None, cout=None, upsample=True, tiled=False) -> torch.Tensor:
@@ -146,20 +141,22 @@ class ModuleTapProducer(torch.nn.Module):
         self.bias = torch.nn.Parameter(torch.zeros(out_channels))
         torch.nn.init.kaiming_uniform_(self.weight, a=5 ** 0.5)
         self.upsample, self.tiled, self.trainable = upsample, tiled, trainable
-        self._packed, self._packed_version = None, None
-        self._packed_adjoint, self._packed_adjoint_version = None, None
+        self._packed = self._packed_adjoint = None
+        self._versions = {}
+
+    def _cached(self, name, pack, device):
+        """``self.<name>``, packed again from the weight whenever the weight or the device changed."""
+        key = (self.weight._version, self.weight.data_ptr())
+        packed = getattr(self, name)
+        if packed is None or self._versions.get(name) != key or packed.device != device:
+            setattr(self, name, pack(self.weight.detach()))
+            self._versions[name] = key
+        return getattr(self, name)
 
     def forward(self, x):
-        key = (self.weight._version, self.weight.data_ptr())
-        if self._packed is None or self._packed_version != key or self._packed.device != x.device:
-            self._packed = pack_tap_conv_weight(self.weight.detach())
-            self._packed_version = key
+        packed = self._cached("_packed", pack_tap_conv_weight, x.device)
         if not self.trainable:
-            return tap_conv3x3(x, self._packed, self.bias.detach(), upsample=self.upsample, tiled=self.tiled)
-        adjoint = None
-        if torch.is_grad_enabled() and x.requires_grad:
-            if self._packed_adjoint is None or self._packed_adjoint_version != key or self._packed_adjoint.device != x.device:
-                self._packed_adjoint = pack_tap_conv_weight_adjoint(self.weight.detach())
-                self._packed_adjoint_version = key
-            adjoint = self._packed_adjoint
-        return TapConv3x3Function.apply(x, self.weight, self.bias, self.upsample, self.tiled, self._packed, adjoint)
+            return tap_conv3x3(x, packed, self.bias.detach(), upsample=self.upsample, tiled=self.tiled)
+        need_adjoint = torch.is_grad_enabled() and x.requires_grad
+        adjoint = self._cached("_packed_adjoint", pack_tap_conv_weight_adjoint, x.device) if need_adjoint else None
+        return TapConv3x3Function.apply(x, self.weight, self.bias, self.upsample, self.tiled, packed, adjoint)
