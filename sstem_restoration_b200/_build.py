@@ -62,7 +62,7 @@ def build(force: bool = False, verbose: bool = False, lib_path: str = LIB_PATH, 
     """Compile every CUDA source (in parallel) and link one shared library; returns its path.
 
     `extra` / $SSTEM_NVCC_EXTRA: additional nvcc flags for kernel-tuning experiments
-    (e.g. -DSSTEM_BWD_NPRE=5), normally together with another `lib_path`."""
+    (e.g. -DSSTEM_BWD3_MINB=1), normally together with another `lib_path`."""
     if not force and not needs_build(lib_path):
         return lib_path
     from concurrent.futures import ThreadPoolExecutor

@@ -33,6 +33,8 @@
 //     shuffles: once per tile (forward) or once per step for gv (backward).
 #pragma once
 #include "common.cuh"
+#include <type_traits>
+#include <utility>
 
 namespace sstem {
 
@@ -41,32 +43,14 @@ namespace {
 constexpr int K51 = 51;
 constexpr int VDEPTH = 8;                  // steps of vertical taps in flight per warp
 
-#ifndef SSTEM_FWD_G
-#define SSTEM_FWD_G 4
-#endif
-#ifndef SSTEM_FWD_R
-#define SSTEM_FWD_R 8
-#endif
-#ifndef SSTEM_BWD_G
-#define SSTEM_BWD_G 4
-#endif
-#ifndef SSTEM_BWD_R
-#define SSTEM_BWD_R 4
-#endif
-#ifndef SSTEM_FWD_NPRE
-#define SSTEM_FWD_NPRE 13                  // taps of the next row (channel 0) preloaded during the current step;
+constexpr int FWD_G = 4, FWD_R = 8;        // forward, grad_input and the fused tail forward
+constexpr int BWD_G = 4, BWD_R = 4;        // tap gradients
+constexpr int FWD_NPRE = 13;               // taps of the next row (channel 0) preloaded during the current step;
                                            // 3-channel kernel (measured: +2 % there; 13 at C = 1 costs 5 %)
-#endif
-#ifndef SSTEM_FWD_NPRE1
-#define SSTEM_FWD_NPRE1 4                  // the same for the one- / two-channel kernels and the fused tail (measured:
+constexpr int FWD_NPRE1 = 4;               // the same for the one- / two-channel kernels and the fused tail (measured:
                                            // gray x3 forward +5 %, tail +0.4 %; 8 is no better)
-#endif
-#ifndef SSTEM_UNROLL2
-#define SSTEM_UNROLL2 1                    // one-channel kernels: steady loop two steps per iteration, v registers ping-pong
-#endif
-#ifndef SSTEM_BWD_NPRE
-#define SSTEM_BWD_NPRE 7                   // taps of the next row preloaded during the current step
-#endif
+constexpr int BWD_NPRE = 7;                // taps of the next row preloaded during the current step
+constexpr int MIN_CTAS = 2;                // CTAs per SM in every __launch_bounds__ (3 spills in the step loop: DESIGN 7)
 
 // ---- geometry of one configuration --------------------------------------------------------
 template <int G, int R>
@@ -257,6 +241,12 @@ struct VRing {
             dst[pp] = make_float2(slot[(2 * pp) * Gm::COLS], slot[(2 * pp + 1) * Gm::COLS]);
         slot_r = (slot_r + 1 == VDEPTH) ? 0 : slot_r + 1;
     }
+    __device__ __forceinline__ void advance(float2 (&dst)[R / 2]) {   // make the next step readable, refill the ring
+        cp_async_wait<VDEPTH - 3>();
+        __syncwarp();
+        issue();
+        read(dst);
+    }
 };
 
 // Transpose-reduce over the G tap-group lanes of a pixel: on return lane g holds, in
@@ -305,6 +295,40 @@ __device__ __forceinline__ void load_h(float2 (&h2)[R / 2][Geo<G, R>::NT], const
     }
 }
 
+template <int S0, class Step, int... I>
+__device__ __forceinline__ void edge_steps(Step& step, std::integer_sequence<int, I...>) {
+    (step(std::integral_constant<int, S0 + I>{}, S0 + I), ...);
+}
+
+// The R + 50 steps of a window.  The edge steps 0 .. R-2 and 51 .. R+49, where some rows have fy = s - p outside
+// [0, 50], are compile-time steps; the steady steps R-1 .. 50 between them run in a loop.  step(S, s, vuse, vfill)
+// runs step s from the vertical taps in vuse and fills vfill with the next step's; S is an integral_constant, the step
+// at an edge and -1 in the steady loop.  TWO_STEP: two steady steps per iteration, vcur and vnext swapping roles (no
+// register copies).  The one-channel kernels use it (measured +8 % on the gray forward, +2-6 % on the tail kernels);
+// the others keep one step per iteration (two-step at three channels: 0 % forward, -3 % on the tap gradients).
+template <int R, bool TWO_STEP, class Step>
+__device__ __forceinline__ void walk_steps(Step&& step, float2 (&vcur)[R / 2], float2 (&vnext)[R / 2]) {
+    auto one_step = [&](auto S, int s) {
+        step(S, s, vcur, vnext);
+#pragma unroll
+        for (int pp = 0; pp < R / 2; ++pp) vcur[pp] = vnext[pp];
+    };
+    edge_steps<0>(one_step, std::make_integer_sequence<int, R - 1>{});
+    constexpr std::integral_constant<int, -1> STEADY{};
+    if constexpr (TWO_STEP) {
+        static_assert((K51 - R + 1) % 2 == 0, "the two-step steady loop needs an even number of steady steps");
+#pragma unroll 1
+        for (int s = R - 1; s < K51; s += 2) {
+            step(STEADY, s, vcur, vnext);
+            step(STEADY, s + 1, vnext, vcur);
+        }
+    } else {
+#pragma unroll 1
+        for (int s = R - 1; s < K51; ++s) one_step(STEADY, s);
+    }
+    edge_steps<K51>(one_step, std::make_integer_sequence<int, R - 1>{});
+}
+
 // =====================================================================================
 // Forward
 // =====================================================================================
@@ -314,9 +338,9 @@ __device__ __forceinline__ void load_h(float2 (&h2)[R / 2][Geo<G, R>::NT], const
 template <int CC, int G, int R, int S>
 __device__ __forceinline__ void fwd_step(const float* __restrict__ prow0, bool novalid,
                                          const float2 (&h2)[R / 2][Geo<G, R>::NT], const float2 (&v2)[R / 2],
-                                         float2 (&acc)[CC][R / 2], float (&pre)[SSTEM_FWD_NPRE + 1]) {
+                                         float2 (&acc)[CC][R / 2], float (&pre)[FWD_NPRE + 1]) {
     using Gm = Geo<G, R>;
-    constexpr int NPRE = (CC >= 3) ? SSTEM_FWD_NPRE : SSTEM_FWD_NPRE1;   // channel 0's first taps were loaded during the previous step
+    constexpr int NPRE = (CC >= 3) ? FWD_NPRE : FWD_NPRE1;   // channel 0's first taps were loaded during the previous step
 #pragma unroll
     for (int c = 0; c < CC; ++c) {
         const float* prow = prow0 + c * Gm::ROWS * Gm::PITCH;
@@ -350,7 +374,7 @@ __device__ __forceinline__ void fwd_step(const float* __restrict__ prow0, bool n
 
 // VEC: W % 4 == 0 and v 16-byte aligned -> the ring is fed with 16-byte cp.async.
 template <int CC, int G, int R, bool VEC, bool PAIR>
-__global__ void __launch_bounds__(128, 2)
+__global__ void __launch_bounds__(128, MIN_CTAS)
 sepconv_fwd_k51_kernel(const float* __restrict__ in, const float* __restrict__ v,
                        const float* __restrict__ h, float* __restrict__ out,
                        int C, int c0, int H, int W, int replicas, const int* gate, int gate_want) {
@@ -392,52 +416,14 @@ sepconv_fwd_k51_kernel(const float* __restrict__ in, const float* __restrict__ v
     float2 vcur[Gm::NP], vnext[Gm::NP];
     vr.read(vcur);
     const float* prow = tile + xl + g;                  // P column of tap slot t is xl + g + G*t
-    auto advance = [&](float2 (&vdst)[Gm::NP]) {        // make the next step readable, refill the ring
-        cp_async_wait<VDEPTH - 3>();
-        __syncwarp();
-        vr.issue();
-        vr.read(vdst);
-    };
-    float pre[SSTEM_FWD_NPRE + 1];
+    float pre[FWD_NPRE + 1];
 #pragma unroll
-    for (int t = 0; t < ((CC >= 3) ? SSTEM_FWD_NPRE : SSTEM_FWD_NPRE1); ++t) pre[t] = prow[G * t];
-#define SSTEM_FWD_EDGE_STEP(S)                                                     \
-    if ((S) < R - 1 || ((S) >= K51 && (S) < Gm::ROWS)) {                           \
-        advance(vnext);                                                            \
-        fwd_step<CC, G, R, S>(prow, novalid, h2, vcur, acc, pre);                       \
-        _Pragma("unroll") for (int pp = 0; pp < Gm::NP; ++pp) vcur[pp] = vnext[pp]; \
-        prow += Gm::PITCH;                                                         \
-    }
-    SSTEM_FWD_EDGE_STEP(0) SSTEM_FWD_EDGE_STEP(1) SSTEM_FWD_EDGE_STEP(2) SSTEM_FWD_EDGE_STEP(3)
-    SSTEM_FWD_EDGE_STEP(4) SSTEM_FWD_EDGE_STEP(5) SSTEM_FWD_EDGE_STEP(6)
-    // One channel: two steps per iteration with vcur / vnext swapping roles (no register copies; measured +8 % on the
-    // gray forward, +2-6 % on the tail kernels).  Three channels keep the one-step loop (two-step: 0 % forward, -3 %
-    // on the tap gradients).
-    static_assert((K51 - R + 1) % 2 == 0, "the two-step steady loop needs an even number of steady steps");
-    if constexpr (SSTEM_UNROLL2 && CC == 1) {
-#pragma unroll 1
-        for (int s = R - 1; s < K51; s += 2) {          // steady state: all rows active
-            advance(vnext);
-            fwd_step<CC, G, R, -1>(prow, novalid, h2, vcur, acc, pre);
-            prow += Gm::PITCH;
-            advance(vcur);
-            fwd_step<CC, G, R, -1>(prow, novalid, h2, vnext, acc, pre);
-            prow += Gm::PITCH;
-        }
-    } else {
-#pragma unroll 1
-        for (int s = R - 1; s < K51; ++s) {             // steady state: all rows active
-            advance(vnext);
-            fwd_step<CC, G, R, -1>(prow, novalid, h2, vcur, acc, pre);
-#pragma unroll
-            for (int pp = 0; pp < Gm::NP; ++pp) vcur[pp] = vnext[pp];
-            prow += Gm::PITCH;
-        }
-    }
-    SSTEM_FWD_EDGE_STEP(51) SSTEM_FWD_EDGE_STEP(52) SSTEM_FWD_EDGE_STEP(53) SSTEM_FWD_EDGE_STEP(54)
-    SSTEM_FWD_EDGE_STEP(55) SSTEM_FWD_EDGE_STEP(56) SSTEM_FWD_EDGE_STEP(57)
-#undef SSTEM_FWD_EDGE_STEP
-    static_assert(R <= 8, "edge-step list covers R <= 8");
+    for (int t = 0; t < ((CC >= 3) ? FWD_NPRE : FWD_NPRE1); ++t) pre[t] = prow[G * t];
+    walk_steps<R, CC == 1>([&](auto S, int, auto& vuse, auto& vfill) {
+        vr.advance(vfill);
+        fwd_step<CC, G, R, decltype(S)::value>(prow, novalid, h2, vuse, acc, pre);
+        prow += Gm::PITCH;
+    }, vcur, vnext);
 
     // ---- sum the G tap groups of each pixel: lane g ends up with rows g*(R/G).. of every channel
     constexpr int NV = (R >= G) ? R : G;
@@ -479,10 +465,10 @@ template <int CC, int G, int R, int S, bool WV, bool WH>
 __device__ __forceinline__ void bwd_step(const float* __restrict__ prow0, bool novalid,
                                          const float2 (&g2)[CC][R / 2], const float2 (&h2)[R / 2][Geo<G, R>::NT],
                                          const float2 (&v2)[R / 2], float2 (&gh2)[R / 2][Geo<G, R>::NT],
-                                         float2 (&gvp)[R / 2], float (&pre)[CC][SSTEM_BWD_NPRE + 1]) {
+                                         float2 (&gvp)[R / 2], float (&pre)[CC][BWD_NPRE + 1]) {
     using Gm = Geo<G, R>;
     constexpr int NP = Gm::NP, NT = Gm::NT;
-    constexpr int NPRE = SSTEM_BWD_NPRE;                 // first taps of the NEXT row are loaded one step early
+    constexpr int NPRE = BWD_NPRE;                       // first taps of the NEXT row are loaded one step early
     if (CC == 1) {
         // One channel (also the gray x3 shortcut): t = g * P, so g factors out of both sums --
         //   gv[fy] = g * sum_fx P h[fx],   gh[fx] = g * sum_fy P v[fy]
@@ -511,10 +497,7 @@ __device__ __forceinline__ void bwd_step(const float* __restrict__ prow0, bool n
         for (int t = 0; t < NPRE; ++t) pre[0][t] = prow0[Gm::PITCH + G * t];
         return;
     }
-#ifndef SSTEM_BWD_TB
-#define SSTEM_BWD_TB ((NT + 1) / 2)
-#endif
-    constexpr int TB = SSTEM_BWD_TB;                     // taps per block: NP*TB independent FFMA2 chains
+    constexpr int TB = (NT + 1) / 2;                     // taps per block: NP*TB independent FFMA2 chains
     float2 gva[NP], gvb[NP];                             // two partial sums per row pair
 #pragma unroll
     for (int pp = 0; pp < NP; ++pp) gva[pp] = gvb[pp] = make_float2(0.f, 0.f);
@@ -573,11 +556,8 @@ __device__ __forceinline__ void bwd_step(const float* __restrict__ prow0, bool n
 // TAIL (fused interpolation tail, CC == 1): `in` is the UNPADDED frame [B, cs.., H, W] with batch
 // stride `in_bstride`; the window is its replicate-padded channel sum, gout is [B,1,H,W] and is
 // scaled by `gscale` (= 1/C of the channel mean) -- see interp_tail_fwd_k51_kernel.
-#ifndef SSTEM_BWD_MINB
-#define SSTEM_BWD_MINB 2
-#endif
 template <int CC, int G, int R, bool VEC, bool PAIR, bool WV, bool WH, bool ACCUM, bool TAIL = false>
-__global__ void __launch_bounds__(128, SSTEM_BWD_MINB)
+__global__ void __launch_bounds__(128, MIN_CTAS)
 sepconv_bwd_taps_k51_kernel(const float* __restrict__ gout, const float* __restrict__ in,
                             const float* __restrict__ v, const float* __restrict__ h,
                             float* __restrict__ gv, float* __restrict__ gh,
@@ -659,11 +639,6 @@ sepconv_bwd_taps_k51_kernel(const float* __restrict__ gout, const float* __restr
     // gv[fy = s - g][y0 + g][x]: pointer for s = 0, advanced by one plane per step
     float* gv_ptr = WV ? gv + b * K51 * plane + (int64_t)min(y0 + g, H - 1) * W + x - (int64_t)g * plane : nullptr;
     const bool gv_row_ok = col_ok && (y0 + g < H);
-    auto advance = [&](float2 (&vdst)[NP]) {
-        cp_async_wait<VDEPTH - 3>();
-        __syncwarp();
-        if (WH) { vr.issue(); vr.read(vdst); } else cp_async_commit();
-    };
     auto store_gv = [&](int s, float2 (&gvp)[NP]) {
         if (WV) {
             float val[R];
@@ -676,49 +651,23 @@ sepconv_bwd_taps_k51_kernel(const float* __restrict__ gout, const float* __restr
         }
     };
     float2 gvp[NP];
-    float pre[CC][SSTEM_BWD_NPRE + 1];
+    float pre[CC][BWD_NPRE + 1];
 #pragma unroll
     for (int c = 0; c < CC; ++c)
 #pragma unroll
-        for (int t = 0; t < SSTEM_BWD_NPRE; ++t) pre[c][t] = prow[c * Gm::ROWS * Gm::PITCH + G * t];
-#define SSTEM_BWD_EDGE_STEP(S)                                                        \
-    if ((S) < R - 1 || ((S) >= K51 && (S) < Gm::ROWS)) {                              \
-        advance(vnext);                                                               \
-        bwd_step<CC, G, R, S, WV, WH>(prow, novalid, g2, h2, vcur, gh2, gvp, pre);    \
-        store_gv(S, gvp);                                                             \
-        _Pragma("unroll") for (int pp = 0; pp < NP; ++pp) vcur[pp] = vnext[pp];       \
-        prow += Gm::PITCH;                                                            \
-    }
-    SSTEM_BWD_EDGE_STEP(0) SSTEM_BWD_EDGE_STEP(1) SSTEM_BWD_EDGE_STEP(2) SSTEM_BWD_EDGE_STEP(3)
-    SSTEM_BWD_EDGE_STEP(4) SSTEM_BWD_EDGE_STEP(5) SSTEM_BWD_EDGE_STEP(6)
-    static_assert((K51 - R + 1) % 2 == 0, "the two-step steady loop needs an even number of steady steps");
-    if constexpr (SSTEM_UNROLL2 && CC == 1) {            // see sepconv_fwd_k51_kernel
-#pragma unroll 1
-        for (int s = R - 1; s < K51; s += 2) {
-            advance(vnext);
-            bwd_step<CC, G, R, -1, WV, WH>(prow, novalid, g2, h2, vcur, gh2, gvp, pre);
-            store_gv(s, gvp);
-            prow += Gm::PITCH;
-            advance(vcur);
-            bwd_step<CC, G, R, -1, WV, WH>(prow, novalid, g2, h2, vnext, gh2, gvp, pre);
-            store_gv(s + 1, gvp);
-            prow += Gm::PITCH;
+        for (int t = 0; t < BWD_NPRE; ++t) pre[c][t] = prow[c * Gm::ROWS * Gm::PITCH + G * t];
+    walk_steps<R, CC == 1>([&](auto S, int s, auto& vuse, auto& vfill) {
+        if (WH) {
+            vr.advance(vfill);
+        } else {                                         // no v taps: keep the cp.async group arithmetic
+            cp_async_wait<VDEPTH - 3>();
+            __syncwarp();
+            cp_async_commit();
         }
-    } else {
-#pragma unroll 1
-        for (int s = R - 1; s < K51; ++s) {
-            advance(vnext);
-            bwd_step<CC, G, R, -1, WV, WH>(prow, novalid, g2, h2, vcur, gh2, gvp, pre);
-            store_gv(s, gvp);
-#pragma unroll
-            for (int pp = 0; pp < NP; ++pp) vcur[pp] = vnext[pp];
-            prow += Gm::PITCH;
-        }
-    }
-    SSTEM_BWD_EDGE_STEP(51) SSTEM_BWD_EDGE_STEP(52) SSTEM_BWD_EDGE_STEP(53) SSTEM_BWD_EDGE_STEP(54)
-    SSTEM_BWD_EDGE_STEP(55) SSTEM_BWD_EDGE_STEP(56) SSTEM_BWD_EDGE_STEP(57)
-#undef SSTEM_BWD_EDGE_STEP
-    static_assert(R <= 8, "edge-step list covers R <= 8");
+        bwd_step<CC, G, R, decltype(S)::value, WV, WH>(prow, novalid, g2, h2, vuse, gh2, gvp, pre);
+        store_gv(s, gvp);
+        prow += Gm::PITCH;
+    }, vcur, vnext);
 
     // ---- gh: complete per lane (the sum over fy happened in registers) ---------------------------
     if (WH && col_ok) {
@@ -804,11 +753,11 @@ __device__ __forceinline__ void gi_step(float* __restrict__ trowA, int thr, bool
 }
 
 template <int CC, int R, bool VEC>
-__global__ void __launch_bounds__(128, 2)
+__global__ void __launch_bounds__(128, MIN_CTAS)
 sepconv_bwd_input_k51_kernel(const float* __restrict__ gout, const float* __restrict__ v,
                              const float* __restrict__ h, float* __restrict__ gi,
                              int C, int c0, int H, int W) {
-    constexpr int G = 4;
+    constexpr int G = FWD_G;
     using Gm = Geo<G, R>;
     static_assert(Gm::NT == 13, "rotation scheme is written for 4 tap groups of 13");
     extern __shared__ __align__(16) float tile[];      // [CC][ROWS][PITCH] gi accumulators + 4 warps x v ring
@@ -866,35 +815,13 @@ sepconv_bwd_input_k51_kernel(const float* __restrict__ gout, const float* __rest
     vr.read(vcur);
     float* trow = tile + xl + g + 8 * g;                // word of slot 0: x + g + 4*(2g)
     const int thr = 13 - 2 * g;
-    auto advance = [&]() {
-        cp_async_wait<VDEPTH - 3>();
-        __syncwarp();
-        vr.issue();
-        vr.read(vnext);
-    };
     for (int i = 0; i < warp; ++i) __syncthreads();     // skew: warp w runs w steps behind warp 0
-#define SSTEM_GI_EDGE_STEP(S)                                                       \
-    if ((S) < R - 1 || ((S) >= K51 && (S) < Gm::ROWS)) {                            \
-        advance();                                                                  \
-        gi_step<CC, R, S>(trow, thr, g3, g2, h2, vcur);                             \
-        _Pragma("unroll") for (int pp = 0; pp < Gm::NP; ++pp) vcur[pp] = vnext[pp]; \
-        trow += Gm::PITCH;                                                          \
-        __syncthreads();                                                            \
-    }
-    SSTEM_GI_EDGE_STEP(0) SSTEM_GI_EDGE_STEP(1) SSTEM_GI_EDGE_STEP(2) SSTEM_GI_EDGE_STEP(3)
-    SSTEM_GI_EDGE_STEP(4) SSTEM_GI_EDGE_STEP(5) SSTEM_GI_EDGE_STEP(6)
-#pragma unroll 1
-    for (int s = R - 1; s < K51; ++s) {
-        advance();
-        gi_step<CC, R, -1>(trow, thr, g3, g2, h2, vcur);
-#pragma unroll
-        for (int pp = 0; pp < Gm::NP; ++pp) vcur[pp] = vnext[pp];
+    walk_steps<R, false>([&](auto S, int, auto& vuse, auto& vfill) {
+        vr.advance(vfill);
+        gi_step<CC, R, decltype(S)::value>(trow, thr, g3, g2, h2, vuse);
         trow += Gm::PITCH;
         __syncthreads();
-    }
-    SSTEM_GI_EDGE_STEP(51) SSTEM_GI_EDGE_STEP(52) SSTEM_GI_EDGE_STEP(53) SSTEM_GI_EDGE_STEP(54)
-    SSTEM_GI_EDGE_STEP(55) SSTEM_GI_EDGE_STEP(56) SSTEM_GI_EDGE_STEP(57)
-#undef SSTEM_GI_EDGE_STEP
+    }, vcur, vnext);
     for (int i = warp; i < 3; ++i) __syncthreads();     // every warp passes the same number of barriers
     __syncthreads();
 
@@ -934,11 +861,8 @@ struct TailFrames {                                     // indexed by the frame 
     const float* h[2];
 };
 
-#ifndef SSTEM_TAIL_MINB
-#define SSTEM_TAIL_MINB 2
-#endif
 template <int G, int R, bool VEC>
-__global__ void __launch_bounds__(128, SSTEM_TAIL_MINB)
+__global__ void __launch_bounds__(128, MIN_CTAS)
 interp_tail_fwd_k51_kernel(const __grid_constant__ TailFrames fa, int64_t frame_bstride, int cs, int nplanes,
                            float* __restrict__ out, float scale, int H, int W) {
     using Gm = Geo<G, R>;
@@ -984,48 +908,14 @@ interp_tail_fwd_k51_kernel(const __grid_constant__ TailFrames fa, int64_t frame_
         float2 vcur[Gm::NP], vnext[Gm::NP];
         vr.read(vcur);
         const float* prow = tile + xl + g;
-        auto advance = [&](float2 (&vdst)[Gm::NP]) {
-            cp_async_wait<VDEPTH - 3>();
-            __syncwarp();
-            vr.issue();
-            vr.read(vdst);
-        };
-        float pre[SSTEM_FWD_NPRE + 1];
+        float pre[FWD_NPRE + 1];
 #pragma unroll
-        for (int t = 0; t < SSTEM_FWD_NPRE1; ++t) pre[t] = prow[G * t];
-#define SSTEM_TAIL_EDGE_STEP(S)                                                    \
-    if ((S) < R - 1 || ((S) >= K51 && (S) < Gm::ROWS)) {                           \
-        advance(vnext);                                                            \
-        fwd_step<1, G, R, S>(prow, novalid, h2, vcur, acc, pre);                   \
-        _Pragma("unroll") for (int pp = 0; pp < Gm::NP; ++pp) vcur[pp] = vnext[pp]; \
-        prow += Gm::PITCH;                                                         \
-    }
-        SSTEM_TAIL_EDGE_STEP(0) SSTEM_TAIL_EDGE_STEP(1) SSTEM_TAIL_EDGE_STEP(2) SSTEM_TAIL_EDGE_STEP(3)
-        SSTEM_TAIL_EDGE_STEP(4) SSTEM_TAIL_EDGE_STEP(5) SSTEM_TAIL_EDGE_STEP(6)
-#if SSTEM_UNROLL2
-#pragma unroll 1
-        for (int s = R - 1; s < K51; s += 2) {
-            advance(vnext);
-            fwd_step<1, G, R, -1>(prow, novalid, h2, vcur, acc, pre);
+        for (int t = 0; t < FWD_NPRE1; ++t) pre[t] = prow[G * t];
+        walk_steps<R, true>([&](auto S, int, auto& vuse, auto& vfill) {
+            vr.advance(vfill);
+            fwd_step<1, G, R, decltype(S)::value>(prow, novalid, h2, vuse, acc, pre);
             prow += Gm::PITCH;
-            advance(vcur);
-            fwd_step<1, G, R, -1>(prow, novalid, h2, vnext, acc, pre);
-            prow += Gm::PITCH;
-        }
-#else
-#pragma unroll 1
-        for (int s = R - 1; s < K51; ++s) {
-            advance(vnext);
-            fwd_step<1, G, R, -1>(prow, novalid, h2, vcur, acc, pre);
-#pragma unroll
-            for (int pp = 0; pp < Gm::NP; ++pp) vcur[pp] = vnext[pp];
-            prow += Gm::PITCH;
-        }
-#endif
-        SSTEM_TAIL_EDGE_STEP(51) SSTEM_TAIL_EDGE_STEP(52) SSTEM_TAIL_EDGE_STEP(53) SSTEM_TAIL_EDGE_STEP(54)
-        SSTEM_TAIL_EDGE_STEP(55) SSTEM_TAIL_EDGE_STEP(56) SSTEM_TAIL_EDGE_STEP(57)
-#undef SSTEM_TAIL_EDGE_STEP
-        static_assert(R <= 8, "edge-step list covers R <= 8");
+        }, vcur, vnext);
     }
 
     constexpr int NV = (R >= G) ? R : G;
@@ -1063,6 +953,52 @@ int set_smem_once(Kern kern, size_t smem, PerDeviceOnce& done) {
 template <int G, int R, int CC>
 constexpr size_t smem_bytes() {
     return ((size_t)CC * Geo<G, R>::ROWS * Geo<G, R>::PITCH + 4 * VDEPTH * Geo<G, R>::SLOT) * sizeof(float);
+}
+
+// grid.y (row tiles) and grid.z (images) of a generation-1 launch are limited to 65535
+template <int R>
+bool fits_grid(int64_t B, int64_t H) { return B <= 65535 && (H + R - 1) / R <= 65535; }
+
+// VEC: the v ring is fed with 16-byte copies (W % 4 == 0, v 16-byte aligned)
+inline bool ring_vec(int64_t W, const float* v) { return (W & 3) == 0 && aligned16(v); }
+// PAIR: the padded input window is staged with 8-byte copies ((W + 50) even, `in` 8-byte aligned)
+inline bool window_pair(int64_t W, const float* in) {
+    return ((W + K51 - 1) & 1) == 0 && (reinterpret_cast<uintptr_t>(in) & 7u) == 0;
+}
+
+// f(std::true_type or std::false_type for each flag, in order): the runtime flags become template arguments
+template <class F>
+int dispatch(F&& f) { return f(); }
+template <class F, class... Flags>
+int dispatch(F&& f, bool flag, Flags... rest) {
+    if (flag) return dispatch([&](auto... t) { return f(std::true_type{}, t...); }, rest...);
+    return dispatch([&](auto... t) { return f(std::false_type{}, t...); }, rest...);
+}
+
+// One launch of a generation-1 kernel on 128 threads per R-row x TILE_W-column tile of each of B images.  `smem` is the
+// most the kernel may use (its attribute, set once per device; one PerDeviceOnce per kernel, as launch_persistent),
+// `smem_used` what this launch uses.
+template <auto Kern, int G, int R, class... Args>
+int launch_k51(size_t smem, size_t smem_used, int64_t B, int H, int W, cudaStream_t s, const Args&... args) {
+    static PerDeviceOnce done;
+    if (int e = set_smem_once(Kern, smem, done)) return e;
+    const dim3 grid((unsigned)((W + Geo<G, R>::TILE_W - 1) / Geo<G, R>::TILE_W), (unsigned)((H + R - 1) / R), (unsigned)B);
+    Kern<<<grid, 128, smem_used, s>>>(args...);
+    count_launch();
+    return finish_launch();
+}
+
+// Channel chunks of at most three planes, in order: f(std::integral_constant<int, CC>, c0) for each, until one fails.
+template <class F>
+int for_each_chunk(int64_t C, F&& f) {
+    for (int c0 = 0; c0 < C;) {
+        const int cc = C - c0 < 3 ? (int)(C - c0) : 3;
+        const int e = cc == 3 ? f(std::integral_constant<int, 3>{}, c0)
+                              : (cc == 2 ? f(std::integral_constant<int, 2>{}, c0) : f(std::integral_constant<int, 1>{}, c0));
+        if (e) return e;
+        c0 += cc;
+    }
+    return 0;
 }
 
 }  // namespace

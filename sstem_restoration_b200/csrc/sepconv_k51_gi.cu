@@ -5,33 +5,16 @@ namespace sstem {
 
 int launch_sepconv_bwd_input_k51(const float* g, const float* v, const float* h, float* gi,
                                  int64_t B, int64_t C, int64_t H, int64_t W, cudaStream_t s) {
-    constexpr int G = 4, R = 8;
-    if (B > 65535 || (H + R - 1) / R > 65535)
-        return launch_sepconv_bwd_input_generic(g, v, h, gi, B, C, H, W, 51, s);
+    if (!fits_grid<FWD_R>(B, H)) return launch_sepconv_bwd_input_generic(g, v, h, gi, B, C, H, W, 51, s);
     cudaError_t e = cudaMemsetAsync(gi, 0, (size_t)B * C * (H + K51 - 1) * (W + K51 - 1) * sizeof(float), s);
     if (e != cudaSuccess) return (int)e;
-    const bool vec = ((W & 3) == 0) && aligned16(v);
-    dim3 grid((unsigned)((W + Geo<G, R>::TILE_W - 1) / Geo<G, R>::TILE_W), (unsigned)((H + R - 1) / R), (unsigned)B);
-    int c0 = 0;
-    while (c0 < C) {
-        const int cc = (C - c0) < 3 ? (int)(C - c0) : 3;
-#define SSTEM_GI_LAUNCH(CC_, VEC_)                                                                   \
-    {                                                                                                 \
-        constexpr size_t smem = smem_bytes<G, R, CC_>();                                              \
-        static PerDeviceOnce done;                                                                    \
-        auto kern = sepconv_bwd_input_k51_kernel<CC_, R, VEC_>;                                    \
-        if (int err = set_smem_once(kern, smem, done)) return err;                                    \
-        kern<<<grid, 128, smem, s>>>(g, v, h, gi, (int)C, c0, (int)H, (int)W);                        \
-    }
-        if (cc == 3) { if (vec) SSTEM_GI_LAUNCH(3, true) else SSTEM_GI_LAUNCH(3, false) }
-        else if (cc == 2) { if (vec) SSTEM_GI_LAUNCH(2, true) else SSTEM_GI_LAUNCH(2, false) }
-        else { if (vec) SSTEM_GI_LAUNCH(1, true) else SSTEM_GI_LAUNCH(1, false) }
-#undef SSTEM_GI_LAUNCH
-        count_launch();
-        if (int err = finish_launch()) return err;
-        c0 += cc;
-    }
-    return 0;
+    return for_each_chunk(C, [&](auto cc, int c0) {
+        return dispatch([&](auto vec) {
+            constexpr size_t smem = smem_bytes<FWD_G, FWD_R, decltype(cc)::value>();
+            return launch_k51<sepconv_bwd_input_k51_kernel<decltype(cc)::value, FWD_R, decltype(vec)::value>, FWD_G, FWD_R>(
+                smem, smem, B, (int)H, (int)W, s, g, v, h, gi, (int)C, c0, (int)H, (int)W);
+        }, ring_vec(W, v));
+    });
 }
 
 }  // namespace sstem

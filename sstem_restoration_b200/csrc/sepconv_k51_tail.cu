@@ -2,68 +2,52 @@
 #include "sepconv_k51.cuh"
 
 namespace sstem {
+namespace {
+
+// up to 3 channel planes are staged side by side: the kernel's attribute allows 3, a launch uses `nplanes`
+template <int G, int R>
+size_t tail_smem_used(int nplanes) {
+    return nplanes == 1 ? smem_bytes<G, R, 1>() : (nplanes == 2 ? smem_bytes<G, R, 2>() : smem_bytes<G, R, 3>());
+}
+
+}  // namespace
 
 int launch_interp_tail_fwd_k51(const float* frame1, const float* frame2, int64_t frame_bstride,
                                const float* k1v, const float* k1h, const float* k2v, const float* k2h, float* out,
                                int64_t B, int64_t C, int64_t H, int64_t W, bool gray, cudaStream_t s) {
-    constexpr int G = SSTEM_FWD_G, R = SSTEM_FWD_R;
-    if (B > 65535 || (H + R - 1) / R > 65535) return SSTEM_E_SHAPE;
-    constexpr size_t smem = smem_bytes<G, R, 3>();          // up to 3 channel planes are staged side by side
+    if (!fits_grid<FWD_R>(B, H)) return SSTEM_E_SHAPE;
     const int cs = gray ? 1 : (int)C;
     const int nplanes = cs <= 3 ? cs : 1;
-    const size_t smem_used = nplanes == 1 ? smem_bytes<G, R, 1>() : (nplanes == 2 ? smem_bytes<G, R, 2>() : smem);
     const float scale = gray ? 1.f : 1.f / (float)C;
-    const bool vec = ((W & 3) == 0) && aligned16(k1v) && aligned16(k2v);
-    dim3 grid((unsigned)((W + Geo<G, R>::TILE_W - 1) / Geo<G, R>::TILE_W), (unsigned)((H + R - 1) / R), (unsigned)B);
     const TailFrames fa = {{frame2, frame1}, {k2v, k1v}, {k2h, k1h}};   // frame 2 first, as the reference's expression
-    if (vec) {
-        static PerDeviceOnce done;
-        auto kern = interp_tail_fwd_k51_kernel<G, R, true>;
-        if (int e = set_smem_once(kern, smem, done)) return e;
-        kern<<<grid, 128, smem_used, s>>>(fa, frame_bstride, cs, nplanes, out, scale, (int)H, (int)W);
-    } else {
-        static PerDeviceOnce done;
-        auto kern = interp_tail_fwd_k51_kernel<G, R, false>;
-        if (int e = set_smem_once(kern, smem, done)) return e;
-        kern<<<grid, 128, smem_used, s>>>(fa, frame_bstride, cs, nplanes, out, scale, (int)H, (int)W);
-    }
-    count_launch();
-    return finish_launch();
+    return dispatch([&](auto vec) {
+        return launch_k51<interp_tail_fwd_k51_kernel<FWD_G, FWD_R, decltype(vec)::value>, FWD_G, FWD_R>(
+            smem_bytes<FWD_G, FWD_R, 3>(), tail_smem_used<FWD_G, FWD_R>(nplanes), B, (int)H, (int)W, s,
+            fa, frame_bstride, cs, nplanes, out, scale, (int)H, (int)W);
+    }, ring_vec(W, k1v) && ring_vec(W, k2v));
 }
-
-namespace {
-template <bool VEC, bool WV, bool WH>
-int launch_tail_bwd_variant(const float* g, const float* frame, int64_t frame_bstride, const float* v, const float* h,
-                            float* gv, float* gh, int64_t B, int H, int W, int cs, float gscale, cudaStream_t s) {
-    constexpr int G = SSTEM_BWD_G, R = SSTEM_BWD_R;
-    constexpr size_t smem = smem_bytes<G, R, 3>();          // up to 3 channel planes are staged side by side
-    const int nplanes = cs <= 3 ? cs : 1;
-    const size_t smem_used = nplanes == 1 ? smem_bytes<G, R, 1>() : (nplanes == 2 ? smem_bytes<G, R, 2>() : smem);
-    static PerDeviceOnce done;
-    auto kern = sepconv_bwd_taps_k51_kernel<1, G, R, VEC, false, WV, WH, false, true>;
-    if (int e = set_smem_once(kern, smem, done)) return e;
-    dim3 grid((unsigned)((W + Geo<G, R>::TILE_W - 1) / Geo<G, R>::TILE_W), (unsigned)((H + R - 1) / R), (unsigned)B);
-    kern<<<grid, 128, smem_used, s>>>(g, frame, v, h, gv, gh, 1, 0, H, W, 1, frame_bstride, cs, nplanes, gscale, nullptr, 0);
-    count_launch();
-    return finish_launch();
-}
-}  // namespace
 
 // tap gradients of ONE frame of the fused tail (the two frames are independent)
 int launch_interp_tail_bwd_k51(const float* g, const float* frame, int64_t frame_bstride, const float* v, const float* h,
                                float* gv, float* gh, int64_t B, int64_t C, int64_t H, int64_t W, bool gray, cudaStream_t s) {
-    if (B > 65535 || (H + SSTEM_BWD_R - 1) / SSTEM_BWD_R > 65535) return SSTEM_E_SHAPE;
+    if (!fits_grid<BWD_R>(B, H)) return SSTEM_E_SHAPE;
     const int cs = gray ? 1 : (int)C;
+    const int nplanes = cs <= 3 ? cs : 1;
     const float gscale = gray ? 1.f : 1.f / (float)C;
-    const bool vec = ((W & 3) == 0) && aligned16(v);
-#define SSTEM_TAIL_BWD(VEC_)                                                                                              \
-    {                                                                                                                      \
-        if (gv && gh) return launch_tail_bwd_variant<VEC_, true, true>(g, frame, frame_bstride, v, h, gv, gh, B, (int)H, (int)W, cs, gscale, s);  \
-        if (gv) return launch_tail_bwd_variant<VEC_, true, false>(g, frame, frame_bstride, v, h, gv, gh, B, (int)H, (int)W, cs, gscale, s);       \
-        return launch_tail_bwd_variant<VEC_, false, true>(g, frame, frame_bstride, v, h, gv, gh, B, (int)H, (int)W, cs, gscale, s);               \
-    }
-    if (vec) SSTEM_TAIL_BWD(true) else SSTEM_TAIL_BWD(false)
-#undef SSTEM_TAIL_BWD
+    auto launch = [&](auto vec, auto wv, auto wh) {
+        return launch_k51<sepconv_bwd_taps_k51_kernel<1, BWD_G, BWD_R, decltype(vec)::value, false, decltype(wv)::value,
+                                                      decltype(wh)::value, false, true>, BWD_G, BWD_R>(
+            smem_bytes<BWD_G, BWD_R, 3>(), tail_smem_used<BWD_G, BWD_R>(nplanes), B, (int)H, (int)W, s,
+            g, frame, v, h, gv, gh, 1, 0, (int)H, (int)W, 1, frame_bstride, cs, nplanes, gscale, nullptr, 0);
+    };
+    // one kernel per combination of gradients written: gv and gh, gv only, gh only
+    using T = std::true_type;
+    using F = std::false_type;
+    return dispatch([&](auto vec) {
+        if (gv && gh) return launch(vec, T{}, T{});
+        if (gv) return launch(vec, T{}, F{});
+        return launch(vec, F{}, T{});
+    }, ring_vec(W, v));
 }
 
 }  // namespace sstem

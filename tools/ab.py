@@ -1,6 +1,6 @@
 """A/B harness for compile-time kernel variants.
 
-    python tools/ab.py build  NAME=-DSSTEM_BWD_NPRE=5 OTHER="-DSSTEM_FWD_NPRE1=8 -DSSTEM_TAIL_MINB=3"   # here (no GPU): nvcc
+    python tools/ab.py build  MINB1=-DSSTEM_BWD3_MINB=1 PHASES=-DSSTEM_V3_PHASES                      # here (no GPU): nvcc
     gpurun -- 'python tools/ab.py run fwd bwd tail'                                                       # on the GPU box
 
 `build` compiles one extra copy of the library per NAME into gpurun_scratch/lib_NAME.so (they travel to the GPU box with
