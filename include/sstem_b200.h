@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define SSTEM_ABI_VERSION 5
+#define SSTEM_ABI_VERSION 6
 
 /* argument errors (negative) */
 #define SSTEM_E_NULL      (-1)  /* a required pointer is NULL */
@@ -364,6 +364,34 @@ int sstem_tap_conv3x3_pack_weights_adjoint(const float* weight, float* packed, i
 int sstem_tap_conv3x3_backward(const float* grad_out, const float* x, const float* packed_adjoint,
                                float* grad_x, float* grad_weight, float* grad_bias,
                                int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream);
+
+/*
+ * Tap branch convolutions: the three half-resolution layers of IFNet._kernel_module in front of the tap producer,
+ *     Conv2d(cin, cout, 3, 1, 1) -> ReLU       (sff_scripts_interp/model/model_interp.py:129-137, run at :86-89)
+ * as one sm_100a kernel per layer: y = relu?(conv3x3(x, W) + b), stride 1, zero padding 1, no upsample; tcgen05 TF32
+ * implicit GEMM with the producer's operand encoding (same arithmetic class as sstem_tap_conv3x3).
+ *
+ * Chunk-major layout (the activations between the layers): [B][C8/4][h][w][4], C8 = channels rounded up to 8, i.e.
+ * element (b, ch, y, x) at ((b * C8/4 + ch/4) * h + y) * w + x) * 4 + ch % 4; sstem_chunked_elems(B, c, h, w) floats.
+ * Values are rounded to TF32 (cvt.rna) and the padding channels hold 0.  A chunk-major input must obey both; the kernel
+ * writes its chunk-major output that way.
+ *
+ *   x       [B, cin, h, w] NCHW (converted to chunk-major in a stream-ordered workspace, TF32-rounded), or chunk-major
+ *           with SSTEM_BRANCH_IN_CHUNKED (16-byte aligned).  Both give bit-identical results.
+ *   weight  [cout, cin, 3, 3], cin <= 64, cout <= 64; packed once by sstem_branch_conv3x3_pack_weights into
+ *           sstem_branch_conv3x3_packed_elems() floats ([tap][cin chunk of 4 < 16][64][4], zero padded, rounded to TF32)
+ *   bias    [cout] or NULL
+ *   out     [B, cout, h, w] NCHW in full fp32, or chunk-major with SSTEM_BRANCH_OUT_CHUNKED (16-byte aligned)
+ * SSTEM_BRANCH_RELU applies ReLU (before the TF32 rounding of a chunk-major output).
+ */
+#define SSTEM_BRANCH_RELU 1u
+#define SSTEM_BRANCH_IN_CHUNKED 2u
+#define SSTEM_BRANCH_OUT_CHUNKED 4u
+int64_t sstem_branch_conv3x3_packed_elems(void);
+int sstem_branch_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream);
+int64_t sstem_chunked_elems(int64_t B, int64_t c, int64_t h, int64_t w);
+int sstem_branch_conv3x3(const float* x, const float* packed_weight, const float* bias, float* out,
+                         int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream);
 
 /*
  * Gray x3 detection on the device, without a host round trip.  Every reference caller feeds sepconv a grayscale section

@@ -22,7 +22,10 @@ from .warp import SpatialTransformation, image_warp  # noqa: F401
 from .host import sepconv_forward_backward_host, join_host_pipeline  # noqa: F401
 from .stack_io import sections_to_input, prediction_to_uint8  # noqa: F401
 from .stack import restore_stack, warp_stitch, warp_and_stitch  # noqa: F401
-from .tapconv import tap_conv3x3, pack_tap_conv_weight, pack_tap_conv_weight_adjoint, TapConv3x3Function, ModuleTapProducer  # noqa: F401
+from .tapconv import (  # noqa: F401
+    tap_conv3x3, pack_tap_conv_weight, pack_tap_conv_weight_adjoint, TapConv3x3Function, ModuleTapProducer,
+    branch_conv3x3, pack_branch_conv_weight, ModuleTapBranch,
+)
 from . import shard, synth, sff_sim  # noqa: F401
 
 __all__ = [
@@ -31,5 +34,6 @@ __all__ = [
     "taps_from_tiled", "SeparableConvolutionTiled", "ModuleInterpolationTailTiled",
     "SpatialTransformation", "image_warp", "sepconv_forward_backward_host", "join_host_pipeline", "SstemError", "launch_count", "fp32_peak_probe",
     "sections_to_input", "prediction_to_uint8", "restore_stack", "warp_stitch", "warp_and_stitch",
-    "tap_conv3x3", "pack_tap_conv_weight", "pack_tap_conv_weight_adjoint", "TapConv3x3Function", "ModuleTapProducer", "shard", "synth", "sff_sim",
+    "tap_conv3x3", "pack_tap_conv_weight", "pack_tap_conv_weight_adjoint", "TapConv3x3Function", "ModuleTapProducer",
+    "branch_conv3x3", "pack_branch_conv_weight", "ModuleTapBranch", "shard", "synth", "sff_sim",
 ]

@@ -13,7 +13,7 @@ import threading
 from ._build import LIB_PATH as _DEFAULT_LIB_PATH, needs_build as _needs_build
 
 #: must equal SSTEM_ABI_VERSION of include/sstem_b200.h (checked against the loaded library in load())
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 #: SSTEM_LIB_PATH selects another build of the same library (kernel-tuning experiments)
 LIB_PATH = os.environ.get("SSTEM_LIB_PATH") or _DEFAULT_LIB_PATH
@@ -29,6 +29,9 @@ SEPCONV_GRAY_REPLICATED = 2
 SEPCONV_ACCUMULATE = 4
 TAPCONV_UPSAMPLE2X = 1
 TAPCONV_TILED = 2
+BRANCH_RELU = 1
+BRANCH_IN_CHUNKED = 2
+BRANCH_OUT_CHUNKED = 4
 LAYOUT_NCHW = 0
 LAYOUT_NHWC = 1
 PIX_U8 = 0
@@ -46,6 +49,7 @@ EXPORTED_SYMBOLS = (
     "sstem_sepconv_forward_detect", "sstem_sepconv_backward_detect",
     "sstem_tap_conv3x3_packed_elems", "sstem_tap_conv3x3_pack_weights", "sstem_tap_conv3x3",
     "sstem_tap_conv3x3_pack_weights_adjoint", "sstem_tap_conv3x3_backward",
+    "sstem_branch_conv3x3_packed_elems", "sstem_branch_conv3x3_pack_weights", "sstem_chunked_elems", "sstem_branch_conv3x3",
     "sstem_fp32_peak_probe", "sstem_launch_count", "sstem_abi_version", "sstem_error_string",
 )
 
@@ -122,6 +126,14 @@ def load() -> ctypes.CDLL:
         lib.sstem_tap_conv3x3_pack_weights_adjoint.restype = ctypes.c_int
         lib.sstem_tap_conv3x3_backward.argtypes = [_c_p] * 6 + [_c_i64, _c_i32, _c_i32, _c_i64, _c_i64, _c_u32, _c_p]
         lib.sstem_tap_conv3x3_backward.restype = ctypes.c_int
+        lib.sstem_branch_conv3x3_packed_elems.argtypes = []
+        lib.sstem_branch_conv3x3_packed_elems.restype = _c_i64
+        lib.sstem_branch_conv3x3_pack_weights.argtypes = [_c_p, _c_p, _c_i32, _c_i32, _c_p]
+        lib.sstem_branch_conv3x3_pack_weights.restype = ctypes.c_int
+        lib.sstem_chunked_elems.argtypes = [_c_i64] * 4
+        lib.sstem_chunked_elems.restype = _c_i64
+        lib.sstem_branch_conv3x3.argtypes = [_c_p, _c_p, _c_p, _c_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i64, _c_u32, _c_p]
+        lib.sstem_branch_conv3x3.restype = ctypes.c_int
         lib.sstem_fp32_peak_probe.argtypes = [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
         lib.sstem_fp32_peak_probe.restype = ctypes.c_int
         lib.sstem_launch_count.argtypes = []

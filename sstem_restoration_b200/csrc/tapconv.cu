@@ -24,6 +24,8 @@
 // and profiles/tapconv_r2.md.
 // The backward (sstem_tap_conv3x3_backward, DESIGN 4.11b) is at the end of this file: the input gradient reuses this kernel
 // on the adjoint weights, the weight gradient is tap_conv3x3_wgrad_kernel.
+// The three half-resolution convolutions in front of the producer (sstem_branch_conv3x3, DESIGN 4.11c) follow the
+// producer's weight packing, on the same machinery fed by TMA from a chunk-major activation layout.
 #include <string.h>
 
 #include <algorithm>
@@ -795,6 +797,242 @@ int pack_weights(const float* weight, float* packed, int cin, int cout, int max_
     return finish_launch();
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Tap branch convolutions (sstem_branch_conv3x3, DESIGN 4.11c): the three half-resolution layers in front of the
+// producer, Conv2d(cin <= 64, cout <= 64, 3, 1, 1) -> ReLU, on the producer's operand encoding.  Activations between the
+// layers are chunk-major, [B][C8/4][h][w][4] (C8 = channels rounded up to 8; padding channels 0), already rounded to TF32,
+// so the patch needs no producer warps: one TMA box {40 floats = 10 pixels x 4 channels, 18 rows, 4 chunks} of that
+// layout lands as [chunk][patch pixel][4], the canonical K-major operand of tap_conv3x3_kernel, and its out-of-image part
+// is zero-filled, which is the convolution's zero padding.  Roles: 4 epilogue warps (TMEM -> + bias -> ReLU -> store), 1
+// MMA warp (walks the loop uniformly, one lane issues), 1 warp whose lane 0 issues the bulk / TMA copies.
+constexpr int BC_MAXC = 64;
+constexpr int BC_CHUNKS = BC_MAXC / 4;                     // 16 weight chunks per tap
+constexpr int BC_SLOT_CHUNKS = 4;                          // a ring slot holds a quarter of a 64-channel patch: 2 K-steps
+constexpr int BC_SLOTS = 6;                                // 1.5 tiles of 64-channel patches in flight
+constexpr unsigned BC_W_TAP_BYTES = BC_CHUNKS * TC_N * 16;                     // 16384
+constexpr unsigned BC_W_BYTES = 9 * BC_W_TAP_BYTES;                            // 147456
+constexpr unsigned BC_SLOT_BYTES = BC_SLOT_CHUNKS * TC_NPIX * 16;              // 11520
+constexpr unsigned BC_OFF_A = BC_W_BYTES;
+constexpr unsigned BC_OFF_BIAS = BC_OFF_A + BC_SLOTS * BC_SLOT_BYTES;          // 216576
+constexpr unsigned BC_OFF_BAR = BC_OFF_BIAS + TC_N * 4;
+constexpr unsigned BC_SMEM = BC_OFF_BAR + 256 + 128;       // + barriers and the TMEM address + alignment slack = 217 216
+static_assert(BC_SMEM <= 232448, "shared memory budget");
+static_assert(8 * (1 + 2 * BC_SLOTS + 4) + 4 <= 256, "barrier block");
+constexpr int BC_THREADS = (TC_EPI_WARPS + 2) * 32;        // 192
+
+struct BranchConvShape {
+    int h, w, cout;
+    int tiles_x, tiles_y, ntiles;
+    int in_chunks, out_chunks;                             // C8 / 4 of the input and of the output
+    int k_steps;                                           // C8in / 8
+    int slots_per_tile;                                    // ceil(k_steps / 2)
+    int relu;
+};
+
+// OUT_CHUNKED: the output is chunk-major and TF32-rounded (the next layer's input); else NCHW in full fp32
+template <bool OUT_CHUNKED>
+__global__ void __launch_bounds__(BC_THREADS, 1)
+branch_conv3x3_kernel(const __grid_constant__ CUtensorMap map_x, const float* __restrict__ wpacked,
+                      const float* __restrict__ bias, float* __restrict__ out, const BranchConvShape sh) {
+    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
+    const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
+    unsigned char* gen = tc_smem_raw + (base - (unsigned)__cvta_generic_to_shared(tc_smem_raw));
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    // barriers: weights, slot full x 6, slot empty x 6, acc_full x 2, acc_empty x 2; the TMEM base address after them
+    const unsigned bar = base + BC_OFF_BAR;
+    const unsigned b_w = bar, b_full = bar + 8, b_empty = b_full + 8 * BC_SLOTS, b_accfull = b_empty + 8 * BC_SLOTS,
+                   b_accempty = b_accfull + 16;
+    if (tid == 0) {
+        mbar_init(b_w, 1);
+        for (int s = 0; s < BC_SLOTS; ++s) {
+            mbar_init(b_full + 8 * s, 1);
+            mbar_init(b_empty + 8 * s, 1);
+        }
+        for (int s = 0; s < 2; ++s) {
+            mbar_init(b_accfull + 8 * s, 1);
+            mbar_init(b_accempty + 8 * s, TC_EPI_WARPS * 32);
+        }
+        mbar_fence_init();
+    }
+    if (tid < TC_N) reinterpret_cast<float*>(gen + BC_OFF_BIAS)[tid] = (bias != nullptr && tid < sh.cout) ? bias[tid] : 0.f;
+    const unsigned tmem = tmem_alloc<TC_TMEM_COLS>(bar + 8 * (1 + 2 * BC_SLOTS + 4), warp);
+
+    // tiles blockIdx.x, + gridDim.x, ... walked without divisions, as in tap_conv3x3_kernel
+    struct TileIter {
+        int tile, tx, ty, b;
+    };
+    const int step_tx = (int)gridDim.x % sh.tiles_x, step_r = (int)gridDim.x / sh.tiles_x;
+    auto first_tile = [&]() {
+        TileIter t;
+        t.tile = blockIdx.x;
+        const int r = t.tile / sh.tiles_x;
+        t.tx = t.tile - r * sh.tiles_x;
+        t.b = r / sh.tiles_y;
+        t.ty = r - t.b * sh.tiles_y;
+        return t;
+    };
+    auto advance = [&](TileIter& t) {
+        t.tile += gridDim.x;
+        t.tx += step_tx;
+        int dr = step_r;
+        if (t.tx >= sh.tiles_x) { t.tx -= sh.tiles_x; ++dr; }
+        t.ty += dr;
+        while (t.ty >= sh.tiles_y) { t.ty -= sh.tiles_y; ++t.b; }
+    };
+
+    if (warp < TC_EPI_WARPS) {
+        // ===================== epilogue: TMEM lanes 32 * warp .. + 31 = tile pixels (row 4 * warp + lane / 8, column lane % 8)
+        const float* sbias = reinterpret_cast<const float*>(gen + BC_OFF_BIAS);
+        const int r = warp * 4 + (lane >> 3), c = lane & 7;
+        const int64_t plane = (int64_t)sh.h * sh.w;
+        int it = 0;
+        for (TileIter ti = first_tile(); ti.tile < sh.ntiles; advance(ti), ++it) {
+            const int as = it & 1;
+            tc_wait(b_accfull + 8 * as, (it >> 1) & 1);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            unsigned v[64];
+#pragma unroll
+            for (int hh = 0; hh < 2; ++hh) {
+                const unsigned ta = tmem + ((unsigned)(warp * 32) << 16) + as * TC_N + hh * 32;
+                asm volatile(
+                    "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
+                    "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+                    : "=r"(v[hh*32+0]), "=r"(v[hh*32+1]), "=r"(v[hh*32+2]), "=r"(v[hh*32+3]), "=r"(v[hh*32+4]), "=r"(v[hh*32+5]),
+                      "=r"(v[hh*32+6]), "=r"(v[hh*32+7]), "=r"(v[hh*32+8]), "=r"(v[hh*32+9]), "=r"(v[hh*32+10]), "=r"(v[hh*32+11]),
+                      "=r"(v[hh*32+12]), "=r"(v[hh*32+13]), "=r"(v[hh*32+14]), "=r"(v[hh*32+15]), "=r"(v[hh*32+16]), "=r"(v[hh*32+17]),
+                      "=r"(v[hh*32+18]), "=r"(v[hh*32+19]), "=r"(v[hh*32+20]), "=r"(v[hh*32+21]), "=r"(v[hh*32+22]), "=r"(v[hh*32+23]),
+                      "=r"(v[hh*32+24]), "=r"(v[hh*32+25]), "=r"(v[hh*32+26]), "=r"(v[hh*32+27]), "=r"(v[hh*32+28]), "=r"(v[hh*32+29]),
+                      "=r"(v[hh*32+30]), "=r"(v[hh*32+31])
+                    : "r"(ta));
+            }
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tc_arrive(b_accempty + 8 * as);                // the accumulator stage is free: the MMAs of tile it + 2 may start
+            const int Y = ti.ty * TC_TH + r, X = ti.tx * TC_TW + c;
+            if (Y >= sh.h || X >= sh.w) continue;
+            // ReLU before rounding (rounding keeps the sign); `x < 0` keeps a NaN a NaN, as torch's ReLU does
+            auto act = [&](int n) {
+                const float y = __uint_as_float(v[n]) + sbias[n];
+                return (sh.relu && y < 0.f) ? 0.f : y;
+            };
+            if (OUT_CHUNKED) {
+                // chunk k of the pixel: 16 bytes; a warp row of 8 pixels writes 128 contiguous bytes per chunk.  Padding
+                // channels come out 0: their weights and bias are 0.
+                float4* p = reinterpret_cast<float4*>(out) + ((int64_t)ti.b * sh.out_chunks * sh.h + Y) * sh.w + X;
+#pragma unroll
+                for (int k = 0; k < BC_CHUNKS; ++k)
+                    if (k < sh.out_chunks)
+                        p[k * plane] = make_float4(to_tf32(act(4 * k)), to_tf32(act(4 * k + 1)), to_tf32(act(4 * k + 2)), to_tf32(act(4 * k + 3)));
+            } else {
+                float* p = out + (int64_t)ti.b * sh.cout * plane + (int64_t)Y * sh.w + X;
+#pragma unroll
+                for (int n = 0; n < TC_N; ++n)
+                    if (n < sh.cout) p[(int64_t)n * plane] = act(n);
+            }
+        }
+    } else if (warp == TC_EPI_WARPS) {
+        // ===================== MMA issuer: the whole warp walks the loop (uniform descriptors), one lane issues
+        const unsigned tmem_u = __shfl_sync(0xffffffffu, tmem, 0);
+        tc_wait(b_w, 0);
+        constexpr unsigned idesc = tc_idesc_tf32(128, TC_N);
+        constexpr int KS_SLOT = BC_SLOT_CHUNKS / 2;        // K-steps per slot
+        // start-address fields only (units of 16 bytes): per tap + (dy * 10 + dx) pixels of the patch and + 16 chunks of
+        // the weights, per K-step + 2 chunks of each
+        const uint64_t db0 = tc_desc(base, TC_N * 16, 128);
+        int slot = 0;
+        unsigned sph = 0;
+        int it = 0;
+        for (int tile = blockIdx.x; tile < sh.ntiles; tile += gridDim.x, ++it) {
+            const int as = it & 1;
+            tc_wait(b_accempty + 8 * as, ((it >> 1) & 1) ^ 1);   // accumulator stage drained (passes at once the first time)
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const unsigned d_tmem = tmem_u + as * TC_N;
+#pragma unroll 1
+            for (int q = 0; q < sh.slots_per_tile; ++q) {
+                tc_wait(b_full + 8 * slot, sph);           // the TMA box of this quarter patch has landed
+                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                const uint64_t da0 = tc_desc(base + BC_OFF_A + slot * BC_SLOT_BYTES, TC_NPIX * 16, TC_PW * 16);
+                const uint64_t dbq = db0 + (uint64_t)(q * KS_SLOT * 2 * TC_N);
+                const int ks_n = min(sh.k_steps - q * KS_SLOT, KS_SLOT);
+#pragma unroll
+                for (int tap = 0; tap < 9; ++tap) {
+#pragma unroll
+                    for (int ks = 0; ks < KS_SLOT; ++ks) {
+                        if (ks >= ks_n) break;
+                        const uint64_t da = da0 + (uint64_t)((tap / 3) * TC_PW + (tap % 3) + ks * 2 * TC_NPIX);
+                        const uint64_t db = dbq + (uint64_t)((tap * BC_W_TAP_BYTES + ks * 2 * TC_N * 16) >> 4);
+                        if (lane == 0) tc_mma(d_tmem, da, db, idesc, (q | tap | ks) != 0);
+                    }
+                }
+                __syncwarp();
+                if (lane == 0) tc_commit(b_empty + 8 * slot);   // slot may be refilled once these MMAs have read it
+                if (++slot == BC_SLOTS) { slot = 0; sph ^= 1; }
+            }
+            __syncwarp();
+            if (lane == 0) tc_commit(b_accfull + 8 * as);  // accumulator complete
+        }
+    } else {
+        // ===================== copies: the weights once, then a quarter patch per slot, running up to 6 slots ahead
+        if (lane == 0) {
+            tma_prefetch_desc(&map_x);
+            mbar_expect_tx(b_w, BC_W_BYTES);
+            for (int t = 0; t < 9; ++t)
+                bulk_load(base + t * BC_W_TAP_BYTES, reinterpret_cast<const char*>(wpacked) + (size_t)t * BC_W_TAP_BYTES, BC_W_TAP_BYTES, b_w);
+            int slot = 0;
+            unsigned sph = 0;
+            for (TileIter ti = first_tile(); ti.tile < sh.ntiles; advance(ti)) {
+                // box origin: one pixel up and left of the tile (zero-filled outside the image), chunk q of image b
+                const int x0 = 4 * (ti.tx * TC_TW - 1), y0 = ti.ty * TC_TH - 1, c0 = ti.b * sh.in_chunks;
+                for (int q = 0; q < sh.slots_per_tile; ++q) {
+                    tc_wait(b_empty + 8 * slot, sph ^ 1);
+                    mbar_expect_tx(b_full + 8 * slot, BC_SLOT_BYTES);
+                    tma_load_3d(base + BC_OFF_A + slot * BC_SLOT_BYTES, &map_x, b_full + 8 * slot, x0, y0, c0 + q * BC_SLOT_CHUNKS);
+                    if (++slot == BC_SLOTS) { slot = 0; sph ^= 1; }
+                }
+            }
+        }
+        __syncwarp();
+    }
+
+    tmem_dealloc<TC_TMEM_COLS>(tmem, warp);
+}
+
+// weights [cout][cin][3][3] -> [tap][chunk < 16][n = 64][4], zero padded, rounded to TF32
+__global__ void branch_conv3x3_pack_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int)(BC_W_BYTES / 4)) return;
+    const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % BC_CHUNKS, tap = (i >> 2) / TC_N / BC_CHUNKS;
+    const int ch = ck * 4 + j;
+    packed[i] = (n < cout && ch < cin) ? to_tf32(w[((int64_t)n * cin + ch) * 9 + tap]) : 0.f;
+}
+
+// [B][c][h][w] -> chunk-major [B][chunks][h][w][4], rounded to TF32, channels past c = 0.  Thread = (image, chunk, pixel).
+__global__ void __launch_bounds__(256)
+nchw_to_chunked_kernel(const float* __restrict__ x, float* __restrict__ out, int64_t n, int c, int chunks, int64_t plane) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int64_t p = i % plane, bk = i / plane;
+    const int k = (int)(bk % chunks);
+    const float* src = x + ((bk / chunks) * c + 4 * k) * plane + p;
+    float q[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) q[j] = 4 * k + j < c ? to_tf32(__ldg(src + j * plane)) : 0.f;
+    reinterpret_cast<float4*>(out)[i] = make_float4(q[0], q[1], q[2], q[3]);
+}
+
+int launch_branch_conv(const float* xc, const float* wpacked, const float* bias, float* out, int64_t B, const BranchConvShape& sh,
+                       bool out_chunked, cudaStream_t s) {
+    // 3-D map over the chunk-major input: (chunk channel x column) merged into 160-byte box rows, rows, (image x chunk)
+    CUtensorMap map;
+    const int64_t dims[3] = {4 * (int64_t)sh.w, sh.h, B * sh.in_chunks};
+    const int64_t strides[3] = {1, 4 * (int64_t)sh.w, 4 * (int64_t)sh.h * sh.w};
+    const int box[3] = {4 * TC_PW, TC_PH, BC_SLOT_CHUNKS};
+    if (!make_map_f32(&map, xc, 3, dims, strides, box)) return SSTEM_E_SHAPE;
+    const int ctas = std::min(sh.ntiles, sm_count());
+    return out_chunked ? launch_tc<branch_conv3x3_kernel<true>>(BC_SMEM, BC_THREADS, ctas, s, map, wpacked, bias, out, sh)
+                       : launch_tc<branch_conv3x3_kernel<false>>(BC_SMEM, BC_THREADS, ctas, s, map, wpacked, bias, out, sh);
+}
+
 }  // namespace
 
 }  // namespace sstem
@@ -884,4 +1122,66 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
         if (e) return e;
     }
     return 0;
+}
+
+extern "C" int64_t sstem_branch_conv3x3_packed_elems(void) { return (int64_t)BC_W_BYTES / 4; }
+
+extern "C" int sstem_branch_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
+    if (!weight || !packed) return SSTEM_E_NULL;
+    if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
+    if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
+    DeviceGuard guard(packed);
+    if (guard.err) return guard.err;
+    const int total = (int)(BC_W_BYTES / 4);
+    branch_conv3x3_pack_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(weight, packed, cin, cout);
+    count_launch();
+    return finish_launch();
+}
+
+extern "C" int64_t sstem_chunked_elems(int64_t B, int64_t c, int64_t h, int64_t w) {
+    if (B <= 0 || c <= 0 || h <= 0 || w <= 0) return 0;
+    return B * ((c + 7) / 8 * 8) * h * w;
+}
+
+extern "C" int sstem_branch_conv3x3(const float* x, const float* packed_weight, const float* bias, float* out,
+                                    int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream) {
+    if (!x || !packed_weight || !out) return SSTEM_E_NULL;
+    if (flags & ~(SSTEM_BRANCH_RELU | SSTEM_BRANCH_IN_CHUNKED | SSTEM_BRANCH_OUT_CHUNKED)) return SSTEM_E_FLAG;
+    const bool in_chunked = flags & SSTEM_BRANCH_IN_CHUNKED, out_chunked = flags & SSTEM_BRANCH_OUT_CHUNKED;
+    if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
+    if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
+    BranchConvShape sh;
+    sh.h = (int)h; sh.w = (int)w; sh.cout = cout;
+    sh.tiles_x = (sh.w + TC_TW - 1) / TC_TW;
+    sh.tiles_y = (sh.h + TC_TH - 1) / TC_TH;
+    sh.in_chunks = (cin + 7) / 8 * 2;
+    sh.out_chunks = (cout + 7) / 8 * 2;
+    sh.k_steps = sh.in_chunks / 2;
+    sh.slots_per_tile = (sh.in_chunks + BC_SLOT_CHUNKS - 1) / BC_SLOT_CHUNKS;
+    sh.relu = (flags & SSTEM_BRANCH_RELU) ? 1 : 0;
+    // tile indices and the TMA chunk coordinate are 32-bit
+    if ((int64_t)sh.tiles_x * sh.tiles_y * B > INT32_MAX / 2 || B * sh.in_chunks > INT32_MAX / 2) return SSTEM_E_SHAPE;
+    sh.ntiles = (int)((int64_t)sh.tiles_x * sh.tiles_y * B);
+    if (!(in_chunked ? aligned16(x) : aligned4(x)) || !aligned16(packed_weight) || !(out_chunked ? aligned16(out) : aligned4(out)) ||
+        (bias && !aligned4(bias)))
+        return SSTEM_E_ALIGN;
+    DeviceGuard guard(out);
+    if (guard.err) return guard.err;
+    cudaStream_t s = (cudaStream_t)stream;
+    const float* xc = x;
+    float* ws = nullptr;
+    if (!in_chunked) {   // NCHW input: a TF32-rounded chunk-major copy in a stream-ordered workspace
+        const int64_t n = B * sh.in_chunks * h * w;
+        if (workspace_alloc(reinterpret_cast<void**>(&ws), (size_t)n * 16, s)) return cudaErrorMemoryAllocation;
+        nchw_to_chunked_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(x, ws, n, cin, sh.in_chunks, h * w);
+        count_launch();
+        if (int e = finish_launch()) {
+            cudaFreeAsync(ws, s);
+            return e;
+        }
+        xc = ws;
+    }
+    const int e = launch_branch_conv(xc, packed_weight, bias, out, B, sh, out_chunked, s);
+    if (ws) cudaFreeAsync(ws, s);
+    return e;
 }

@@ -43,6 +43,11 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, u
         ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(map), "r"((unsigned)__cvta_generic_to_shared(bar)),
           "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
+__device__ __forceinline__ void tma_load_3d(unsigned dst, const CUtensorMap* map, unsigned bar, int c0, int c1, int c2) {
+    asm volatile(
+        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
+}
 __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
     asm volatile(
         "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"

@@ -6,7 +6,11 @@
 (csrc/tapconv.cu: tcgen05 TF32 implicit GEMM, the upsample folded into the operand producer), writing the taps in the
 layout of ``Conv2d`` or directly tile-major for :func:`sstem_restoration_b200.sepconv_forward_tiled`.
 :func:`tap_conv3x3` is forward only (the stack-restoration path, c5); :class:`TapConv3x3Function` and
-``ModuleTapProducer(trainable=True)`` add the backward (tcgen05 kernels as well) for training.  No CPU / PyTorch fallback.
+``ModuleTapProducer(trainable=True)`` add the backward (tcgen05 kernels as well) for training.
+
+The three half-resolution ``Conv2d -> ReLU`` layers in front of them run on :func:`branch_conv3x3` (csrc/tapconv.cu, the same
+tcgen05 machinery fed by TMA from a chunk-major activation layout); :class:`ModuleTapBranch` is the whole branch, forward
+only.  No CPU / PyTorch fallback.
 """
 import torch
 
@@ -160,3 +164,96 @@ class ModuleTapProducer(torch.nn.Module):
         need_adjoint = torch.is_grad_enabled() and x.requires_grad
         adjoint = self._cached("_packed_adjoint", pack_tap_conv_weight_adjoint, x.device) if need_adjoint else None
         return TapConv3x3Function.apply(x, self.weight, self.bias, self.upsample, self.tiled, packed, adjoint)
+
+
+def pack_branch_conv_weight(weight: torch.Tensor) -> torch.Tensor:
+    """``Conv2d.weight`` ``[cout<=64, cin<=64, 3, 3]`` -> the resident image of :func:`branch_conv3x3` (144 KB,
+    TF32-rounded).  Pack once per layer, reuse for every call."""
+    if weight.is_cuda == False:
+        raise NotImplementedError()
+    if weight.dtype != torch.float32 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3):
+        raise TypeError("pack_branch_conv_weight: float32 [cout, cin, 3, 3] required")
+    cout, cin = weight.shape[:2]
+    if cin > 64 or cout > 64:
+        raise ValueError("pack_branch_conv_weight: cin <= 64 and cout <= 64 required")
+    lib = _lib.load()
+    packed = torch.empty(lib.sstem_branch_conv3x3_packed_elems(), dtype=torch.float32, device=weight.device)
+    code = lib.sstem_branch_conv3x3_pack_weights(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
+    if code:
+        _lib.check(code, "sstem_branch_conv3x3_pack_weights")
+    packed._sstem_cin_cout = (int(cin), int(cout))
+    return packed
+
+
+def branch_conv3x3(x: torch.Tensor, packed: torch.Tensor, bias=None, relu=True, chunked_in=False, chunked_out=False) -> torch.Tensor:
+    """``relu?(conv2d(x, weight, bias, stride 1, padding 1))``, one half-resolution layer of a tap branch.
+
+    ``packed`` comes from :func:`pack_branch_conv_weight` (it carries cin / cout).  x is ``[B, cin, h, w]`` or, with
+    ``chunked_in``, chunk-major ``[B, C8/4, h, w, 4]`` (C8 = cin rounded up to 8; values TF32-rounded, padding channels 0:
+    what ``chunked_out`` returns).  Returns ``[B, cout, h, w]`` in full fp32 or, with ``chunked_out``, chunk-major.
+    Forward only."""
+    if x.is_cuda == False:
+        raise NotImplementedError()
+    if x.dtype != torch.float32 or x.dim() != (5 if chunked_in else 4) or not x.is_contiguous():
+        raise TypeError("branch_conv3x3: contiguous float32 [B, cin, h, w] (chunk-major: [B, C8/4, h, w, 4]) required")
+    if torch.is_grad_enabled() and x.requires_grad:
+        raise NotImplementedError("branch_conv3x3 is forward only: call it under torch.no_grad() or detach its input")
+    cin, cout = getattr(packed, "_sstem_cin_cout", (None, None))
+    if cin is None:
+        raise ValueError("branch_conv3x3: the packed weight must come from pack_branch_conv_weight")
+    B, c, h, w = x.shape[:4]
+    if (c, x.shape[-1]) != (((cin + 7) // 8 * 2, 4) if chunked_in else (cin, w)):
+        raise ValueError(f"branch_conv3x3: x {tuple(x.shape)} does not match the weight's {cin} input channels")
+    shape = (B, (cout + 7) // 8 * 2, h, w, 4) if chunked_out else (B, cout, h, w)
+    out = torch.empty(shape, dtype=torch.float32, device=x.device)
+    if out.numel():
+        flags = ((_lib.BRANCH_RELU if relu else 0) | (_lib.BRANCH_IN_CHUNKED if chunked_in else 0)
+                 | (_lib.BRANCH_OUT_CHUNKED if chunked_out else 0))
+        code = _lib.load().sstem_branch_conv3x3(x.data_ptr(), packed.data_ptr(), bias.contiguous().data_ptr() if bias is not None else None,
+                                                out.data_ptr(), B, cin, cout, h, w, flags, _stream_ptr(x))
+        if code:
+            _lib.check(code, "sstem_branch_conv3x3")
+    return out
+
+
+class _BranchConv(ModuleTapProducer):
+    """One ``Conv2d(cin, cout, 3, 1, 1) -> ReLU`` of a tap branch on :func:`branch_conv3x3`, its weight packed on first use
+    and again whenever it changes."""
+
+    def __init__(self, in_channels, out_channels):
+        super().__init__(in_channels, out_channels, upsample=False)
+
+    def forward(self, x, chunked_in, chunked_out):
+        packed = self._cached("_packed", pack_branch_conv_weight, x.device)
+        return branch_conv3x3(x, packed, self.bias.detach(), relu=True, chunked_in=chunked_in, chunked_out=chunked_out)
+
+
+class ModuleTapBranch(torch.nn.Module):
+    """Drop-in for a whole tap branch, ``IFNet._kernel_module`` (model_interp.py:129-137):
+
+        Conv2d(in, mid, 3, 1, 1), ReLU, Conv2d(mid, mid, 3, 1, 1), ReLU, Conv2d(mid, taps, 3, 1, 1), ReLU,
+        Upsample(scale_factor=2, mode='bilinear', align_corners=True), Conv2d(taps, taps, 3, 1, 1)
+
+    Its state_dict has the keys of that ``nn.Sequential`` (``0.*``, ``2.*``, ``4.*``, ``7.*``), so
+    ``m.load_state_dict(net.upconv51_1.state_dict())`` loads a reference branch.  The three half-resolution layers run on
+    :func:`branch_conv3x3` (NCHW in, chunk-major between them, ``[B, taps, h, w]`` out), the last two on the tap producer;
+    ``tiled=True`` returns the taps tile-major (:func:`sstem_restoration_b200.sepconv_forward_tiled`'s layout).  Forward
+    only: an input that requires grad raises."""
+
+    def __init__(self, in_channels=64, mid_channels=64, taps=51, tiled=True):
+        super().__init__()
+        self.in_channels = in_channels
+        self.add_module("0", _BranchConv(in_channels, mid_channels))
+        self.add_module("2", _BranchConv(mid_channels, mid_channels))
+        self.add_module("4", _BranchConv(mid_channels, taps))
+        self.add_module("7", ModuleTapProducer(taps, taps, upsample=True, tiled=tiled))
+
+    def forward(self, x):
+        if torch.is_grad_enabled() and x.requires_grad:
+            raise NotImplementedError("ModuleTapBranch is forward only: call it under torch.no_grad() or detach its input")
+        if x.dim() != 4 or x.shape[1] != self.in_channels:
+            raise ValueError(f"ModuleTapBranch: x [B, {self.in_channels}, h, w] required, got {tuple(x.shape)}")
+        a = getattr(self, "0")(x.contiguous(), chunked_in=False, chunked_out=True)
+        a = getattr(self, "2")(a, chunked_in=True, chunked_out=True)
+        a = getattr(self, "4")(a, chunked_in=True, chunked_out=False)
+        return getattr(self, "7")(a)
