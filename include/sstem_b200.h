@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define SSTEM_ABI_VERSION 6
+#define SSTEM_ABI_VERSION 7
 
 /* argument errors (negative) */
 #define SSTEM_E_NULL      (-1)  /* a required pointer is NULL */
@@ -392,6 +392,30 @@ int sstem_branch_conv3x3_pack_weights(const float* weight, float* packed, int32_
 int64_t sstem_chunked_elems(int64_t B, int64_t c, int64_t h, int64_t w);
 int sstem_branch_conv3x3(const float* x, const float* packed_weight, const float* bias, float* out,
                          int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream);
+
+/*
+ * Backward of one branch convolution, y = relu?(conv3x3(x, W) + b) as in sstem_branch_conv3x3 (for training IFNet with the
+ * tap branches in the graph), with the forward's flag bits: SSTEM_BRANCH_RELU masks with y, g = (y <= 0) ? 0 : grad_out
+ * (torch's threshold_backward: y == 0 gives 0, a NaN y passes the gradient); SSTEM_BRANCH_IN_CHUNKED says x is chunk-major and
+ * SSTEM_BRANCH_OUT_CHUNKED that y is, i.e. the saved activations come in the layouts the forward read and wrote.
+ * grad_out is [B, cout, h, w] NCHW.  Each non-NULL output is overwritten:
+ *
+ *   grad_x       [B, cin, h, w] NCHW   conv3x3(g, W'), W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]: the forward's tcgen05
+ *                                      convolution on W' (packed by sstem_branch_conv3x3_pack_weights_adjoint into
+ *                                      sstem_branch_conv3x3_packed_elems() floats) fed g chunk-major and TF32-rounded
+ *   grad_weight  [cout, cin, 3, 3]     sum over pixels of g x x shifted per tap: a persistent tcgen05 TF32 kernel
+ *   grad_bias    [cout]                fp32 sum of the unrounded g over pixels
+ *
+ * y may be NULL without SSTEM_BRANCH_RELU; packed_adjoint may be NULL when grad_x is.  cin, cout <= 64.  Chunk-major
+ * pointers 16-byte aligned.  Operands of products are rounded to TF32, sums accumulated in fp32; every gradient is
+ * run-to-run bit-identical on a given device and identical for either layout of x and y.  One stream-ordered workspace of
+ * B*C8out*h*w (g) + ~64*cout (bias partials) floats, plus B*C8in*h*w (NCHW x, grad_weight) and
+ * min(tiles, SMs / (cin > 32 ? 2 : 1)) * cout*cin*9 (grad_weight partials).
+ */
+int sstem_branch_conv3x3_pack_weights_adjoint(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream);
+int sstem_branch_conv3x3_backward(const float* grad_out, const float* y, const float* x, const float* packed_adjoint,
+                                  float* grad_x, float* grad_weight, float* grad_bias,
+                                  int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream);
 
 /*
  * Gray x3 detection on the device, without a host round trip.  Every reference caller feeds sepconv a grayscale section

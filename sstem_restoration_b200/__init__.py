@@ -24,7 +24,7 @@ from .stack_io import sections_to_input, prediction_to_uint8  # noqa: F401
 from .stack import restore_stack, warp_stitch, warp_and_stitch  # noqa: F401
 from .tapconv import (  # noqa: F401
     tap_conv3x3, pack_tap_conv_weight, pack_tap_conv_weight_adjoint, TapConv3x3Function, ModuleTapProducer,
-    branch_conv3x3, pack_branch_conv_weight, ModuleTapBranch,
+    branch_conv3x3, pack_branch_conv_weight, pack_branch_conv_weight_adjoint, branch_conv3x3_backward, ModuleTapBranch,
 )
 from . import shard, synth, sff_sim  # noqa: F401
 
@@ -35,5 +35,5 @@ __all__ = [
     "SpatialTransformation", "image_warp", "sepconv_forward_backward_host", "join_host_pipeline", "SstemError", "launch_count", "fp32_peak_probe",
     "sections_to_input", "prediction_to_uint8", "restore_stack", "warp_stitch", "warp_and_stitch",
     "tap_conv3x3", "pack_tap_conv_weight", "pack_tap_conv_weight_adjoint", "TapConv3x3Function", "ModuleTapProducer",
-    "branch_conv3x3", "pack_branch_conv_weight", "ModuleTapBranch", "shard", "synth", "sff_sim",
+    "branch_conv3x3", "pack_branch_conv_weight", "pack_branch_conv_weight_adjoint", "branch_conv3x3_backward", "ModuleTapBranch", "shard", "synth", "sff_sim",
 ]

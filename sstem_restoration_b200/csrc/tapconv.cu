@@ -25,7 +25,8 @@
 // The backward (sstem_tap_conv3x3_backward, DESIGN 4.11b) is at the end of this file: the input gradient reuses this kernel
 // on the adjoint weights, the weight gradient is tap_conv3x3_wgrad_kernel.
 // The three half-resolution convolutions in front of the producer (sstem_branch_conv3x3, DESIGN 4.11c) follow the
-// producer's weight packing, on the same machinery fed by TMA from a chunk-major activation layout.
+// producer's weight packing, on the same machinery fed by TMA from a chunk-major activation layout; their backward
+// (sstem_branch_conv3x3_backward, DESIGN 4.11d) runs that kernel on the adjoint weights and branch_conv3x3_wgrad_kernel.
 #include <string.h>
 
 #include <algorithm>
@@ -997,13 +998,18 @@ branch_conv3x3_kernel(const __grid_constant__ CUtensorMap map_x, const float* __
     tmem_dealloc<TC_TMEM_COLS>(tmem, warp);
 }
 
-// weights [cout][cin][3][3] -> [tap][chunk < 16][n = 64][4], zero padded, rounded to TF32
+// weights [cout][cin][3][3] -> [tap][chunk < 16][n = 64][4], zero padded, rounded to TF32.  ADJOINT: the image of
+// W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx] instead (cout -> cin channels), which the input gradient runs.
+template <bool ADJOINT>
 __global__ void branch_conv3x3_pack_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (int)(BC_W_BYTES / 4)) return;
     const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % BC_CHUNKS, tap = (i >> 2) / TC_N / BC_CHUNKS;
     const int ch = ck * 4 + j;
-    packed[i] = (n < cout && ch < cin) ? to_tf32(w[((int64_t)n * cin + ch) * 9 + tap]) : 0.f;
+    if (ADJOINT)                                           // W'[n][ch][tap] = W[ch][n][8 - tap]
+        packed[i] = (n < cin && ch < cout) ? to_tf32(w[((int64_t)ch * cin + n) * 9 + (8 - tap)]) : 0.f;
+    else
+        packed[i] = (n < cout && ch < cin) ? to_tf32(w[((int64_t)n * cin + ch) * 9 + tap]) : 0.f;
 }
 
 // [B][c][h][w] -> chunk-major [B][chunks][h][w][4], rounded to TF32, channels past c = 0.  Thread = (image, chunk, pixel).
@@ -1031,6 +1037,247 @@ int launch_branch_conv(const float* xc, const float* wpacked, const float* bias,
     const int ctas = std::min(sh.ntiles, sm_count());
     return out_chunked ? launch_tc<branch_conv3x3_kernel<true>>(BC_SMEM, BC_THREADS, ctas, s, map, wpacked, bias, out, sh)
                        : launch_tc<branch_conv3x3_kernel<false>>(BC_SMEM, BC_THREADS, ctas, s, map, wpacked, bias, out, sh);
+}
+
+// The callers check the limits first (see sstem_branch_conv3x3).
+BranchConvShape branch_conv_shape(int64_t B, int cin, int cout, int64_t h, int64_t w, bool relu) {
+    BranchConvShape sh;
+    sh.h = (int)h; sh.w = (int)w; sh.cout = cout;
+    sh.tiles_x = (sh.w + TC_TW - 1) / TC_TW;
+    sh.tiles_y = (sh.h + TC_TH - 1) / TC_TH;
+    sh.in_chunks = (cin + 7) / 8 * 2;
+    sh.out_chunks = (cout + 7) / 8 * 2;
+    sh.k_steps = sh.in_chunks / 2;
+    sh.slots_per_tile = (sh.in_chunks + BC_SLOT_CHUNKS - 1) / BC_SLOT_CHUNKS;
+    sh.relu = relu ? 1 : 0;
+    sh.ntiles = (int)((int64_t)sh.tiles_x * sh.tiles_y * B);
+    return sh;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Backward of y = relu?(conv3x3(x, W) + b) (sstem_branch_conv3x3_backward, DESIGN 4.11d).
+//
+// g = (y <= 0) ? 0 : grad_out (grad_out without the ReLU), NCHW -> chunk-major [B][C8/4][h][w][4] rounded to TF32: the input
+// of the adjoint convolution (grad_x = branch_conv3x3_kernel on W') and the A operand of the weight gradient.  The mask is
+// torch's threshold_backward on the output: y == 0 gives 0, a NaN y passes the gradient.  Each block also writes the fp32 sums of the UNROUNDED g of its
+// chunk's four channels (grad_bias, summed over blocks by tap_conv3x3_wgrad_reduce_kernel): per thread in pixel order, then
+// a fixed shuffle tree, then the warps in order, so the result is bit-identical from run to run.  Block = (image b,
+// chunk k, part bx of the plane), blockIdx.x = (b * chunks + k) * nbx + bx; bias partial p = b * nbx + bx.
+template <bool Y_CHUNKED>
+__global__ void __launch_bounds__(256)
+branch_grad_mask_kernel(const float* __restrict__ gy, const float* __restrict__ y, float* __restrict__ gc,
+                        float* __restrict__ part_b, int cout, int chunks, int nbx, int64_t plane) {
+    const int bx = blockIdx.x % nbx, bk = blockIdx.x / nbx, k = bk % chunks, b = bk / chunks;
+    const float* src = gy + ((int64_t)b * cout + 4 * k) * plane;
+    const float* ysrc = Y_CHUNKED ? y + (int64_t)bk * plane * 4 : y + ((int64_t)b * cout + 4 * k) * plane;
+    float4* dst = reinterpret_cast<float4*>(gc) + (int64_t)bk * plane;
+    float s[4] = {0.f, 0.f, 0.f, 0.f};
+    for (int64_t p = (int64_t)bx * blockDim.x + threadIdx.x; p < plane; p += (int64_t)nbx * blockDim.x) {
+        float yv[4] = {1.f, 1.f, 1.f, 1.f};                // no ReLU: every gradient passes
+        if (y && Y_CHUNKED) {
+            const float4 t = __ldg(reinterpret_cast<const float4*>(ysrc) + p);
+            yv[0] = t.x; yv[1] = t.y; yv[2] = t.z; yv[3] = t.w;
+        }
+        float q[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            float v = 0.f;
+            if (4 * k + j < cout) {
+                v = __ldg(src + j * plane + p);
+                if (y && !Y_CHUNKED) yv[j] = __ldg(ysrc + j * plane + p);
+                if (yv[j] <= 0.f) v = 0.f;
+            }
+            s[j] += v;
+            q[j] = to_tf32(v);
+        }
+        dst[p] = make_float4(q[0], q[1], q[2], q[3]);
+    }
+    __shared__ float red[8][4];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) s[j] += __shfl_xor_sync(0xffffffffu, s[j], o);
+        if (lane == 0) red[warp][j] = s[j];
+    }
+    __syncthreads();
+    if (threadIdx.x < 4 && 4 * k + (int)threadIdx.x < cout) {
+        float t = 0.f;
+        for (int q = 0; q < (int)(blockDim.x >> 5); ++q) t += red[q][threadIdx.x];
+        part_b[((int64_t)b * nbx + bx) * cout + 4 * k + threadIdx.x] = t;
+    }
+}
+
+// grad_weight.  Per 16 x 8 tile and tap (dy, dx):
+//     D_tap[co][ci] += sum_{pixels p} g[co][p] * x[ci][p + (dy, dx)]               (x zero padded by 1)
+// as tcgen05.mma kind::tf32, M = 64 (co, padded), N = 32 (ci), K = 8 = one tile row: 16 K-steps x 9 taps = 144 MMAs per
+// tile.  Nine accumulators of N = 64 would need 576 TMEM columns, so a CTA owns one half of the input channels (32, nine
+// accumulators = 288 columns, resident for the whole tile loop); CTAs 2j and 2j + 1 walk the same tiles for the two halves
+// (one CTA per pair when cin <= 32) and write the two halves of partial j.
+// Both operands are K-major, no swizzle (the encoding of the forward and of tap_conv3x3_wgrad_kernel), staged from the
+// chunk-major activations, which are already TF32-rounded: a thread loads four or more pixels of one chunk (16 bytes
+// each) and stores them transposed, one 16-byte row of four pixels per channel -- nothing is blended or rounded here:
+//   * A = g of the tile: [tile row][K half][co group of 8][8 co][4 pixels], 2 KB per row;
+//   * B = the 18 x 10 patch of x as three copies shifted by dx = 0, 1, 2 columns: [dx][patch row][K half][ci group of
+//     8][8 ci][4 pixels], 1 KB per row.  Tap (dy, dx), K-step ky reads copy dx at patch row ky + dy.
+// Two stages: the 8 staging warps load tile i + 1 into registers while the MMAs of tile i run, store it once the MMAs of
+// tile i - 1 have released its stage (tcgen05.commit), and 1 warp issues.  At the end warps 0-3 write the CTA's partial.
+constexpr int BW_STAGE_THREADS = 256;                      // thread = A item (tile row, co chunk) and B item (patch row, ci chunk)
+constexpr int BW_THREADS = BW_STAGE_THREADS + 32;          // + the MMA warp = 288
+constexpr int BW_M = 64, BW_N = 32;
+constexpr unsigned BW_A_ROW = 2 * (BW_M / 8) * 128;        // 2048
+constexpr unsigned BW_A_BYTES = TC_TH * BW_A_ROW;          // 32768
+constexpr unsigned BW_B_ROW = 2 * (BW_N / 8) * 128;        // 1024
+constexpr unsigned BW_B_COPY = TC_PH * BW_B_ROW;           // 18432
+constexpr unsigned BW_STAGE = BW_A_BYTES + 3 * BW_B_COPY;  // 88064
+constexpr unsigned BW_OFF_BAR = 2 * BW_STAGE;              // 176128
+constexpr unsigned BW_SMEM = BW_OFF_BAR + 64 + 128;        // + barriers, TMEM address, alignment slack = 176 320
+constexpr unsigned BW_TMEM_COLS = 512;                     // 288 used; an allocation is a power of 2
+static_assert(BW_SMEM <= 232448, "shared memory budget");
+static_assert(9 * BW_N <= (int)BW_TMEM_COLS, "nine accumulators in tensor memory");
+static_assert(TC_TH * (BW_M / 4) == BW_STAGE_THREADS && TC_PH * (BW_N / 4) <= BW_STAGE_THREADS, "one A and one B item per thread");
+
+struct BranchWgradShape {
+    int h, w, cin, cout;
+    int tiles_x, tiles_y, ntiles;
+    int in_chunks, out_chunks;                             // C8 / 4 of x and of g
+    int halves;                                            // CTAs per pair: 2 when cin > 32
+};
+
+__global__ void __launch_bounds__(BW_THREADS, 1)
+branch_conv3x3_wgrad_kernel(const float* __restrict__ g, const float* __restrict__ x, float* __restrict__ part_w,
+                            const BranchWgradShape sh) {
+    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
+    const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    // barriers: full x 2, empty x 2, done; the TMEM base address after them
+    const unsigned bar = base + BW_OFF_BAR;
+    const unsigned b_full = bar, b_empty = bar + 16, b_done = bar + 32;
+    if (tid == 0) {
+        for (int s = 0; s < 2; ++s) {
+            mbar_init(b_full + 8 * s, BW_STAGE_THREADS);
+            mbar_init(b_empty + 8 * s, 1);
+        }
+        mbar_init(b_done, 1);
+        mbar_fence_init();
+    }
+    // channels past cout / cin are never written and stay zero
+    for (unsigned i = tid; i < BW_OFF_BAR / 16; i += BW_THREADS) sts128(base + i * 16, 0.f, 0.f, 0.f, 0.f);
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    const unsigned tmem = tmem_alloc<BW_TMEM_COLS>(bar + 40, warp);
+    const int half = blockIdx.x % sh.halves, pair = blockIdx.x / sh.halves, npairs = gridDim.x / sh.halves;
+
+    if (warp < BW_STAGE_THREADS / 32) {
+        // ===================== staging
+        const int ay = tid >> 4, ak = tid & 15;            // A: tile row, g chunk (co 4 ak .. 4 ak + 3)
+        const int by = tid >> 3, bk = tid & 7;             // B: patch row, x chunk 8 half + bk (ci 32 half + 4 bk ..)
+        const bool a_item = ak < sh.out_chunks, b_item = by < TC_PH && 8 * half + bk < sh.in_chunks;
+        const float4* g4 = reinterpret_cast<const float4*>(g);
+        const float4* x4 = reinterpret_cast<const float4*>(x);
+        const unsigned a_off = ay * BW_A_ROW + ak * 64, b_off = BW_A_BYTES + by * BW_B_ROW + bk * 64;
+        // 4 pixels x 4 channels -> one 16-byte row of 4 pixels per channel (rows of a core matrix are 16 bytes apart)
+        auto store_t = [](unsigned dst, const float4& p0, const float4& p1, const float4& p2, const float4& p3) {
+            sts128(dst, p0.x, p1.x, p2.x, p3.x);
+            sts128(dst + 16, p0.y, p1.y, p2.y, p3.y);
+            sts128(dst + 32, p0.z, p1.z, p2.z, p3.z);
+            sts128(dst + 48, p0.w, p1.w, p2.w, p3.w);
+        };
+        const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+        int it = 0;
+        for (int tile = pair; tile < sh.ntiles; tile += npairs, ++it) {
+            const int s = it & 1;
+            const int r = tile / sh.tiles_x, tx = tile - r * sh.tiles_x, b = r / sh.tiles_y, ty = r - b * sh.tiles_y;
+            const int Y0 = ty * TC_TH, X0 = tx * TC_TW;
+            float4 av[8], bv[TC_PW];
+            if (a_item) {
+                const int Y = Y0 + ay;
+                const float4* p = g4 + ((int64_t)(b * sh.out_chunks + ak) * sh.h + min(Y, sh.h - 1)) * sh.w + X0;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) av[j] = (Y < sh.h && X0 + j < sh.w) ? __ldg(p + j) : zero;
+            }
+            if (b_item) {
+                const int Y = Y0 - 1 + by;
+                const bool row_in = Y >= 0 && Y < sh.h;
+                const float4* p = x4 + ((int64_t)(b * sh.in_chunks + 8 * half + bk) * sh.h + min(max(Y, 0), sh.h - 1)) * sh.w;
+#pragma unroll
+                for (int c = 0; c < TC_PW; ++c) {
+                    const int X = X0 - 1 + c;
+                    bv[c] = (row_in && X >= 0 && X < sh.w) ? __ldg(p + X) : zero;
+                }
+            }
+            tc_wait(b_empty + 8 * s, ((it >> 1) & 1) ^ 1);   // the MMAs of tile it - 2 have read this stage
+            const unsigned st = base + s * BW_STAGE;
+            if (a_item) {
+                store_t(st + a_off, av[0], av[1], av[2], av[3]);
+                store_t(st + a_off + BW_A_ROW / 2, av[4], av[5], av[6], av[7]);
+            }
+            if (b_item) {
+#pragma unroll
+                for (int dx = 0; dx < 3; ++dx) {
+                    store_t(st + b_off + dx * BW_B_COPY, bv[dx], bv[dx + 1], bv[dx + 2], bv[dx + 3]);
+                    store_t(st + b_off + dx * BW_B_COPY + BW_B_ROW / 2, bv[dx + 4], bv[dx + 5], bv[dx + 6], bv[dx + 7]);
+                }
+            }
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy stores -> visible to the tensor core
+            tc_arrive(b_full + 8 * s);
+        }
+    } else {
+        // ===================== MMA issuer: the whole warp walks the loop (uniform descriptors), one lane issues
+        const unsigned tmem_u = __shfl_sync(0xffffffffu, tmem, 0);
+        constexpr unsigned idesc = tc_idesc_tf32(BW_M, BW_N);
+        int it = 0;
+        for (int tile = pair; tile < sh.ntiles; tile += npairs, ++it) {
+            const int s = it & 1;
+            tc_wait(b_full + 8 * s, (it >> 1) & 1);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const uint64_t da0 = tc_desc(base + s * BW_STAGE, BW_A_ROW / 2, 128);
+            const uint64_t db0 = tc_desc(base + s * BW_STAGE + BW_A_BYTES, BW_B_ROW / 2, 128);
+#pragma unroll 1
+            for (int tap = 0; tap < 9; ++tap) {
+                const int dy = tap / 3, dx = tap % 3;
+                const unsigned d_tmem = tmem_u + tap * BW_N;
+#pragma unroll
+                for (int ky = 0; ky < TC_TH; ++ky) {
+                    const uint64_t da = da0 + (uint64_t)((ky * BW_A_ROW) >> 4);
+                    const uint64_t db = db0 + (uint64_t)((dx * BW_B_COPY + (ky + dy) * BW_B_ROW) >> 4);
+                    if (lane == 0) tc_mma(d_tmem, da, db, idesc, (it | ky) != 0);
+                }
+            }
+            __syncwarp();
+            if (lane == 0) tc_commit(b_empty + 8 * s);     // the stage may be refilled once these MMAs have read it
+            __syncwarp();
+        }
+        if (lane == 0) tc_commit(b_done);                  // every accumulator complete
+        __syncwarp();
+    }
+
+    if (warp < 4) {
+        // M = 64: row m of D is TMEM lane 32 (m / 16) + m % 16 (as in tap_conv3x3_wgrad_kernel), so warp q reads co
+        // 16 q .. 16 q + 15 in its lanes 0..15
+        tc_wait(b_done, 0);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        const int co = warp * 16 + lane, nci = min(sh.cin - half * BW_N, BW_N);
+        float* pw = part_w + (int64_t)pair * (sh.cout * sh.cin * 9) + ((int64_t)co * sh.cin + half * BW_N) * 9;
+#pragma unroll 1
+        for (int tap = 0; tap < 9; ++tap) {
+            unsigned v[32];
+            asm volatile(
+                "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
+                "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+                : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
+                  "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
+                  "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
+                  "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+                : "r"(tmem + ((unsigned)(warp * 32) << 16) + tap * BW_N));
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            if (lane < 16 && co < sh.cout) {
+#pragma unroll
+                for (int c = 0; c < BW_N; ++c)
+                    if (c < nci) pw[c * 9 + tap] = __uint_as_float(v[c]);
+            }
+        }
+    }
+    tmem_dealloc<BW_TMEM_COLS>(tmem, warp);
 }
 
 }  // namespace
@@ -1126,16 +1373,25 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
 
 extern "C" int64_t sstem_branch_conv3x3_packed_elems(void) { return (int64_t)BC_W_BYTES / 4; }
 
-extern "C" int sstem_branch_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
+template <bool ADJOINT>
+static int branch_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
     if (!weight || !packed) return SSTEM_E_NULL;
     if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
     if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
     DeviceGuard guard(packed);
     if (guard.err) return guard.err;
     const int total = (int)(BC_W_BYTES / 4);
-    branch_conv3x3_pack_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(weight, packed, cin, cout);
+    branch_conv3x3_pack_kernel<ADJOINT><<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(weight, packed, cin, cout);
     count_launch();
     return finish_launch();
+}
+
+extern "C" int sstem_branch_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
+    return branch_pack_weights<false>(weight, packed, cin, cout, stream);
+}
+
+extern "C" int sstem_branch_conv3x3_pack_weights_adjoint(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
+    return branch_pack_weights<true>(weight, packed, cin, cout, stream);
 }
 
 extern "C" int64_t sstem_chunked_elems(int64_t B, int64_t c, int64_t h, int64_t w) {
@@ -1150,18 +1406,10 @@ extern "C" int sstem_branch_conv3x3(const float* x, const float* packed_weight, 
     const bool in_chunked = flags & SSTEM_BRANCH_IN_CHUNKED, out_chunked = flags & SSTEM_BRANCH_OUT_CHUNKED;
     if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
     if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
-    BranchConvShape sh;
-    sh.h = (int)h; sh.w = (int)w; sh.cout = cout;
-    sh.tiles_x = (sh.w + TC_TW - 1) / TC_TW;
-    sh.tiles_y = (sh.h + TC_TH - 1) / TC_TH;
-    sh.in_chunks = (cin + 7) / 8 * 2;
-    sh.out_chunks = (cout + 7) / 8 * 2;
-    sh.k_steps = sh.in_chunks / 2;
-    sh.slots_per_tile = (sh.in_chunks + BC_SLOT_CHUNKS - 1) / BC_SLOT_CHUNKS;
-    sh.relu = (flags & SSTEM_BRANCH_RELU) ? 1 : 0;
     // tile indices and the TMA chunk coordinate are 32-bit
-    if ((int64_t)sh.tiles_x * sh.tiles_y * B > INT32_MAX / 2 || B * sh.in_chunks > INT32_MAX / 2) return SSTEM_E_SHAPE;
-    sh.ntiles = (int)((int64_t)sh.tiles_x * sh.tiles_y * B);
+    if (((w + TC_TW - 1) / TC_TW) * ((h + TC_TH - 1) / TC_TH) * B > INT32_MAX / 2 || B * ((cin + 7) / 8 * 2) > INT32_MAX / 2)
+        return SSTEM_E_SHAPE;
+    const BranchConvShape sh = branch_conv_shape(B, cin, cout, h, w, flags & SSTEM_BRANCH_RELU);
     if (!(in_chunked ? aligned16(x) : aligned4(x)) || !aligned16(packed_weight) || !(out_chunked ? aligned16(out) : aligned4(out)) ||
         (bias && !aligned4(bias)))
         return SSTEM_E_ALIGN;
@@ -1183,5 +1431,83 @@ extern "C" int sstem_branch_conv3x3(const float* x, const float* packed_weight, 
     }
     const int e = launch_branch_conv(xc, packed_weight, bias, out, B, sh, out_chunked, s);
     if (ws) cudaFreeAsync(ws, s);
+    return e;
+}
+
+extern "C" int sstem_branch_conv3x3_backward(const float* grad_out, const float* y, const float* x, const float* packed_adjoint,
+                                             float* grad_x, float* grad_weight, float* grad_bias,
+                                             int64_t B, int32_t cin, int32_t cout, int64_t h, int64_t w, uint32_t flags, void* stream) {
+    const bool relu = flags & SSTEM_BRANCH_RELU, in_chunked = flags & SSTEM_BRANCH_IN_CHUNKED, out_chunked = flags & SSTEM_BRANCH_OUT_CHUNKED;
+    if (!grad_out || !x || (relu && !y) || (grad_x && !packed_adjoint)) return SSTEM_E_NULL;
+    if (flags & ~(SSTEM_BRANCH_RELU | SSTEM_BRANCH_IN_CHUNKED | SSTEM_BRANCH_OUT_CHUNKED)) return SSTEM_E_FLAG;
+    if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
+    if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > BC_MAXC) return SSTEM_E_SHAPE;
+    const int in_chunks = (cin + 7) / 8 * 2, out_chunks = (cout + 7) / 8 * 2;
+    // tile indices, the TMA chunk coordinate of the adjoint convolution and the mask kernel's block index are 32-bit
+    if (((w + TC_TW - 1) / TC_TW) * ((h + TC_TH - 1) / TC_TH) * B > INT32_MAX / 2 || B * out_chunks * 64 > INT32_MAX / 2)
+        return SSTEM_E_SHAPE;
+    if (!aligned4(grad_out) || (y && !(out_chunked ? aligned16(y) : aligned4(y))) || !(in_chunked ? aligned16(x) : aligned4(x)) ||
+        (packed_adjoint && !aligned16(packed_adjoint)) || (grad_x && !aligned4(grad_x)) || (grad_weight && !aligned4(grad_weight)) ||
+        (grad_bias && !aligned4(grad_bias)))
+        return SSTEM_E_ALIGN;
+    if (!grad_x && !grad_weight && !grad_bias) return 0;
+    DeviceGuard guard(grad_out);
+    if (guard.err) return guard.err;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t plane = h * w;
+    const bool wgrad = grad_weight != nullptr;
+    const int halves = cin > BW_N ? 2 : 1;
+    const int pairs = (int)std::min<int64_t>(((w + TC_TW - 1) / TC_TW) * ((h + TC_TH - 1) / TC_TH) * B, std::max(sm_count() / halves, 1));
+    const int nw = cout * cin * 9;
+    // about 64 bias partials per channel whatever the batch: (64 / B) blocks per image and chunk
+    const int nbx = (int)std::max<int64_t>(64 / B, 1);
+    // one stream-ordered workspace: g chunk-major | bias partials | x chunk-major (NCHW x, weight gradient) | weight partials
+    const size_t g_floats = (size_t)(B * out_chunks * plane) * 4, pb_floats = (size_t)(B * nbx * cout);
+    const size_t xc_floats = (wgrad && !in_chunked) ? (size_t)(B * in_chunks * plane) * 4 : 0, pw_floats = wgrad ? (size_t)pairs * nw : 0;
+    const size_t off_pb = (g_floats + 3) / 4 * 4, off_xc = off_pb + (pb_floats + 3) / 4 * 4, off_pw = off_xc + xc_floats;
+    float* ws = nullptr;
+    if (workspace_alloc(reinterpret_cast<void**>(&ws), (off_pw + pw_floats) * sizeof(float), s)) return cudaErrorMemoryAllocation;
+    float *gc = ws, *part_b = ws + off_pb, *xc = ws + off_xc, *part_w = ws + off_pw;
+    int e = 0;
+    {
+        const unsigned blocks = (unsigned)(B * out_chunks * nbx);
+        if (out_chunked)
+            branch_grad_mask_kernel<true><<<blocks, 256, 0, s>>>(grad_out, relu ? y : nullptr, gc, part_b, cout, out_chunks, nbx, plane);
+        else
+            branch_grad_mask_kernel<false><<<blocks, 256, 0, s>>>(grad_out, relu ? y : nullptr, gc, part_b, cout, out_chunks, nbx, plane);
+        count_launch();
+        e = finish_launch();
+    }
+    if (!e && grad_bias) {
+        tap_conv3x3_wgrad_reduce_kernel<<<(cout + 255) / 256, 256, 0, s>>>(nullptr, part_b, nullptr, grad_bias, 0, cout, (int)(B * nbx));
+        count_launch();
+        e = finish_launch();
+    }
+    if (!e && grad_x)   // the adjoint convolution, cout -> cin channels, from g: no bias, no ReLU, NCHW out
+        e = launch_branch_conv(gc, packed_adjoint, nullptr, grad_x, B, branch_conv_shape(B, cout, cin, h, w, false), false, s);
+    if (!e && wgrad) {
+        const float* xw = x;
+        if (!in_chunked) {   // as the forward does: a TF32-rounded chunk-major copy
+            const int64_t n = B * in_chunks * plane;
+            nchw_to_chunked_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(x, xc, n, cin, in_chunks, plane);
+            count_launch();
+            e = finish_launch();
+            xw = xc;
+        }
+        if (!e) {
+            const BranchConvShape bs = branch_conv_shape(B, cin, cout, h, w, false);
+            BranchWgradShape sh;
+            sh.h = (int)h; sh.w = (int)w; sh.cin = cin; sh.cout = cout;
+            sh.tiles_x = bs.tiles_x; sh.tiles_y = bs.tiles_y; sh.ntiles = bs.ntiles;
+            sh.in_chunks = in_chunks; sh.out_chunks = out_chunks; sh.halves = halves;
+            e = launch_tc<branch_conv3x3_wgrad_kernel>(BW_SMEM, BW_THREADS, pairs * halves, s, gc, xw, part_w, sh);
+        }
+        if (!e) {
+            tap_conv3x3_wgrad_reduce_kernel<<<(nw + 255) / 256, 256, 0, s>>>(part_w, nullptr, grad_weight, nullptr, nw, 0, pairs);
+            count_launch();
+            e = finish_launch();
+        }
+    }
+    cudaFreeAsync(ws, s);
     return e;
 }

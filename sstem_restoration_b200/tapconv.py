@@ -9,8 +9,9 @@ layout of ``Conv2d`` or directly tile-major for :func:`sstem_restoration_b200.se
 ``ModuleTapProducer(trainable=True)`` add the backward (tcgen05 kernels as well) for training.
 
 The three half-resolution ``Conv2d -> ReLU`` layers in front of them run on :func:`branch_conv3x3` (csrc/tapconv.cu, the same
-tcgen05 machinery fed by TMA from a chunk-major activation layout); :class:`ModuleTapBranch` is the whole branch, forward
-only.  No CPU / PyTorch fallback.
+tcgen05 machinery fed by TMA from a chunk-major activation layout), their gradients on :func:`branch_conv3x3_backward`;
+:class:`ModuleTapBranch` is the whole branch, forward only by default and trainable with ``trainable=True``.  No CPU /
+PyTorch fallback.
 """
 import torch
 
@@ -166,23 +167,34 @@ class ModuleTapProducer(torch.nn.Module):
         return TapConv3x3Function.apply(x, self.weight, self.bias, self.upsample, self.tiled, packed, adjoint)
 
 
-def pack_branch_conv_weight(weight: torch.Tensor) -> torch.Tensor:
-    """``Conv2d.weight`` ``[cout<=64, cin<=64, 3, 3]`` -> the resident image of :func:`branch_conv3x3` (144 KB,
-    TF32-rounded).  Pack once per layer, reuse for every call."""
+def _pack_branch(weight: torch.Tensor, name: str, entry: str) -> torch.Tensor:
     if weight.is_cuda == False:
         raise NotImplementedError()
     if weight.dtype != torch.float32 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3):
-        raise TypeError("pack_branch_conv_weight: float32 [cout, cin, 3, 3] required")
+        raise TypeError(f"{name}: float32 [cout, cin, 3, 3] required")
     cout, cin = weight.shape[:2]
     if cin > 64 or cout > 64:
-        raise ValueError("pack_branch_conv_weight: cin <= 64 and cout <= 64 required")
+        raise ValueError(f"{name}: cin <= 64 and cout <= 64 required")
     lib = _lib.load()
     packed = torch.empty(lib.sstem_branch_conv3x3_packed_elems(), dtype=torch.float32, device=weight.device)
-    code = lib.sstem_branch_conv3x3_pack_weights(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
+    code = getattr(lib, entry)(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
     if code:
-        _lib.check(code, "sstem_branch_conv3x3_pack_weights")
+        _lib.check(code, entry)
     packed._sstem_cin_cout = (int(cin), int(cout))
     return packed
+
+
+def pack_branch_conv_weight(weight: torch.Tensor) -> torch.Tensor:
+    """``Conv2d.weight`` ``[cout<=64, cin<=64, 3, 3]`` -> the resident image of :func:`branch_conv3x3` (144 KB,
+    TF32-rounded).  Pack once per layer, reuse for every call."""
+    return _pack_branch(weight, "pack_branch_conv_weight", "sstem_branch_conv3x3_pack_weights")
+
+
+def pack_branch_conv_weight_adjoint(weight: torch.Tensor) -> torch.Tensor:
+    """``Conv2d.weight`` ``[cout<=64, cin<=64, 3, 3]`` -> the resident image of the adjoint convolution's weight
+    ``W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]`` (cout -> cin channels), which the input gradient of
+    :func:`branch_conv3x3_backward` runs.  It carries (cin, cout) of ``weight``."""
+    return _pack_branch(weight, "pack_branch_conv_weight_adjoint", "sstem_branch_conv3x3_pack_weights_adjoint")
 
 
 def branch_conv3x3(x: torch.Tensor, packed: torch.Tensor, bias=None, relu=True, chunked_in=False, chunked_out=False) -> torch.Tensor:
@@ -216,6 +228,76 @@ def branch_conv3x3(x: torch.Tensor, packed: torch.Tensor, bias=None, relu=True, 
     return out
 
 
+def branch_conv3x3_backward(grad_out, y, x, packed_adjoint, cin, cout, relu=True, chunked_in=False, chunked_out=False,
+                            need=(True, True, True)):
+    """Gradients of ``y = relu?(conv2d(x, weight, bias, stride 1, padding 1))`` (:func:`branch_conv3x3`) from ``grad_out``
+    ``[B, cout, h, w]``: returns ``(grad_x [B, cin, h, w], grad_weight [cout, cin, 3, 3], grad_bias [cout])``, ``None``
+    for each one ``need`` does not ask for.
+
+    ``y`` and ``x`` are the forward's output and input in the layouts it wrote and read (``chunked_out`` / ``chunked_in``:
+    chunk-major ``[B, C8/4, h, w, 4]``); ``y`` is only read with ``relu`` (zero gradient where ``y <= 0``, as torch's ReLU backward)
+    and may then be None otherwise.  ``packed_adjoint`` from :func:`pack_branch_conv_weight_adjoint` (None when grad_x is
+    not needed).  TF32 products, fp32 sums, deterministic; grad_bias sums the unrounded masked gradient."""
+    if grad_out.is_cuda == False or x.is_cuda == False:
+        raise NotImplementedError()
+    if grad_out.dtype != torch.float32 or x.dtype != torch.float32:
+        raise TypeError("branch_conv3x3_backward: float32 tensors required")
+    B, _, h, w = x.shape[:4]
+    if tuple(grad_out.shape) != (B, cout, h, w):
+        raise ValueError(f"branch_conv3x3_backward: grad_out {tuple(grad_out.shape)} is not [{B}, {cout}, {h}, {w}]")
+    if tuple(x.shape) != ((B, (cin + 7) // 8 * 2, h, w, 4) if chunked_in else (B, cin, h, w)) or not x.is_contiguous():
+        raise ValueError(f"branch_conv3x3_backward: x {tuple(x.shape)} does not match cin = {cin} (chunked_in={chunked_in})")
+    if relu and (y is None or tuple(y.shape) != ((B, (cout + 7) // 8 * 2, h, w, 4) if chunked_out else (B, cout, h, w))
+                 or not y.is_contiguous()):
+        raise ValueError("branch_conv3x3_backward: relu needs the forward's contiguous output y in its layout")
+    need_x, need_w, need_b = need
+    if need_x and (packed_adjoint is None or getattr(packed_adjoint, "_sstem_cin_cout", None) != (cin, cout)):
+        raise ValueError("branch_conv3x3_backward: grad_x needs packed_adjoint = pack_branch_conv_weight_adjoint(weight)")
+    gx = torch.empty((B, cin, h, w), dtype=torch.float32, device=x.device) if need_x else None
+    gw = torch.empty((cout, cin, 3, 3), dtype=torch.float32, device=x.device) if need_w else None
+    gb = torch.empty(cout, dtype=torch.float32, device=x.device) if need_b else None
+    if (need_x or need_w or need_b) and grad_out.numel():
+        grad_out = grad_out.contiguous()
+        flags = ((_lib.BRANCH_RELU if relu else 0) | (_lib.BRANCH_IN_CHUNKED if chunked_in else 0)
+                 | (_lib.BRANCH_OUT_CHUNKED if chunked_out else 0))
+        ptr = lambda t: None if t is None else t.data_ptr()
+        code = _lib.load().sstem_branch_conv3x3_backward(grad_out.data_ptr(), ptr(y) if relu else None, x.data_ptr(),
+                                                         ptr(packed_adjoint) if need_x else None, ptr(gx), ptr(gw), ptr(gb),
+                                                         B, cin, cout, h, w, flags, _stream_ptr(x))
+        if code:
+            _lib.check(code, "sstem_branch_conv3x3_backward")
+    return gx, gw, gb
+
+
+class _TapBranchConvs(torch.autograd.Function):
+    """The three half-resolution ``Conv2d -> ReLU`` layers of a tap branch with their backward: the forward chains
+    :func:`branch_conv3x3` (NCHW -> chunk-major -> chunk-major -> NCHW) and keeps x, the two chunk-major activations and
+    the output; the backward runs :func:`branch_conv3x3_backward` once per layer, last layer first."""
+
+    @staticmethod
+    def forward(ctx, x, w0, b0, w2, b2, w4, b4, packs, adjoints):
+        a1 = branch_conv3x3(x, packs[0], b0.detach(), relu=True, chunked_in=False, chunked_out=True)
+        a2 = branch_conv3x3(a1, packs[1], b2.detach(), relu=True, chunked_in=True, chunked_out=True)
+        a3 = branch_conv3x3(a2, packs[2], b4.detach(), relu=True, chunked_in=True, chunked_out=False)
+        ctx.save_for_backward(x, a1, a2, a3)
+        ctx.adjoints, ctx.shapes = adjoints, tuple(tuple(t.shape[:2]) for t in (w0, w2, w4))
+        return a3
+
+    @staticmethod
+    def backward(ctx, g3):
+        x, a1, a2, a3 = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        (c1, c0), (c2, _), (c3, _) = ctx.shapes
+        adj = ctx.adjoints
+        g2, gw4, gb4 = branch_conv3x3_backward(g3, a3, a2, adj[2], c2, c3, chunked_in=True, chunked_out=False,
+                                               need=(True, need[5], need[6]))
+        g1, gw2, gb2 = branch_conv3x3_backward(g2, a2, a1, adj[1], c1, c2, chunked_in=True, chunked_out=True,
+                                               need=(True, need[3], need[4]))
+        gx, gw0, gb0 = branch_conv3x3_backward(g1, a1, x, adj[0] if need[0] else None, c0, c1, chunked_in=False, chunked_out=True,
+                                               need=(need[0], need[1], need[2]))
+        return gx, gw0, gb0, gw2, gb2, gw4, gb4, None, None
+
+
 class _BranchConv(ModuleTapProducer):
     """One ``Conv2d(cin, cout, 3, 1, 1) -> ReLU`` of a tap branch on :func:`branch_conv3x3`, its weight packed on first use
     and again whenever it changes."""
@@ -238,21 +320,30 @@ class ModuleTapBranch(torch.nn.Module):
     ``m.load_state_dict(net.upconv51_1.state_dict())`` loads a reference branch.  The three half-resolution layers run on
     :func:`branch_conv3x3` (NCHW in, chunk-major between them, ``[B, taps, h, w]`` out), the last two on the tap producer;
     ``tiled=True`` returns the taps tile-major (:func:`sstem_restoration_b200.sepconv_forward_tiled`'s layout).  Forward
-    only: an input that requires grad raises."""
+    only by default: an input that requires grad raises.  ``trainable=True`` runs the three layers with their backward
+    (:func:`branch_conv3x3_backward`) and the producer as ``ModuleTapProducer(trainable=True)``: gradients reach all
+    eight parameters, and ``x`` when it requires grad."""
 
-    def __init__(self, in_channels=64, mid_channels=64, taps=51, tiled=True):
+    def __init__(self, in_channels=64, mid_channels=64, taps=51, tiled=True, trainable=False):
         super().__init__()
-        self.in_channels = in_channels
+        self.in_channels, self.trainable = in_channels, trainable
         self.add_module("0", _BranchConv(in_channels, mid_channels))
         self.add_module("2", _BranchConv(mid_channels, mid_channels))
         self.add_module("4", _BranchConv(mid_channels, taps))
-        self.add_module("7", ModuleTapProducer(taps, taps, upsample=True, tiled=tiled))
+        self.add_module("7", ModuleTapProducer(taps, taps, upsample=True, tiled=tiled, trainable=trainable))
 
     def forward(self, x):
-        if torch.is_grad_enabled() and x.requires_grad:
+        if not self.trainable and torch.is_grad_enabled() and x.requires_grad:
             raise NotImplementedError("ModuleTapBranch is forward only: call it under torch.no_grad() or detach its input")
         if x.dim() != 4 or x.shape[1] != self.in_channels:
             raise ValueError(f"ModuleTapBranch: x [B, {self.in_channels}, h, w] required, got {tuple(x.shape)}")
+        if self.trainable:
+            convs = [getattr(self, k) for k in ("0", "2", "4")]
+            packs = tuple(c._cached("_packed", pack_branch_conv_weight, x.device) for c in convs)
+            adjoints = (tuple(c._cached("_packed_adjoint", pack_branch_conv_weight_adjoint, x.device) for c in convs)
+                        if torch.is_grad_enabled() else None)
+            a = _TapBranchConvs.apply(x.contiguous(), *(t for c in convs for t in (c.weight, c.bias)), packs, adjoints)
+            return getattr(self, "7")(a)
         a = getattr(self, "0")(x.contiguous(), chunked_in=False, chunked_out=True)
         a = getattr(self, "2")(a, chunked_in=True, chunked_out=True)
         a = getattr(self, "4")(a, chunked_in=True, chunked_out=False)
