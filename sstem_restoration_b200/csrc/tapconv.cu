@@ -139,6 +139,74 @@ __device__ __forceinline__ float to_tf32(float x) {        // round to nearest (
 __device__ __forceinline__ void sts128(unsigned addr, float a, float b, float c, float d) {
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
+// columns taddr .. + 31 of the warp's 32 tensor-memory lanes, one per register; valid after tcgen05.wait::ld
+__device__ __forceinline__ void tc_ld32(unsigned taddr, unsigned (&v)[32]) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
+        "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
+          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
+          "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
+          "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+        : "r"(taddr));
+}
+// The M = 128 epilogues, two accumulator stages of 64 columns: wait until the stage of the CTA's tile `it` is complete
+// (barriers b_accfull / b_accempty + 8 * stage), read it from the warp's lanes and release it, so the MMAs of tile
+// it + 2 may start.  tmem_lanes = the TMEM base address + the warp's first lane, computed by the caller: there the
+// compiler knows the range of warp = tid / 32, and computed here the address arithmetic reschedules the whole kernel.
+__device__ __forceinline__ void tc_take_acc(unsigned tmem_lanes, int it, unsigned b_accfull, unsigned b_accempty,
+                                            unsigned (&v)[64]) {
+    const int as = it & 1;
+    tc_wait(b_accfull + 8 * as, (it >> 1) & 1);
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const unsigned ta = tmem_lanes + as * TC_N;
+    tc_ld32(ta, reinterpret_cast<unsigned (&)[32]>(v[0]));
+    tc_ld32(ta + 32, reinterpret_cast<unsigned (&)[32]>(v[32]));
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_arrive(b_accempty + 8 * as);
+}
+
+// The dynamic shared memory from its first 128-byte boundary: shared-window address and generic pointer.
+struct AlignedSmem {
+    unsigned addr;
+    unsigned char* ptr;
+};
+__device__ __forceinline__ AlignedSmem aligned_smem() {
+    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
+    const unsigned raw = (unsigned)__cvta_generic_to_shared(tc_smem_raw);
+    const unsigned addr = (raw + 127u) & ~127u;
+    return {addr, tc_smem_raw + (addr - raw)};
+}
+
+// The tiles of a persistent CTA, blockIdx.x, + gridDim.x, ..., as (tile, column, row, image).  The coordinates advance
+// by a fixed (column, row) step, so the walk needs no division (two 32-bit divisions per tile and warp were 15 % of all
+// instructions issued in tap_conv3x3_kernel).
+struct TileIter {
+    int tile, tx, ty, b;
+};
+struct TileWalker {
+    int tiles_x, tiles_y, step_tx, step_r;
+    __device__ TileWalker(int tiles_x_, int tiles_y_)
+        : tiles_x(tiles_x_), tiles_y(tiles_y_), step_tx((int)gridDim.x % tiles_x_), step_r((int)gridDim.x / tiles_x_) {}
+    __device__ TileIter first() const {
+        TileIter t;
+        t.tile = blockIdx.x;
+        const int r = t.tile / tiles_x;
+        t.tx = t.tile - r * tiles_x;
+        t.b = r / tiles_y;
+        t.ty = r - t.b * tiles_y;
+        return t;
+    }
+    __device__ void advance(TileIter& t) const {
+        t.tile += gridDim.x;
+        t.tx += step_tx;
+        int dr = step_r;
+        if (t.tx >= tiles_x) { t.tx -= tiles_x; ++dr; }
+        t.ty += dr;
+        while (t.ty >= tiles_y) { t.ty -= tiles_y; ++t.b; }
+    }
+};
 
 // How the producers read x.
 enum class TapSrc {
@@ -156,9 +224,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
 tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacked,
                    const float* __restrict__ bias, float* __restrict__ out, const TapConvShape sh) {
     constexpr bool UPS = SRC == TapSrc::UP || SRC == TapSrc::UP_VEC, VEC = SRC == TapSrc::UP_VEC;
-    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
-    const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
-    unsigned char* gen = tc_smem_raw + (base - (unsigned)__cvta_generic_to_shared(tc_smem_raw));
+    const auto [base, gen] = aligned_smem();
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     // barriers: 0 weights, 1-2 a_full, 3-4 a_empty, 5-6 acc_full, 7-8 acc_empty; the TMEM base address after them
     const unsigned bar = base + TC_OFF_BAR;
@@ -179,30 +245,7 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
         if (tid < TC_N) reinterpret_cast<float*>(gen + TC_OFF_BIAS)[tid] = (bias != nullptr && tid < sh.cout) ? bias[tid] : 0.f;
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     const unsigned tmem = tmem_alloc<TC_TMEM_COLS>(bar + 96, warp);
-
-    // A CTA walks tiles blockIdx.x, + gridDim.x, ...; the tile coordinates advance by a fixed (column, row) step, so
-    // the loop needs no division (two 32-bit divisions per tile and warp were 15 % of all instructions issued).
-    struct TileIter {
-        int tile, tx, ty, b;
-    };
-    const int step_tx = (int)gridDim.x % sh.tiles_x, step_r = (int)gridDim.x / sh.tiles_x;
-    auto first_tile = [&]() {
-        TileIter t;
-        t.tile = blockIdx.x;
-        const int r = t.tile / sh.tiles_x;
-        t.tx = t.tile - r * sh.tiles_x;
-        t.b = r / sh.tiles_y;
-        t.ty = r - t.b * sh.tiles_y;
-        return t;
-    };
-    auto advance = [&](TileIter& t) {
-        t.tile += gridDim.x;
-        t.tx += step_tx;
-        int dr = step_r;
-        if (t.tx >= sh.tiles_x) { t.tx -= sh.tiles_x; ++dr; }
-        t.ty += dr;
-        while (t.ty >= sh.tiles_y) { t.ty -= sh.tiles_y; ++t.b; }
-    };
+    const TileWalker walk(sh.tiles_x, sh.tiles_y);
 
     if (warp < TC_EPI_WARPS) {
         // ===================== epilogue: TMEM lanes 32 * warp .. + 31 = tile pixels (row 4 * warp + lane / 8, column lane % 8)
@@ -211,29 +254,10 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
         const int64_t plane = (int64_t)sh.H * sh.W;
         const int tiles_y8 = (sh.H + 7) / 8, tiles_x8 = (sh.W + 7) / 8;
         int it = 0;
-        for (TileIter ti = first_tile(); ti.tile < sh.ntiles; advance(ti), ++it) {
-            const int as = it & 1;
+        for (TileIter ti = walk.first(); ti.tile < sh.ntiles; walk.advance(ti), ++it) {
             const int b = ti.b, Y0 = ti.ty * TC_TH, X0 = ti.tx * TC_TW;
-            tc_wait(b_accfull + 8 * as, (it >> 1) & 1);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             unsigned v[64];
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-                const unsigned ta = tmem + ((unsigned)(warp * 32) << 16) + as * TC_N + hh * 32;
-                asm volatile(
-                    "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-                    "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-                    : "=r"(v[hh*32+0]), "=r"(v[hh*32+1]), "=r"(v[hh*32+2]), "=r"(v[hh*32+3]), "=r"(v[hh*32+4]), "=r"(v[hh*32+5]),
-                      "=r"(v[hh*32+6]), "=r"(v[hh*32+7]), "=r"(v[hh*32+8]), "=r"(v[hh*32+9]), "=r"(v[hh*32+10]), "=r"(v[hh*32+11]),
-                      "=r"(v[hh*32+12]), "=r"(v[hh*32+13]), "=r"(v[hh*32+14]), "=r"(v[hh*32+15]), "=r"(v[hh*32+16]), "=r"(v[hh*32+17]),
-                      "=r"(v[hh*32+18]), "=r"(v[hh*32+19]), "=r"(v[hh*32+20]), "=r"(v[hh*32+21]), "=r"(v[hh*32+22]), "=r"(v[hh*32+23]),
-                      "=r"(v[hh*32+24]), "=r"(v[hh*32+25]), "=r"(v[hh*32+26]), "=r"(v[hh*32+27]), "=r"(v[hh*32+28]), "=r"(v[hh*32+29]),
-                      "=r"(v[hh*32+30]), "=r"(v[hh*32+31])
-                    : "r"(ta));
-            }
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            tc_arrive(b_accempty + 8 * as);                // the accumulator stage is free: the MMAs of tile it + 2 may start
+            tc_take_acc(tmem + ((unsigned)(warp * 32) << 16), it, b_accfull, b_accempty, v);
             const int Y = Y0 + r, X = X0 + c;
             if (TILED_OUT) {
                 // the 16 x 8 tile is two 8 x 8 blocks of the tile-major layout; a warp writes 32 consecutive floats per tap
@@ -381,14 +405,14 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
                 }
             }
         };
-        TileIter ti = first_tile(), tn = ti;               // this tile and the next one of this CTA
-        advance(tn);
+        TileIter ti = walk.first(), tn = ti;               // this tile and the next one of this CTA
+        walk.advance(tn);
         if (UPS && ti.tile < sh.ntiles) load_window(ti);
         // per-thread constants of the blend: chunk parity folded into the base addresses, so every shared-memory offset
         // below is an immediate
         const unsigned half_win = half * 4 * (TC_WIN_CH * 4), half_dst = half * TC_NPIX * 16;
         int it = 0;
-        for (; ti.tile < sh.ntiles; ti = tn, advance(tn), ++it) {
+        for (; ti.tile < sh.ntiles; ti = tn, walk.advance(tn), ++it) {
             const int s = it & 1;
             const unsigned ph = (it >> 1) & 1;
             const int b = ti.b, Y0 = ti.ty * TC_TH, X0 = ti.tx * TC_TW;
@@ -471,15 +495,19 @@ tap_conv3x3_kernel(const float* __restrict__ x, const float* __restrict__ wpacke
     tmem_dealloc<TC_TMEM_COLS>(tmem, warp);
 }
 
-// weights [cout][cin][3][3] -> [tap][chunk < 13][n = 64][4] + one zero chunk, zero padded, rounded to TF32.  ADJOINT:
+// Weights [cout][cin][3][3] -> [tap][chunk < CHUNKS][n = 64][4], zero padded, rounded to TF32; ZERO_CHUNK: followed by
+// one zero chunk (the producer's, 13 chunks per tap, shared by all taps; the branch has 16 chunks and none).  ADJOINT:
 // the image of W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx] instead, the convolution from cout to cin channels that the
 // input gradient runs.
-template <bool ADJOINT>
-__global__ void tap_conv3x3_pack_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
+__host__ __device__ constexpr int packed_floats(int chunks, bool zero_chunk) { return (9 * chunks + (zero_chunk ? 1 : 0)) * TC_N * 4; }
+static_assert(packed_floats(TC_WCHUNKS, true) == (int)(TC_W_BYTES / 4), "tap producer weight image");
+
+template <bool ADJOINT, int CHUNKS, bool ZERO_CHUNK>
+__global__ void conv3x3_pack_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (int)(TC_W_BYTES / 4)) return;
-    if (i >= (int)(TC_W_ZERO_OFF / 4)) { packed[i] = 0.f; return; }
-    const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % TC_WCHUNKS, tap = (i >> 2) / TC_N / TC_WCHUNKS;
+    if (i >= packed_floats(CHUNKS, ZERO_CHUNK)) return;
+    if (ZERO_CHUNK && i >= 9 * CHUNKS * TC_N * 4) { packed[i] = 0.f; return; }
+    const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % CHUNKS, tap = (i >> 2) / TC_N / CHUNKS;
     const int ch = ck * 4 + j;                             // input channel of the packed convolution
     if (ADJOINT)                                           // W'[n][ch][tap] = W[ch][n][8 - tap]
         packed[i] = (n < cin && ch < cout) ? to_tf32(w[((int64_t)ch * cin + n) * 9 + (8 - tap)]) : 0.f;
@@ -499,6 +527,14 @@ int launch_tc(unsigned smem, int threads, int ctas, cudaStream_t s, const Args&.
         done.set(dev);
     }
     Kern<<<ctas, threads, smem, s>>>(args...);
+    count_launch();
+    return finish_launch();
+}
+
+// The elementwise and reduction kernels: `blocks` blocks of 256 threads.
+template <auto Kern, class... Args>
+int launch256(int64_t blocks, cudaStream_t s, const Args&... args) {
+    Kern<<<(unsigned)blocks, 256, 0, s>>>(args...);
     count_launch();
     return finish_launch();
 }
@@ -531,7 +567,7 @@ int launch_tap_conv(TapSrc src, bool tiled_out, bool full, const float* x, const
 // Backward of y = conv3x3(up(x), W) + b (sstem_tap_conv3x3_backward).
 //
 // grad_x = up^T(conv3x3(gy, W')), W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]: the convolution is tap_conv3x3_kernel on its
-// no-upsample path (weights packed by tap_conv3x3_pack_kernel<true>), up^T is the gather below.
+// no-upsample path (weights packed by the ADJOINT conv3x3_pack_kernel), up^T is the gather below.
 
 // Weight with which output row (column) Y of the align_corners upsample reads source row i: ATen's float32 index and
 // fraction, as the forward producer computes them.  At the last row the neighbour is the row itself (both weights land
@@ -583,7 +619,7 @@ upsample2x_adjoint_kernel(const float* __restrict__ gU, float* __restrict__ gx, 
 //     ky + dy: a start-address shift of one 1792-byte row per dy.
 // One stage: all 12 warps stage a tile, warp 0 issues its 144 MMAs, and the staging of the next tile waits for their
 // completion (tcgen05.commit).  gy is summed per output channel on the way (grad_bias).  Each CTA writes one partial of
-// both gradients at the end; tap_conv3x3_wgrad_reduce_kernel sums the partials over CTAs in a fixed order, so the result
+// both gradients at the end; sum_partials_kernel sums the partials over CTAs in a fixed order, so the result
 // is run-to-run bit-identical.
 constexpr int WG_THREADS = 384;
 constexpr int WG_M = 64, WG_N = 56;
@@ -604,9 +640,7 @@ template <bool UPS, bool GY_TILED>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__ x, float* __restrict__ part_w,
                          float* __restrict__ part_b, const TapConvShape sh) {
-    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
-    const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
-    unsigned char* gen = tc_smem_raw + (base - (unsigned)__cvta_generic_to_shared(tc_smem_raw));
+    const auto [base, gen] = aligned_smem();
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const unsigned bar = base + WG_OFF_BAR;
     if (tid == 0) {
@@ -754,9 +788,10 @@ tap_conv3x3_wgrad_kernel(const float* __restrict__ gy, const float* __restrict__
     tmem_dealloc<WG_TMEM_COLS>(tmem, warp);
 }
 
-// sum of the per-CTA partials in CTA order (deterministic); out[i] for i < n, NULL outputs skipped
-__global__ void tap_conv3x3_wgrad_reduce_kernel(const float* __restrict__ part_w, const float* __restrict__ part_b,
-                                                float* __restrict__ gw, float* __restrict__ gb, int nw, int nb, int parts) {
+// sum of the partials of both weight-gradient kernels and of branch_grad_mask_kernel, in CTA / block order
+// (deterministic); out[i] for i < n, NULL outputs skipped
+__global__ void sum_partials_kernel(const float* __restrict__ part_w, const float* __restrict__ part_b,
+                                    float* __restrict__ gw, float* __restrict__ gb, int nw, int nb, int parts) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const float* src;
     float* dst;
@@ -785,18 +820,23 @@ TapConvShape tap_conv_shape(int64_t B, int cin, int cout, int64_t h, int64_t w, 
     return sh;
 }
 
-template <bool ADJOINT>
-int pack_weights(const float* weight, float* packed, int cin, int cout, int max_cout, cudaStream_t s) {
+// Every pack entry point: conv3x3_pack_kernel for one weight image, within that entry point's channel limits.
+template <bool ADJOINT, int CHUNKS, bool ZERO_CHUNK>
+int pack_weights(const float* weight, float* packed, int cin, int cout, int max_cin, int max_cout, void* stream) {
     if (!weight || !packed) return SSTEM_E_NULL;
-    if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > max_cout) return SSTEM_E_SHAPE;
+    if (cin <= 0 || cin > max_cin || cout <= 0 || cout > max_cout) return SSTEM_E_SHAPE;
     if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
     DeviceGuard guard(packed);
     if (guard.err) return guard.err;
-    const int total = (int)(TC_W_BYTES / 4);
-    tap_conv3x3_pack_kernel<ADJOINT><<<(total + 255) / 256, 256, 0, s>>>(weight, packed, cin, cout);
-    count_launch();
-    return finish_launch();
+    return launch256<conv3x3_pack_kernel<ADJOINT, CHUNKS, ZERO_CHUNK>>((packed_floats(CHUNKS, ZERO_CHUNK) + 255) / 256,
+                                                                       (cudaStream_t)stream, weight, packed, cin, cout);
 }
+
+// Image bounds of every entry point
+bool image_fits(int64_t B, int64_t h, int64_t w) { return B > 0 && h > 0 && w > 0 && h <= (1 << 22) && w <= (1 << 22); }
+
+// 16 x 8 output tiles of B images of H x W
+int64_t tile_count(int64_t B, int64_t H, int64_t W) { return ((W + TC_TW - 1) / TC_TW) * ((H + TC_TH - 1) / TC_TH) * B; }
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Tap branch convolutions (sstem_branch_conv3x3, DESIGN 4.11c): the three half-resolution layers in front of the
@@ -819,6 +859,7 @@ constexpr unsigned BC_OFF_BAR = BC_OFF_BIAS + TC_N * 4;
 constexpr unsigned BC_SMEM = BC_OFF_BAR + 256 + 128;       // + barriers and the TMEM address + alignment slack = 217 216
 static_assert(BC_SMEM <= 232448, "shared memory budget");
 static_assert(8 * (1 + 2 * BC_SLOTS + 4) + 4 <= 256, "barrier block");
+static_assert(packed_floats(BC_CHUNKS, false) == (int)(BC_W_BYTES / 4), "branch weight image");
 constexpr int BC_THREADS = (TC_EPI_WARPS + 2) * 32;        // 192
 
 struct BranchConvShape {
@@ -828,6 +869,8 @@ struct BranchConvShape {
     int k_steps;                                           // C8in / 8
     int slots_per_tile;                                    // ceil(k_steps / 2)
     int relu;
+    int cin;
+    int halves;                                            // weight gradient: CTAs per pair, 2 when cin > 32
 };
 
 // OUT_CHUNKED: the output is chunk-major and TF32-rounded (the next layer's input); else NCHW in full fp32
@@ -835,9 +878,7 @@ template <bool OUT_CHUNKED>
 __global__ void __launch_bounds__(BC_THREADS, 1)
 branch_conv3x3_kernel(const __grid_constant__ CUtensorMap map_x, const float* __restrict__ wpacked,
                       const float* __restrict__ bias, float* __restrict__ out, const BranchConvShape sh) {
-    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
-    const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
-    unsigned char* gen = tc_smem_raw + (base - (unsigned)__cvta_generic_to_shared(tc_smem_raw));
+    const auto [base, gen] = aligned_smem();
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     // barriers: weights, slot full x 6, slot empty x 6, acc_full x 2, acc_empty x 2; the TMEM base address after them
     const unsigned bar = base + BC_OFF_BAR;
@@ -857,29 +898,7 @@ branch_conv3x3_kernel(const __grid_constant__ CUtensorMap map_x, const float* __
     }
     if (tid < TC_N) reinterpret_cast<float*>(gen + BC_OFF_BIAS)[tid] = (bias != nullptr && tid < sh.cout) ? bias[tid] : 0.f;
     const unsigned tmem = tmem_alloc<TC_TMEM_COLS>(bar + 8 * (1 + 2 * BC_SLOTS + 4), warp);
-
-    // tiles blockIdx.x, + gridDim.x, ... walked without divisions, as in tap_conv3x3_kernel
-    struct TileIter {
-        int tile, tx, ty, b;
-    };
-    const int step_tx = (int)gridDim.x % sh.tiles_x, step_r = (int)gridDim.x / sh.tiles_x;
-    auto first_tile = [&]() {
-        TileIter t;
-        t.tile = blockIdx.x;
-        const int r = t.tile / sh.tiles_x;
-        t.tx = t.tile - r * sh.tiles_x;
-        t.b = r / sh.tiles_y;
-        t.ty = r - t.b * sh.tiles_y;
-        return t;
-    };
-    auto advance = [&](TileIter& t) {
-        t.tile += gridDim.x;
-        t.tx += step_tx;
-        int dr = step_r;
-        if (t.tx >= sh.tiles_x) { t.tx -= sh.tiles_x; ++dr; }
-        t.ty += dr;
-        while (t.ty >= sh.tiles_y) { t.ty -= sh.tiles_y; ++t.b; }
-    };
+    const TileWalker walk(sh.tiles_x, sh.tiles_y);
 
     if (warp < TC_EPI_WARPS) {
         // ===================== epilogue: TMEM lanes 32 * warp .. + 31 = tile pixels (row 4 * warp + lane / 8, column lane % 8)
@@ -887,28 +906,9 @@ branch_conv3x3_kernel(const __grid_constant__ CUtensorMap map_x, const float* __
         const int r = warp * 4 + (lane >> 3), c = lane & 7;
         const int64_t plane = (int64_t)sh.h * sh.w;
         int it = 0;
-        for (TileIter ti = first_tile(); ti.tile < sh.ntiles; advance(ti), ++it) {
-            const int as = it & 1;
-            tc_wait(b_accfull + 8 * as, (it >> 1) & 1);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        for (TileIter ti = walk.first(); ti.tile < sh.ntiles; walk.advance(ti), ++it) {
             unsigned v[64];
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-                const unsigned ta = tmem + ((unsigned)(warp * 32) << 16) + as * TC_N + hh * 32;
-                asm volatile(
-                    "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-                    "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-                    : "=r"(v[hh*32+0]), "=r"(v[hh*32+1]), "=r"(v[hh*32+2]), "=r"(v[hh*32+3]), "=r"(v[hh*32+4]), "=r"(v[hh*32+5]),
-                      "=r"(v[hh*32+6]), "=r"(v[hh*32+7]), "=r"(v[hh*32+8]), "=r"(v[hh*32+9]), "=r"(v[hh*32+10]), "=r"(v[hh*32+11]),
-                      "=r"(v[hh*32+12]), "=r"(v[hh*32+13]), "=r"(v[hh*32+14]), "=r"(v[hh*32+15]), "=r"(v[hh*32+16]), "=r"(v[hh*32+17]),
-                      "=r"(v[hh*32+18]), "=r"(v[hh*32+19]), "=r"(v[hh*32+20]), "=r"(v[hh*32+21]), "=r"(v[hh*32+22]), "=r"(v[hh*32+23]),
-                      "=r"(v[hh*32+24]), "=r"(v[hh*32+25]), "=r"(v[hh*32+26]), "=r"(v[hh*32+27]), "=r"(v[hh*32+28]), "=r"(v[hh*32+29]),
-                      "=r"(v[hh*32+30]), "=r"(v[hh*32+31])
-                    : "r"(ta));
-            }
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            tc_arrive(b_accempty + 8 * as);                // the accumulator stage is free: the MMAs of tile it + 2 may start
+            tc_take_acc(tmem + ((unsigned)(warp * 32) << 16), it, b_accfull, b_accempty, v);
             const int Y = ti.ty * TC_TH + r, X = ti.tx * TC_TW + c;
             if (Y >= sh.h || X >= sh.w) continue;
             // ReLU before rounding (rounding keeps the sign); `x < 0` keeps a NaN a NaN, as torch's ReLU does
@@ -981,7 +981,7 @@ branch_conv3x3_kernel(const __grid_constant__ CUtensorMap map_x, const float* __
                 bulk_load(base + t * BC_W_TAP_BYTES, reinterpret_cast<const char*>(wpacked) + (size_t)t * BC_W_TAP_BYTES, BC_W_TAP_BYTES, b_w);
             int slot = 0;
             unsigned sph = 0;
-            for (TileIter ti = first_tile(); ti.tile < sh.ntiles; advance(ti)) {
+            for (TileIter ti = walk.first(); ti.tile < sh.ntiles; walk.advance(ti)) {
                 // box origin: one pixel up and left of the tile (zero-filled outside the image), chunk q of image b
                 const int x0 = 4 * (ti.tx * TC_TW - 1), y0 = ti.ty * TC_TH - 1, c0 = ti.b * sh.in_chunks;
                 for (int q = 0; q < sh.slots_per_tile; ++q) {
@@ -998,20 +998,6 @@ branch_conv3x3_kernel(const __grid_constant__ CUtensorMap map_x, const float* __
     tmem_dealloc<TC_TMEM_COLS>(tmem, warp);
 }
 
-// weights [cout][cin][3][3] -> [tap][chunk < 16][n = 64][4], zero padded, rounded to TF32.  ADJOINT: the image of
-// W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx] instead (cout -> cin channels), which the input gradient runs.
-template <bool ADJOINT>
-__global__ void branch_conv3x3_pack_kernel(const float* __restrict__ w, float* __restrict__ packed, int cin, int cout) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (int)(BC_W_BYTES / 4)) return;
-    const int j = i & 3, n = (i >> 2) % TC_N, ck = (i >> 2) / TC_N % BC_CHUNKS, tap = (i >> 2) / TC_N / BC_CHUNKS;
-    const int ch = ck * 4 + j;
-    if (ADJOINT)                                           // W'[n][ch][tap] = W[ch][n][8 - tap]
-        packed[i] = (n < cin && ch < cout) ? to_tf32(w[((int64_t)ch * cin + n) * 9 + (8 - tap)]) : 0.f;
-    else
-        packed[i] = (n < cout && ch < cin) ? to_tf32(w[((int64_t)n * cin + ch) * 9 + tap]) : 0.f;
-}
-
 // [B][c][h][w] -> chunk-major [B][chunks][h][w][4], rounded to TF32, channels past c = 0.  Thread = (image, chunk, pixel).
 __global__ void __launch_bounds__(256)
 nchw_to_chunked_kernel(const float* __restrict__ x, float* __restrict__ out, int64_t n, int c, int chunks, int64_t plane) {
@@ -1024,6 +1010,12 @@ nchw_to_chunked_kernel(const float* __restrict__ x, float* __restrict__ out, int
 #pragma unroll
     for (int j = 0; j < 4; ++j) q[j] = 4 * k + j < c ? to_tf32(__ldg(src + j * plane)) : 0.f;
     reinterpret_cast<float4*>(out)[i] = make_float4(q[0], q[1], q[2], q[3]);
+}
+
+// x [B][c][h][w] -> xc, its TF32-rounded chunk-major copy with `chunks` chunks per image
+int to_chunked(const float* x, float* xc, int64_t B, int c, int chunks, int64_t plane, cudaStream_t s) {
+    const int64_t n = B * chunks * plane;
+    return launch256<nchw_to_chunked_kernel>((n + 255) / 256, s, x, xc, n, c, chunks, plane);
 }
 
 int launch_branch_conv(const float* xc, const float* wpacked, const float* bias, float* out, int64_t B, const BranchConvShape& sh,
@@ -1039,28 +1031,13 @@ int launch_branch_conv(const float* xc, const float* wpacked, const float* bias,
                        : launch_tc<branch_conv3x3_kernel<false>>(BC_SMEM, BC_THREADS, ctas, s, map, wpacked, bias, out, sh);
 }
 
-// The callers check the limits first (see sstem_branch_conv3x3).
-BranchConvShape branch_conv_shape(int64_t B, int cin, int cout, int64_t h, int64_t w, bool relu) {
-    BranchConvShape sh;
-    sh.h = (int)h; sh.w = (int)w; sh.cout = cout;
-    sh.tiles_x = (sh.w + TC_TW - 1) / TC_TW;
-    sh.tiles_y = (sh.h + TC_TH - 1) / TC_TH;
-    sh.in_chunks = (cin + 7) / 8 * 2;
-    sh.out_chunks = (cout + 7) / 8 * 2;
-    sh.k_steps = sh.in_chunks / 2;
-    sh.slots_per_tile = (sh.in_chunks + BC_SLOT_CHUNKS - 1) / BC_SLOT_CHUNKS;
-    sh.relu = relu ? 1 : 0;
-    sh.ntiles = (int)((int64_t)sh.tiles_x * sh.tiles_y * B);
-    return sh;
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
 // Backward of y = relu?(conv3x3(x, W) + b) (sstem_branch_conv3x3_backward, DESIGN 4.11d).
 //
 // g = (y <= 0) ? 0 : grad_out (grad_out without the ReLU), NCHW -> chunk-major [B][C8/4][h][w][4] rounded to TF32: the input
 // of the adjoint convolution (grad_x = branch_conv3x3_kernel on W') and the A operand of the weight gradient.  The mask is
 // torch's threshold_backward on the output: y == 0 gives 0, a NaN y passes the gradient.  Each block also writes the fp32 sums of the UNROUNDED g of its
-// chunk's four channels (grad_bias, summed over blocks by tap_conv3x3_wgrad_reduce_kernel): per thread in pixel order, then
+// chunk's four channels (grad_bias, summed over blocks by sum_partials_kernel): per thread in pixel order, then
 // a fixed shuffle tree, then the warps in order, so the result is bit-identical from run to run.  Block = (image b,
 // chunk k, part bx of the plane), blockIdx.x = (b * chunks + k) * nbx + bx; bias partial p = b * nbx + bx.
 template <bool Y_CHUNKED>
@@ -1137,18 +1114,27 @@ static_assert(BW_SMEM <= 232448, "shared memory budget");
 static_assert(9 * BW_N <= (int)BW_TMEM_COLS, "nine accumulators in tensor memory");
 static_assert(TC_TH * (BW_M / 4) == BW_STAGE_THREADS && TC_PH * (BW_N / 4) <= BW_STAGE_THREADS, "one A and one B item per thread");
 
-struct BranchWgradShape {
-    int h, w, cin, cout;
-    int tiles_x, tiles_y, ntiles;
-    int in_chunks, out_chunks;                             // C8 / 4 of x and of g
-    int halves;                                            // CTAs per pair: 2 when cin > 32
-};
+// The callers check the limits first (see sstem_branch_conv3x3).
+BranchConvShape branch_conv_shape(int64_t B, int cin, int cout, int64_t h, int64_t w, bool relu) {
+    BranchConvShape sh;
+    sh.h = (int)h; sh.w = (int)w; sh.cin = cin; sh.cout = cout;
+    sh.tiles_x = (sh.w + TC_TW - 1) / TC_TW;
+    sh.tiles_y = (sh.h + TC_TH - 1) / TC_TH;
+    sh.in_chunks = (cin + 7) / 8 * 2;
+    sh.out_chunks = (cout + 7) / 8 * 2;
+    sh.k_steps = sh.in_chunks / 2;
+    sh.slots_per_tile = (sh.in_chunks + BC_SLOT_CHUNKS - 1) / BC_SLOT_CHUNKS;
+    sh.relu = relu ? 1 : 0;
+    sh.ntiles = (int)tile_count(B, h, w);
+    sh.halves = cin > BW_N ? 2 : 1;
+    return sh;
+}
 
+// sh: the shape of the forward convolution (in_chunks: x, out_chunks: g)
 __global__ void __launch_bounds__(BW_THREADS, 1)
 branch_conv3x3_wgrad_kernel(const float* __restrict__ g, const float* __restrict__ x, float* __restrict__ part_w,
-                            const BranchWgradShape sh) {
-    extern __shared__ __align__(128) unsigned char tc_smem_raw[];
-    const unsigned base = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 127u) & ~127u;
+                            const BranchConvShape sh) {
+    const unsigned base = aligned_smem().addr;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     // barriers: full x 2, empty x 2, done; the TMEM base address after them
     const unsigned bar = base + BW_OFF_BAR;
@@ -1261,14 +1247,7 @@ branch_conv3x3_wgrad_kernel(const float* __restrict__ g, const float* __restrict
 #pragma unroll 1
         for (int tap = 0; tap < 9; ++tap) {
             unsigned v[32];
-            asm volatile(
-                "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-                "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-                : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-                  "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-                  "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-                  "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-                : "r"(tmem + ((unsigned)(warp * 32) << 16) + tap * BW_N));
+            tc_ld32(tmem + ((unsigned)(warp * 32) << 16) + tap * BW_N, v);
             asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
             if (lane < 16 && co < sh.cout) {
 #pragma unroll
@@ -1289,7 +1268,7 @@ using namespace sstem;
 extern "C" int64_t sstem_tap_conv3x3_packed_elems(void) { return (int64_t)TC_W_BYTES / 4; }
 
 extern "C" int sstem_tap_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
-    return pack_weights<false>(weight, packed, cin, cout, TC_N, (cudaStream_t)stream);
+    return pack_weights<false, TC_WCHUNKS, true>(weight, packed, cin, cout, TC_MAXC, TC_N, stream);
 }
 
 extern "C" int sstem_tap_conv3x3(const float* x, const float* packed_weight, const float* bias, float* out,
@@ -1297,21 +1276,21 @@ extern "C" int sstem_tap_conv3x3(const float* x, const float* packed_weight, con
     if (!x || !packed_weight || !out) return SSTEM_E_NULL;
     if (flags & ~(SSTEM_TAPCONV_UPSAMPLE2X | SSTEM_TAPCONV_TILED)) return SSTEM_E_FLAG;
     const bool ups = flags & SSTEM_TAPCONV_UPSAMPLE2X, tiled = flags & SSTEM_TAPCONV_TILED;
-    if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
+    if (!image_fits(B, h, w)) return SSTEM_E_SHAPE;
     if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
     if (tiled && cout != 51) return SSTEM_E_SHAPE;         // the tile-major layout is the 51-tap consumer's
     if (!aligned4(x) || !aligned16(packed_weight) || !aligned4(out) || (bias && !aligned4(bias))) return SSTEM_E_ALIGN;
     DeviceGuard guard(out);
     if (guard.err) return guard.err;
     const TapConvShape sh = tap_conv_shape(B, cin, cout, h, w, ups);
-    if ((int64_t)sh.tiles_x * sh.tiles_y * B > INT32_MAX / 2 || (int64_t)cin * h * w > INT32_MAX) return SSTEM_E_SHAPE;
+    if (tile_count(B, sh.H, sh.W) > INT32_MAX / 2 || (int64_t)cin * h * w > INT32_MAX) return SSTEM_E_SHAPE;
     const TapSrc src = !ups ? TapSrc::NCHW : (w % 4 == 0 && aligned16(x)) ? TapSrc::UP_VEC : TapSrc::UP;
     const bool full = cin > 48;                            // all 13 channel chunks exist: the common (51-channel) case, no per-chunk checks
     return launch_tap_conv(src, tiled, full, x, packed_weight, bias, out, sh, (cudaStream_t)stream);
 }
 
 extern "C" int sstem_tap_conv3x3_pack_weights_adjoint(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
-    return pack_weights<true>(weight, packed, cin, cout, TC_MAXC, (cudaStream_t)stream);
+    return pack_weights<true, TC_WCHUNKS, true>(weight, packed, cin, cout, TC_MAXC, TC_MAXC, stream);
 }
 
 extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x, const float* packed_adjoint,
@@ -1320,15 +1299,14 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
     if (!grad_out || !x || (grad_x && !packed_adjoint)) return SSTEM_E_NULL;
     if (flags & ~(SSTEM_TAPCONV_UPSAMPLE2X | SSTEM_TAPCONV_TILED)) return SSTEM_E_FLAG;
     const bool ups = flags & SSTEM_TAPCONV_UPSAMPLE2X, tiled = flags & SSTEM_TAPCONV_TILED;
-    if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
+    if (!image_fits(B, h, w)) return SSTEM_E_SHAPE;
     if (cin <= 0 || cin > TC_MAXC || cout <= 0 || cout > TC_MAXC) return SSTEM_E_SHAPE;
     if (tiled && cout != 51) return SSTEM_E_SHAPE;
     if (!aligned4(grad_out) || !aligned4(x) || (packed_adjoint && !aligned16(packed_adjoint)) || (grad_x && !aligned4(grad_x)) ||
         (grad_weight && !aligned4(grad_weight)) || (grad_bias && !aligned4(grad_bias)))
         return SSTEM_E_ALIGN;
     const int64_t H = ups ? 2 * h : h, W = ups ? 2 * w : w;
-    const int64_t nt = ((W + TC_TW - 1) / TC_TW) * ((H + TC_TH - 1) / TC_TH) * B;
-    if (nt > INT32_MAX / 2 || (int64_t)cout * H * W > INT32_MAX || (int64_t)cin * H * W > INT32_MAX) return SSTEM_E_SHAPE;
+    if (tile_count(B, H, W) > INT32_MAX / 2 || (int64_t)cout * H * W > INT32_MAX || (int64_t)cin * H * W > INT32_MAX) return SSTEM_E_SHAPE;
     if (!grad_x && !grad_weight && !grad_bias) return 0;
     DeviceGuard guard(grad_out);
     if (guard.err) return guard.err;
@@ -1343,9 +1321,7 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
         int e = launch_tap_conv(tiled ? TapSrc::TILE_MAJOR : TapSrc::NCHW, false, cout > 48, grad_out, packed_adjoint, nullptr, gU, sd, s);
         if (!e && ups) {
             const int64_t n = B * cin * h * w;
-            upsample2x_adjoint_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(gU, grad_x, n, (int)h, (int)w, (int)H, (int)W, sh.ry, sh.rx);
-            count_launch();
-            e = finish_launch();
+            e = launch256<upsample2x_adjoint_kernel>((n + 255) / 256, s, gU, grad_x, n, (int)h, (int)w, (int)H, (int)W, sh.ry, sh.rx);
         }
         if (ups) cudaFreeAsync(gU, s);
         if (e) return e;
@@ -1360,11 +1336,7 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
                              : launch_tc<tap_conv3x3_wgrad_kernel<true, false>>(WG_SMEM, WG_THREADS, ctas, s, grad_out, x, part, part_b, sh))
                     : (tiled ? launch_tc<tap_conv3x3_wgrad_kernel<false, true>>(WG_SMEM, WG_THREADS, ctas, s, grad_out, x, part, part_b, sh)
                              : launch_tc<tap_conv3x3_wgrad_kernel<false, false>>(WG_SMEM, WG_THREADS, ctas, s, grad_out, x, part, part_b, sh));
-        if (!e) {
-            tap_conv3x3_wgrad_reduce_kernel<<<(nw + cout + 255) / 256, 256, 0, s>>>(part, part_b, grad_weight, grad_bias, nw, cout, ctas);
-            count_launch();
-            e = finish_launch();
-        }
+        if (!e) e = launch256<sum_partials_kernel>((nw + cout + 255) / 256, s, part, part_b, grad_weight, grad_bias, nw, cout, ctas);
         cudaFreeAsync(part, s);
         if (e) return e;
     }
@@ -1373,25 +1345,12 @@ extern "C" int sstem_tap_conv3x3_backward(const float* grad_out, const float* x,
 
 extern "C" int64_t sstem_branch_conv3x3_packed_elems(void) { return (int64_t)BC_W_BYTES / 4; }
 
-template <bool ADJOINT>
-static int branch_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
-    if (!weight || !packed) return SSTEM_E_NULL;
-    if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
-    if (!aligned4(weight) || !aligned16(packed)) return SSTEM_E_ALIGN;
-    DeviceGuard guard(packed);
-    if (guard.err) return guard.err;
-    const int total = (int)(BC_W_BYTES / 4);
-    branch_conv3x3_pack_kernel<ADJOINT><<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(weight, packed, cin, cout);
-    count_launch();
-    return finish_launch();
-}
-
 extern "C" int sstem_branch_conv3x3_pack_weights(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
-    return branch_pack_weights<false>(weight, packed, cin, cout, stream);
+    return pack_weights<false, BC_CHUNKS, false>(weight, packed, cin, cout, BC_MAXC, TC_N, stream);
 }
 
 extern "C" int sstem_branch_conv3x3_pack_weights_adjoint(const float* weight, float* packed, int32_t cin, int32_t cout, void* stream) {
-    return branch_pack_weights<true>(weight, packed, cin, cout, stream);
+    return pack_weights<true, BC_CHUNKS, false>(weight, packed, cin, cout, BC_MAXC, TC_N, stream);
 }
 
 extern "C" int64_t sstem_chunked_elems(int64_t B, int64_t c, int64_t h, int64_t w) {
@@ -1404,11 +1363,10 @@ extern "C" int sstem_branch_conv3x3(const float* x, const float* packed_weight, 
     if (!x || !packed_weight || !out) return SSTEM_E_NULL;
     if (flags & ~(SSTEM_BRANCH_RELU | SSTEM_BRANCH_IN_CHUNKED | SSTEM_BRANCH_OUT_CHUNKED)) return SSTEM_E_FLAG;
     const bool in_chunked = flags & SSTEM_BRANCH_IN_CHUNKED, out_chunked = flags & SSTEM_BRANCH_OUT_CHUNKED;
-    if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
+    if (!image_fits(B, h, w)) return SSTEM_E_SHAPE;
     if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > TC_N) return SSTEM_E_SHAPE;
     // tile indices and the TMA chunk coordinate are 32-bit
-    if (((w + TC_TW - 1) / TC_TW) * ((h + TC_TH - 1) / TC_TH) * B > INT32_MAX / 2 || B * ((cin + 7) / 8 * 2) > INT32_MAX / 2)
-        return SSTEM_E_SHAPE;
+    if (tile_count(B, h, w) > INT32_MAX / 2 || B * ((cin + 7) / 8 * 2) > INT32_MAX / 2) return SSTEM_E_SHAPE;
     const BranchConvShape sh = branch_conv_shape(B, cin, cout, h, w, flags & SSTEM_BRANCH_RELU);
     if (!(in_chunked ? aligned16(x) : aligned4(x)) || !aligned16(packed_weight) || !(out_chunked ? aligned16(out) : aligned4(out)) ||
         (bias && !aligned4(bias)))
@@ -1419,17 +1377,11 @@ extern "C" int sstem_branch_conv3x3(const float* x, const float* packed_weight, 
     const float* xc = x;
     float* ws = nullptr;
     if (!in_chunked) {   // NCHW input: a TF32-rounded chunk-major copy in a stream-ordered workspace
-        const int64_t n = B * sh.in_chunks * h * w;
-        if (workspace_alloc(reinterpret_cast<void**>(&ws), (size_t)n * 16, s)) return cudaErrorMemoryAllocation;
-        nchw_to_chunked_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(x, ws, n, cin, sh.in_chunks, h * w);
-        count_launch();
-        if (int e = finish_launch()) {
-            cudaFreeAsync(ws, s);
-            return e;
-        }
+        if (workspace_alloc(reinterpret_cast<void**>(&ws), (size_t)(B * sh.in_chunks * h * w) * 16, s)) return cudaErrorMemoryAllocation;
         xc = ws;
     }
-    const int e = launch_branch_conv(xc, packed_weight, bias, out, B, sh, out_chunked, s);
+    int e = in_chunked ? 0 : to_chunked(x, ws, B, cin, sh.in_chunks, h * w, s);
+    if (!e) e = launch_branch_conv(xc, packed_weight, bias, out, B, sh, out_chunked, s);
     if (ws) cudaFreeAsync(ws, s);
     return e;
 }
@@ -1440,12 +1392,10 @@ extern "C" int sstem_branch_conv3x3_backward(const float* grad_out, const float*
     const bool relu = flags & SSTEM_BRANCH_RELU, in_chunked = flags & SSTEM_BRANCH_IN_CHUNKED, out_chunked = flags & SSTEM_BRANCH_OUT_CHUNKED;
     if (!grad_out || !x || (relu && !y) || (grad_x && !packed_adjoint)) return SSTEM_E_NULL;
     if (flags & ~(SSTEM_BRANCH_RELU | SSTEM_BRANCH_IN_CHUNKED | SSTEM_BRANCH_OUT_CHUNKED)) return SSTEM_E_FLAG;
-    if (B <= 0 || h <= 0 || w <= 0 || h > (1 << 22) || w > (1 << 22)) return SSTEM_E_SHAPE;
+    if (!image_fits(B, h, w)) return SSTEM_E_SHAPE;
     if (cin <= 0 || cin > BC_MAXC || cout <= 0 || cout > BC_MAXC) return SSTEM_E_SHAPE;
-    const int in_chunks = (cin + 7) / 8 * 2, out_chunks = (cout + 7) / 8 * 2;
     // tile indices, the TMA chunk coordinate of the adjoint convolution and the mask kernel's block index are 32-bit
-    if (((w + TC_TW - 1) / TC_TW) * ((h + TC_TH - 1) / TC_TH) * B > INT32_MAX / 2 || B * out_chunks * 64 > INT32_MAX / 2)
-        return SSTEM_E_SHAPE;
+    if (tile_count(B, h, w) > INT32_MAX / 2 || B * ((cout + 7) / 8 * 2) * 64 > INT32_MAX / 2) return SSTEM_E_SHAPE;
     if (!aligned4(grad_out) || (y && !(out_chunked ? aligned16(y) : aligned4(y))) || !(in_chunked ? aligned16(x) : aligned4(x)) ||
         (packed_adjoint && !aligned16(packed_adjoint)) || (grad_x && !aligned4(grad_x)) || (grad_weight && !aligned4(grad_weight)) ||
         (grad_bias && !aligned4(grad_bias)))
@@ -1454,59 +1404,32 @@ extern "C" int sstem_branch_conv3x3_backward(const float* grad_out, const float*
     DeviceGuard guard(grad_out);
     if (guard.err) return guard.err;
     cudaStream_t s = (cudaStream_t)stream;
+    const BranchConvShape sh = branch_conv_shape(B, cin, cout, h, w, false);
     const int64_t plane = h * w;
     const bool wgrad = grad_weight != nullptr;
-    const int halves = cin > BW_N ? 2 : 1;
-    const int pairs = (int)std::min<int64_t>(((w + TC_TW - 1) / TC_TW) * ((h + TC_TH - 1) / TC_TH) * B, std::max(sm_count() / halves, 1));
+    const int pairs = std::min(sh.ntiles, std::max(sm_count() / sh.halves, 1));
     const int nw = cout * cin * 9;
     // about 64 bias partials per channel whatever the batch: (64 / B) blocks per image and chunk
     const int nbx = (int)std::max<int64_t>(64 / B, 1);
     // one stream-ordered workspace: g chunk-major | bias partials | x chunk-major (NCHW x, weight gradient) | weight partials
-    const size_t g_floats = (size_t)(B * out_chunks * plane) * 4, pb_floats = (size_t)(B * nbx * cout);
-    const size_t xc_floats = (wgrad && !in_chunked) ? (size_t)(B * in_chunks * plane) * 4 : 0, pw_floats = wgrad ? (size_t)pairs * nw : 0;
+    const size_t g_floats = (size_t)(B * sh.out_chunks * plane) * 4, pb_floats = (size_t)(B * nbx * cout);
+    const size_t xc_floats = (wgrad && !in_chunked) ? (size_t)(B * sh.in_chunks * plane) * 4 : 0, pw_floats = wgrad ? (size_t)pairs * nw : 0;
     const size_t off_pb = (g_floats + 3) / 4 * 4, off_xc = off_pb + (pb_floats + 3) / 4 * 4, off_pw = off_xc + xc_floats;
     float* ws = nullptr;
     if (workspace_alloc(reinterpret_cast<void**>(&ws), (off_pw + pw_floats) * sizeof(float), s)) return cudaErrorMemoryAllocation;
     float *gc = ws, *part_b = ws + off_pb, *xc = ws + off_xc, *part_w = ws + off_pw;
-    int e = 0;
-    {
-        const unsigned blocks = (unsigned)(B * out_chunks * nbx);
-        if (out_chunked)
-            branch_grad_mask_kernel<true><<<blocks, 256, 0, s>>>(grad_out, relu ? y : nullptr, gc, part_b, cout, out_chunks, nbx, plane);
-        else
-            branch_grad_mask_kernel<false><<<blocks, 256, 0, s>>>(grad_out, relu ? y : nullptr, gc, part_b, cout, out_chunks, nbx, plane);
-        count_launch();
-        e = finish_launch();
-    }
-    if (!e && grad_bias) {
-        tap_conv3x3_wgrad_reduce_kernel<<<(cout + 255) / 256, 256, 0, s>>>(nullptr, part_b, nullptr, grad_bias, 0, cout, (int)(B * nbx));
-        count_launch();
-        e = finish_launch();
-    }
+    const float* ym = relu ? y : nullptr;
+    const int64_t mask_blocks = B * sh.out_chunks * nbx;
+    int e = out_chunked ? launch256<branch_grad_mask_kernel<true>>(mask_blocks, s, grad_out, ym, gc, part_b, cout, sh.out_chunks, nbx, plane)
+                        : launch256<branch_grad_mask_kernel<false>>(mask_blocks, s, grad_out, ym, gc, part_b, cout, sh.out_chunks, nbx, plane);
+    if (!e && grad_bias)
+        e = launch256<sum_partials_kernel>((cout + 255) / 256, s, nullptr, part_b, nullptr, grad_bias, 0, cout, (int)(B * nbx));
     if (!e && grad_x)   // the adjoint convolution, cout -> cin channels, from g: no bias, no ReLU, NCHW out
         e = launch_branch_conv(gc, packed_adjoint, nullptr, grad_x, B, branch_conv_shape(B, cout, cin, h, w, false), false, s);
     if (!e && wgrad) {
-        const float* xw = x;
-        if (!in_chunked) {   // as the forward does: a TF32-rounded chunk-major copy
-            const int64_t n = B * in_chunks * plane;
-            nchw_to_chunked_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(x, xc, n, cin, in_chunks, plane);
-            count_launch();
-            e = finish_launch();
-            xw = xc;
-        }
-        if (!e) {
-            const BranchConvShape bs = branch_conv_shape(B, cin, cout, h, w, false);
-            BranchWgradShape sh;
-            sh.h = (int)h; sh.w = (int)w; sh.cin = cin; sh.cout = cout;
-            sh.tiles_x = bs.tiles_x; sh.tiles_y = bs.tiles_y; sh.ntiles = bs.ntiles;
-            sh.in_chunks = in_chunks; sh.out_chunks = out_chunks; sh.halves = halves;
-            e = launch_tc<branch_conv3x3_wgrad_kernel>(BW_SMEM, BW_THREADS, pairs * halves, s, gc, xw, part_w, sh);
-        }
-        if (!e) {
-            tap_conv3x3_wgrad_reduce_kernel<<<(nw + 255) / 256, 256, 0, s>>>(part_w, nullptr, grad_weight, nullptr, nw, 0, pairs);
-            count_launch();
-            e = finish_launch();
-        }
+        if (!in_chunked) e = to_chunked(x, xc, B, cin, sh.in_chunks, plane, s);   // as the forward does
+        if (!e) e = launch_tc<branch_conv3x3_wgrad_kernel>(BW_SMEM, BW_THREADS, pairs * sh.halves, s, gc, in_chunked ? x : xc, part_w, sh);
+        if (!e) e = launch256<sum_partials_kernel>((nw + 255) / 256, s, part_w, nullptr, grad_weight, nullptr, nw, 0, pairs);
     }
     cudaFreeAsync(ws, s);
     return e;

@@ -22,36 +22,38 @@ def _stream_ptr(t: torch.Tensor) -> int:
     return torch.cuda.current_stream(t.device).cuda_stream
 
 
-def _pack(weight: torch.Tensor, adjoint: bool) -> torch.Tensor:
-    name, entry, max_cout = (("pack_tap_conv_weight_adjoint", "sstem_tap_conv3x3_pack_weights_adjoint", 52) if adjoint
-                             else ("pack_tap_conv_weight", "sstem_tap_conv3x3_pack_weights", 64))
+def _pack(weight: torch.Tensor, name: str, entry: str, elems: str, max_cin: int, max_cout: int, tag=True) -> torch.Tensor:
+    """``weight`` packed by the C entry point ``entry`` into an image of ``elems()`` floats, for the public function ``name``
+    and within its channel limits.  ``tag``: the image carries (cin, cout) as ``_sstem_cin_cout``."""
     if weight.is_cuda == False:
         raise NotImplementedError()
     if weight.dtype != torch.float32 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3):
         raise TypeError(f"{name}: float32 [cout, cin, 3, 3] required")
     cout, cin = weight.shape[:2]
-    if cin > 52 or cout > max_cout:
-        raise ValueError(f"{name}: cin <= 52 and cout <= {max_cout} required")
+    if cin > max_cin or cout > max_cout:
+        raise ValueError(f"{name}: cin <= {max_cin} and cout <= {max_cout} required")
     lib = _lib.load()
-    packed = torch.empty(lib.sstem_tap_conv3x3_packed_elems(), dtype=torch.float32, device=weight.device)
+    packed = torch.empty(getattr(lib, elems)(), dtype=torch.float32, device=weight.device)
     code = getattr(lib, entry)(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
     if code:
         _lib.check(code, entry)
+    if tag:
+        packed._sstem_cin_cout = (int(cin), int(cout))
     return packed
 
 
 def pack_tap_conv_weight(weight: torch.Tensor) -> torch.Tensor:
     """``Conv2d.weight`` ``[cout<=64, cin<=52, 3, 3]`` -> the kernel's resident image (118 KB, TF32-rounded).  Pack once per
     layer, reuse for every call."""
-    packed = _pack(weight, adjoint=False)
-    packed._sstem_cin_cout = (int(weight.shape[1]), int(weight.shape[0]))
-    return packed
+    return _pack(weight, "pack_tap_conv_weight", "sstem_tap_conv3x3_pack_weights", "sstem_tap_conv3x3_packed_elems", 52, 64)
 
 
 def pack_tap_conv_weight_adjoint(weight: torch.Tensor) -> torch.Tensor:
     """``Conv2d.weight`` ``[cout<=52, cin<=52, 3, 3]`` -> the resident image of the adjoint convolution's weight
     ``W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]`` (cout -> cin channels), which the input gradient runs."""
-    return _pack(weight, adjoint=True)
+    # untagged: tap_conv3x3 would read the weight's (cin, cout), not the adjoint's (cout, cin)
+    return _pack(weight, "pack_tap_conv_weight_adjoint", "sstem_tap_conv3x3_pack_weights_adjoint", "sstem_tap_conv3x3_packed_elems",
+                 52, 52, tag=False)
 
 
 def tap_conv3x3(x: torch.Tensor, packed_weight: torch.Tensor, bias=None, cin=None, cout=None, upsample=True, tiled=False) -> torch.Tensor:
@@ -167,34 +169,23 @@ class ModuleTapProducer(torch.nn.Module):
         return TapConv3x3Function.apply(x, self.weight, self.bias, self.upsample, self.tiled, packed, adjoint)
 
 
-def _pack_branch(weight: torch.Tensor, name: str, entry: str) -> torch.Tensor:
-    if weight.is_cuda == False:
-        raise NotImplementedError()
-    if weight.dtype != torch.float32 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3):
-        raise TypeError(f"{name}: float32 [cout, cin, 3, 3] required")
-    cout, cin = weight.shape[:2]
-    if cin > 64 or cout > 64:
-        raise ValueError(f"{name}: cin <= 64 and cout <= 64 required")
-    lib = _lib.load()
-    packed = torch.empty(lib.sstem_branch_conv3x3_packed_elems(), dtype=torch.float32, device=weight.device)
-    code = getattr(lib, entry)(weight.contiguous().data_ptr(), packed.data_ptr(), cin, cout, _stream_ptr(weight))
-    if code:
-        _lib.check(code, entry)
-    packed._sstem_cin_cout = (int(cin), int(cout))
-    return packed
-
-
 def pack_branch_conv_weight(weight: torch.Tensor) -> torch.Tensor:
     """``Conv2d.weight`` ``[cout<=64, cin<=64, 3, 3]`` -> the resident image of :func:`branch_conv3x3` (144 KB,
     TF32-rounded).  Pack once per layer, reuse for every call."""
-    return _pack_branch(weight, "pack_branch_conv_weight", "sstem_branch_conv3x3_pack_weights")
+    return _pack(weight, "pack_branch_conv_weight", "sstem_branch_conv3x3_pack_weights", "sstem_branch_conv3x3_packed_elems", 64, 64)
 
 
 def pack_branch_conv_weight_adjoint(weight: torch.Tensor) -> torch.Tensor:
     """``Conv2d.weight`` ``[cout<=64, cin<=64, 3, 3]`` -> the resident image of the adjoint convolution's weight
     ``W'[ci][co][ky][kx] = W[co][ci][2-ky][2-kx]`` (cout -> cin channels), which the input gradient of
     :func:`branch_conv3x3_backward` runs.  It carries (cin, cout) of ``weight``."""
-    return _pack_branch(weight, "pack_branch_conv_weight_adjoint", "sstem_branch_conv3x3_pack_weights_adjoint")
+    return _pack(weight, "pack_branch_conv_weight_adjoint", "sstem_branch_conv3x3_pack_weights_adjoint",
+                 "sstem_branch_conv3x3_packed_elems", 64, 64)
+
+
+def _layout_shape(B, c, h, w, chunked):
+    """The shape of ``c`` channels: chunk-major ``[B, C8/4, h, w, 4]`` (C8 = c rounded up to 8), else ``[B, c, h, w]``."""
+    return (B, (c + 7) // 8 * 2, h, w, 4) if chunked else (B, c, h, w)
 
 
 def branch_conv3x3(x: torch.Tensor, packed: torch.Tensor, bias=None, relu=True, chunked_in=False, chunked_out=False) -> torch.Tensor:
@@ -214,10 +205,9 @@ def branch_conv3x3(x: torch.Tensor, packed: torch.Tensor, bias=None, relu=True, 
     if cin is None:
         raise ValueError("branch_conv3x3: the packed weight must come from pack_branch_conv_weight")
     B, c, h, w = x.shape[:4]
-    if (c, x.shape[-1]) != (((cin + 7) // 8 * 2, 4) if chunked_in else (cin, w)):
+    if tuple(x.shape) != _layout_shape(B, cin, h, w, chunked_in):
         raise ValueError(f"branch_conv3x3: x {tuple(x.shape)} does not match the weight's {cin} input channels")
-    shape = (B, (cout + 7) // 8 * 2, h, w, 4) if chunked_out else (B, cout, h, w)
-    out = torch.empty(shape, dtype=torch.float32, device=x.device)
+    out = torch.empty(_layout_shape(B, cout, h, w, chunked_out), dtype=torch.float32, device=x.device)
     if out.numel():
         flags = ((_lib.BRANCH_RELU if relu else 0) | (_lib.BRANCH_IN_CHUNKED if chunked_in else 0)
                  | (_lib.BRANCH_OUT_CHUNKED if chunked_out else 0))
@@ -245,10 +235,9 @@ def branch_conv3x3_backward(grad_out, y, x, packed_adjoint, cin, cout, relu=True
     B, _, h, w = x.shape[:4]
     if tuple(grad_out.shape) != (B, cout, h, w):
         raise ValueError(f"branch_conv3x3_backward: grad_out {tuple(grad_out.shape)} is not [{B}, {cout}, {h}, {w}]")
-    if tuple(x.shape) != ((B, (cin + 7) // 8 * 2, h, w, 4) if chunked_in else (B, cin, h, w)) or not x.is_contiguous():
+    if tuple(x.shape) != _layout_shape(B, cin, h, w, chunked_in) or not x.is_contiguous():
         raise ValueError(f"branch_conv3x3_backward: x {tuple(x.shape)} does not match cin = {cin} (chunked_in={chunked_in})")
-    if relu and (y is None or tuple(y.shape) != ((B, (cout + 7) // 8 * 2, h, w, 4) if chunked_out else (B, cout, h, w))
-                 or not y.is_contiguous()):
+    if relu and (y is None or tuple(y.shape) != _layout_shape(B, cout, h, w, chunked_out) or not y.is_contiguous()):
         raise ValueError("branch_conv3x3_backward: relu needs the forward's contiguous output y in its layout")
     need_x, need_w, need_b = need
     if need_x and (packed_adjoint is None or getattr(packed_adjoint, "_sstem_cin_cout", None) != (cin, cout)):
@@ -269,16 +258,22 @@ def branch_conv3x3_backward(grad_out, y, x, packed_adjoint, cin, cout, relu=True
     return gx, gw, gb
 
 
+def _branch_convs(x, packs, biases):
+    """The three half-resolution ``Conv2d -> ReLU`` layers of a tap branch, chained on :func:`branch_conv3x3`: NCHW x ->
+    chunk-major -> chunk-major -> NCHW.  Returns the output of each layer."""
+    a1 = branch_conv3x3(x, packs[0], biases[0], relu=True, chunked_in=False, chunked_out=True)
+    a2 = branch_conv3x3(a1, packs[1], biases[1], relu=True, chunked_in=True, chunked_out=True)
+    a3 = branch_conv3x3(a2, packs[2], biases[2], relu=True, chunked_in=True, chunked_out=False)
+    return a1, a2, a3
+
+
 class _TapBranchConvs(torch.autograd.Function):
-    """The three half-resolution ``Conv2d -> ReLU`` layers of a tap branch with their backward: the forward chains
-    :func:`branch_conv3x3` (NCHW -> chunk-major -> chunk-major -> NCHW) and keeps x, the two chunk-major activations and
-    the output; the backward runs :func:`branch_conv3x3_backward` once per layer, last layer first."""
+    """:func:`_branch_convs` with its backward: the forward keeps x, the two chunk-major activations and the output; the
+    backward runs :func:`branch_conv3x3_backward` once per layer, last layer first."""
 
     @staticmethod
     def forward(ctx, x, w0, b0, w2, b2, w4, b4, packs, adjoints):
-        a1 = branch_conv3x3(x, packs[0], b0.detach(), relu=True, chunked_in=False, chunked_out=True)
-        a2 = branch_conv3x3(a1, packs[1], b2.detach(), relu=True, chunked_in=True, chunked_out=True)
-        a3 = branch_conv3x3(a2, packs[2], b4.detach(), relu=True, chunked_in=True, chunked_out=False)
+        a1, a2, a3 = _branch_convs(x, packs, (b0.detach(), b2.detach(), b4.detach()))
         ctx.save_for_backward(x, a1, a2, a3)
         ctx.adjoints, ctx.shapes = adjoints, tuple(tuple(t.shape[:2]) for t in (w0, w2, w4))
         return a3
@@ -299,15 +294,11 @@ class _TapBranchConvs(torch.autograd.Function):
 
 
 class _BranchConv(ModuleTapProducer):
-    """One ``Conv2d(cin, cout, 3, 1, 1) -> ReLU`` of a tap branch on :func:`branch_conv3x3`, its weight packed on first use
-    and again whenever it changes."""
+    """The parameters of one ``Conv2d(cin, cout, 3, 1, 1) -> ReLU`` of a tap branch, with the cache of their packed images
+    (:meth:`ModuleTapProducer._cached`); :class:`ModuleTapBranch` runs the three layers together."""
 
     def __init__(self, in_channels, out_channels):
         super().__init__(in_channels, out_channels, upsample=False)
-
-    def forward(self, x, chunked_in, chunked_out):
-        packed = self._cached("_packed", pack_branch_conv_weight, x.device)
-        return branch_conv3x3(x, packed, self.bias.detach(), relu=True, chunked_in=chunked_in, chunked_out=chunked_out)
 
 
 class ModuleTapBranch(torch.nn.Module):
@@ -337,14 +328,12 @@ class ModuleTapBranch(torch.nn.Module):
             raise NotImplementedError("ModuleTapBranch is forward only: call it under torch.no_grad() or detach its input")
         if x.dim() != 4 or x.shape[1] != self.in_channels:
             raise ValueError(f"ModuleTapBranch: x [B, {self.in_channels}, h, w] required, got {tuple(x.shape)}")
+        convs = [getattr(self, k) for k in ("0", "2", "4")]
+        packs = tuple(c._cached("_packed", pack_branch_conv_weight, x.device) for c in convs)
         if self.trainable:
-            convs = [getattr(self, k) for k in ("0", "2", "4")]
-            packs = tuple(c._cached("_packed", pack_branch_conv_weight, x.device) for c in convs)
             adjoints = (tuple(c._cached("_packed_adjoint", pack_branch_conv_weight_adjoint, x.device) for c in convs)
                         if torch.is_grad_enabled() else None)
             a = _TapBranchConvs.apply(x.contiguous(), *(t for c in convs for t in (c.weight, c.bias)), packs, adjoints)
-            return getattr(self, "7")(a)
-        a = getattr(self, "0")(x.contiguous(), chunked_in=False, chunked_out=True)
-        a = getattr(self, "2")(a, chunked_in=True, chunked_out=True)
-        a = getattr(self, "4")(a, chunked_in=True, chunked_out=False)
+        else:
+            a = _branch_convs(x.contiguous(), packs, tuple(c.bias.detach() for c in convs))[2]
         return getattr(self, "7")(a)
